@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: Mpixel/s of `apply` + `combine_with(mode=3)` on batched 1080p frames (BASELINE.json, cfg 4).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference] [--dump-outputs DIR]
 
 A step = one pass of the target-referenced hot path over one batch of B synthetic 1920x1080 frames per GPU:
   (1) FlowBatch.apply(uint8x3 images, return_valid_area=True)   -> ofk_warp_t      (16 B/px algorithmic)
@@ -12,6 +12,9 @@ inside the timed region). `--impl reference` times the CPU oracle port of the re
 host threads OpenCV uses) on a bounded sample of the same workload.
 
 Multi-GPU: one process per GPU (torchrun), contiguous batch shards, no data-path collective; weak scaling.
+
+--dump-outputs DIR writes rank 0's outputs of the last timed step as float32 .npy files (see dump_outputs). The inputs
+depend on the arguments only, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -44,6 +47,25 @@ def host_inputs(n_distinct, seed=0):
     bm = rng.random((n_distinct, H, W)) > 0.02
     img = rng.integers(0, 256, (n_distinct, H, W, 3), dtype=np.uint8)
     return am, bm, img
+
+
+def dump_outputs(out_dir, arrays, n_sample=1 << 20, seed=0):
+    """Writes arrays (name -> DeviceArray of shape (B, H, W) or (B, H, W, C)) as out_dir/<name>.npy, float32, at the
+    same fixed, seeded sample of about n_sample pixels for every array: (n,) or (n, C). A full batch of outputs is
+    gigabytes; 2**20 pixels of the four outputs are 28 MiB."""
+    os.makedirs(out_dir, exist_ok=True)
+    B = next(iter(arrays.values())).shape[0]
+    idx = np.unique(np.random.default_rng(seed).integers(0, B * H * W, n_sample))
+    frame, pix = np.divmod(idx, H * W)
+    bounds = np.searchsorted(frame, np.arange(B + 1))
+    for name, dev in arrays.items():
+        tail = dev.shape[3:]
+        out = np.empty((len(idx),) + tail, np.float32)
+        for i in range(B):
+            a, b = bounds[i], bounds[i + 1]
+            if b > a:
+                out[a:b] = dev.frames(i, i + 1).numpy().reshape((H * W,) + tail)[pix[a:b]]
+        np.save(os.path.join(out_dir, name + '.npy'), out)
 
 
 class ClockSampler(threading.Thread):
@@ -193,7 +215,13 @@ def main():
     ap.add_argument('--no-e2e', action='store_true')
     ap.add_argument('--no-gather', action='store_true', help='skip the optional NCCL gather of the outputs (N > 1)')
     ap.add_argument('--no-modes12', action='store_true', help='skip the modes 1 / 2 block')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write a seeded sample of the outputs of the last timed step to DIR/<name>.npy (float32)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs needs --impl ours')
     if args.warmup < 3 and args.impl == 'ours':
         args.warmup = 3
 
@@ -302,6 +330,10 @@ def main():
     if dist is not None:
         from oflibnumpy_b200 import dist as ofd
         total_ms, warp_ms, comb_ms = ofd.max_over_ranks([total_ms, warp_ms, comb_ms])
+    if args.dump_outputs and rank == 0:
+        # what callers of FlowBatch.apply(images, return_valid_area=True) and FlowBatch.combine_with(other, 3) receive
+        dump_outputs(args.dump_outputs, {'apply_image': out_img, 'apply_valid': out_valid, 'combine_vecs': out_vecs,
+                                         'combine_mask': out_mask})
     # ---------------------------------------------------------------- optional gather of the outputs (SURVEY 8e)
     # The combined flows of all ranks are collected on rank 0 over NCCL / NVLink, in chunks on a side stream, while
     # this rank's stream already runs the next step (outputs double-buffered). Reported beside the headline: the

@@ -941,24 +941,54 @@ def test_torch_cuda_tensors_pass_through_zero_copy(of):
     assert np.array_equal(r.vecs.numpy()[1], c_n.vecs)
 
 
-def test_matrix_delegates_to_the_reference_on_a_host_copy(of):
+def test_matrix_delegates_to_the_reference_on_a_host_copy(of, monkeypatch):
     """Flow.matrix (OpenCV's robust estimators, SURVEY section 2 row 19: out of the hot path) runs on the reference package
-    with a host copy of the flow; with the vendored reference on the path it recovers the generating transform."""
+    with a host copy of the flow. A stand-in for the package receives the copy (vectors, reference and mask unchanged)
+    and the arguments; OpenCV's estimator on that copy, called as the reference's Flow.matrix calls it, recovers the
+    generating transform."""
     import sys
-    ref_dir = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'baseline', '_ref')
-    if not os.path.isdir(os.path.join(ref_dir, 'oflibnumpy')):
-        pytest.skip("vendored reference not present (baseline/_ref)")
-    sys.path.insert(0, ref_dir)
-    try:
-        tr = [['rotation', 30, 20, 12], ['translation', 4.5, -3.0]]
-        f = of.Flow.from_transforms(tr, (60, 80), 's')
-        m = f.matrix(dof=4, method='ransac')
-        np.testing.assert_allclose(m, of.matrix_from_transforms(tr), atol=1e-3)
-        assert of.get_flow_matrix(f.vecs, 's', dof=6, method='lmeds').shape == (3, 3)
-        assert f.visualise_arrows(grid_dist=10).shape == (60, 80, 3)
-        assert of.visualise_flow(f.vecs, 'bgr').shape == (60, 80, 3)
-    finally:
-        sys.path.remove(ref_dir)
+    import types
+    import cv2
+    made, calls = [], []
+
+    class RefFlow:
+        def __init__(self, vecs, ref, mask):
+            self.vecs, self.ref, self.mask = vecs, ref, mask
+            made.append(self)
+
+        def matrix(self, dof, method, masked):
+            calls.append(('matrix', dof, method, masked))
+            grid = np.stack(np.mgrid[:self.vecs.shape[0], :self.vecs.shape[1]], axis=-1)[..., ::-1]
+            src, dst = (grid - self.vecs, grid) if self.ref == 't' else (grid, grid + self.vecs)
+            keep = self.mask if masked in (None, True) else np.ones(self.mask.shape, bool)
+            est = {4: cv2.estimateAffinePartial2D, 6: cv2.estimateAffine2D}[dof]
+            m = est(src[keep].astype(np.float32), dst[keep].astype(np.float32),
+                    method={'ransac': cv2.RANSAC, 'lmeds': cv2.LMEDS}[method])[0]
+            return np.vstack((m, [0, 0, 1]))
+
+        def visualise_arrows(self, *args):
+            calls.append(('visualise_arrows',) + args)
+            return np.zeros(self.vecs.shape[:2] + (3,), np.uint8)
+
+    stand_in = types.ModuleType('oflibnumpy')
+    stand_in.Flow = RefFlow
+    monkeypatch.setitem(sys.modules, 'oflibnumpy', stand_in)
+    tr = [['rotation', 30, 20, 12], ['translation', 4.5, -3.0]]
+    mask = np.ones((60, 80), bool)
+    mask[10:20, 30:50] = False
+    f = of.Flow(of.Flow.from_transforms(tr, (60, 80), 's').vecs, 's', mask)
+    m = f.matrix(dof=4, method='ransac')
+    np.testing.assert_allclose(m, of.matrix_from_transforms(tr), atol=1e-3)
+    assert calls[-1] == ('matrix', 4, 'ransac', None)
+    copy = made[-1]
+    assert copy.ref == 's' and isinstance(copy.vecs, np.ndarray) and isinstance(copy.mask, np.ndarray)
+    same(copy.vecs, f.vecs)
+    same(copy.mask, mask)
+    assert of.get_flow_matrix(f.vecs, 's', dof=6, method='lmeds').shape == (3, 3)
+    assert calls[-1] == ('matrix', 6, 'lmeds', False)
+    assert f.visualise_arrows(grid_dist=10).shape == (60, 80, 3)
+    assert calls[-1] == ('visualise_arrows', 10, None, None, None, None, None, None)
+    assert of.visualise_flow(f.vecs, 'bgr').shape == (60, 80, 3)
 
 
 def test_resampled_mask_where_the_image_box_reaches_beyond_the_estimate(of):
