@@ -347,10 +347,12 @@ def combine_flows_host(flows_1, flows_2, mode, ref, masks_1=None, masks_2=None, 
 
 def apply_combine_host(flows_1, flows_2, images, ref='t', masks_1=None, masks_2=None, thresholded=False, out_images=None,
                        out_valid=None, out=None, out_masks=None, device=None):
-    """The pair of calls of a frame pipeline on HOST arrays in one pass (ofh_apply_combine3):
-    ``Flow(flows_1[i], ref, masks_1[i]).apply(images[i], return_valid_area=True)`` and
-    ``....combine_with(Flow(flows_2[i], ref, masks_2[i]), 3)``. ``flows_1`` and ``masks_1`` are uploaded once for both
-    kernels (apply_flow_host + combine_flows_host upload them twice). Returns (images, valid areas, vecs, masks)."""
+    """The pair of calls of a frame pipeline on HOST arrays in one pass (ofh_apply_combine3), with
+    ``A = Flow(flows_1[i], ref, masks_1[i])``: ``A.apply(images[i], return_valid_area=True)`` for ref 't',
+    ``A.invert('t').apply(images[i], return_valid_area=True)`` for ref 's' (the images are sampled at
+    p + flows_1[i][p]), and ``A.combine_with(Flow(flows_2[i], ref, masks_2[i]), 3)``. ``flows_1`` and ``masks_1`` are
+    uploaded once for both kernels (apply_flow_host + combine_flows_host upload them twice). Returns (images, valid
+    areas, vecs, masks)."""
     ref = get_valid_ref(ref)
     a, b = _c(flows_1, np.float32), _c(flows_2, np.float32)
     images = _c(images)

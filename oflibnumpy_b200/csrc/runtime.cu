@@ -4,6 +4,7 @@
 #include <stdarg.h>
 #include <string.h>
 
+#include <algorithm>
 #include <mutex>
 
 #include "ofk_common.cuh"
@@ -210,12 +211,13 @@ namespace {
 
 constexpr int kSlots = 3;
 constexpr size_t kChunkTarget = 48u << 20;  // ~48 MiB of traffic per chunk keeps PCIe busy without hoarding HBM
+constexpr size_t kFlagBytes = 2 * sizeof(int);  // per frame: the zero flags of ofk_combine3
+constexpr int kMaxBuffers = 10;             // device buffers of one chunk (ofh_apply_combine3 has the most)
 
 struct Slot {
     cudaStream_t st = nullptr;
     char* dev = nullptr;
     size_t cap = 0;
-    size_t used = 0;
     // Small results (the zero flags of ofh_combine3) come back through a pinned staging buffer: a device-to-host copy
     // into the caller's pageable array would block the host until the chunk has finished and serialise the ring.
     int* hflags = nullptr;
@@ -227,11 +229,6 @@ struct Slot {
         flags_dst = nullptr;
         flags_n = 0;
     }
-    void* take(size_t bytes) {
-        size_t off = (used + 255) & ~size_t(255);
-        used = off + bytes;
-        return dev + off;
-    }
 };
 struct Ring {
     int device = -1;
@@ -240,17 +237,22 @@ struct Ring {
 };
 Ring g_ring;
 
-int ring_prepare(int device, size_t bytes_per_slot) {
+void ring_free() {
+    if (g_ring.device < 0) return;
+    cudaSetDevice(g_ring.device);
+    for (auto& s : g_ring.slot) {
+        if (s.st) cudaStreamSynchronize(s.st);
+        if (s.dev) cudaFree(s.dev);
+        if (s.hflags) cudaFreeHost(s.hflags);
+        if (s.st) cudaStreamDestroy(s.st);
+        s = Slot();
+    }
+    g_ring.device = -1;
+}
+
+int ring_prepare(int device, size_t bytes_per_slot, size_t flag_ints) {
     if (g_ring.device != device) {
-        if (g_ring.device >= 0) {
-            cudaSetDevice(g_ring.device);
-            for (auto& s : g_ring.slot) {
-                if (s.dev) cudaFree(s.dev);
-                if (s.hflags) cudaFreeHost(s.hflags);
-                if (s.st) cudaStreamDestroy(s.st);
-                s = Slot();
-            }
-        }
+        ring_free();
         g_ring.device = device;
     }
     OFK_CUDA(cudaSetDevice(device));
@@ -272,6 +274,13 @@ int ring_prepare(int device, size_t bytes_per_slot) {
                 return OFK_ENOMEM;
             }
             s.cap = bytes_per_slot;
+        }
+        if (s.hflags_cap < flag_ints) {
+            if (s.hflags) OFK_CUDA(cudaFreeHost(s.hflags));
+            s.hflags = nullptr;
+            s.hflags_cap = 0;
+            OFK_CUDA(cudaHostAlloc((void**)&s.hflags, sizeof(int) * flag_ints, cudaHostAllocDefault));
+            s.hflags_cap = flag_ints;
         }
     }
     return OFK_OK;
@@ -322,16 +331,88 @@ int ring_copy(void* dst, const void* src, size_t bytes, bool to_device, cudaStre
         OFK_CUDA(cudaMemcpyAsync(dst, src, bytes, to_device ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToHost, st));
     return OFK_OK;
 }
-#define OFH_COPY_IN(dst, src, bytes)                                                   \
+#define OFH_TRY(call)                                                                  \
     do {                                                                               \
-        const int rc_ = ring_copy(dst, src, bytes, true, s.st);                        \
+        const int rc_ = (call);                                                        \
         if (rc_ != OFK_OK) return rc_;                                                 \
     } while (0)
-#define OFH_COPY_OUT(dst, src, bytes)                                                  \
-    do {                                                                               \
-        const int rc_ = ring_copy(dst, src, bytes, false, s.st);                       \
-        if (rc_ != OFK_OK) return rc_;                                                 \
-    } while (0)
+
+// Frames [n0, n0 + cn) of a ring pass on one slot: cn frames of each buffer the call listed, packed into the slot (a
+// buffer of 0 bytes per frame is absent: nullptr, and its copies do nothing).
+struct Chunk {
+    Slot* slot = nullptr;
+    int n0 = 0, cn = 0;
+    const size_t* frame_bytes = nullptr;
+    char* buf[kMaxBuffers] = {};
+
+    Chunk() = default;
+    Chunk(Slot& s, int n0_, int cn_, const size_t* frame_bytes_, int nbuf)
+        : slot(&s), n0(n0_), cn(cn_), frame_bytes(frame_bytes_) {
+        size_t off = 0;
+        for (int i = 0; i < nbuf; ++i) {
+            buf[i] = frame_bytes[i] ? s.dev + off : nullptr;
+            off += pad256(frame_bytes[i] * cn);
+        }
+    }
+    template <class T = void>
+    T* at(int i) const { return (T*)buf[i]; }
+    ofk_stream_t stream() const { return (ofk_stream_t)slot->st; }
+    // buffer i from / to the caller's array of all N frames
+    int in(int i, const void* host) const {
+        return ring_copy(buf[i], (const char*)host + n0 * frame_bytes[i], frame_bytes[i] * cn, true, slot->st);
+    }
+    int out(void* host, int i) const {
+        return ring_copy((char*)host + n0 * frame_bytes[i], buf[i], frame_bytes[i] * cn, false, slot->st);
+    }
+};
+
+// One pass of N frames through the ring, in chunks of as many frames as kChunkTarget holds, the slots taken in turn.
+// frame_bytes lists the device buffers of a chunk in bytes per frame. launch(chunk) queues the chunk's uploads and
+// kernels on its slot's stream; download(chunk) queues its downloads, after the NEXT chunk has been launched: with
+// pageable user buffers a download blocks the host, and this order keeps the device busy meanwhile (with pinned buffers
+// the order is irrelevant, every copy is asynchronous). Where flags is not NULL, the last buffer holds kFlagBytes per
+// frame, which come back to flags through the slot's pinned staging.
+template <int NB, class Launch, class Download>
+int run_ring(int device, int N, const size_t (&frame_bytes)[NB], int* flags, Launch&& launch, Download&& download) {
+    static_assert(NB <= kMaxBuffers, "raise kMaxBuffers");
+    if (N == 0) return OFK_OK;
+    std::lock_guard<std::mutex> lk(g_ring.mu);
+    DeviceGuard restore_device;
+    size_t per_frame = 0;
+    for (size_t b : frame_bytes) per_frame += b;
+    const int cf = (int)std::min<size_t>(N, std::max<size_t>(1, kChunkTarget / per_frame));
+    size_t per_slot = 0;
+    for (size_t b : frame_bytes) per_slot += pad256(b * cf);
+    OFH_TRY(ring_prepare(device, per_slot, flags ? 2 * (size_t)cf : 0));
+    DrainRing drain_on_exit;
+    auto finish = [&](const Chunk& c) -> int {
+        OFH_TRY(download(c));
+        if (flags) {
+            Slot& s = *c.slot;
+            OFK_CUDA(cudaMemcpyAsync(s.hflags, c.buf[NB - 1], kFlagBytes * c.cn, cudaMemcpyDeviceToHost, s.st));
+            s.flags_dst = flags + (size_t)c.n0 * 2;
+            s.flags_n = (size_t)2 * c.cn;
+        }
+        return OFK_OK;
+    };
+    Chunk prev;
+    for (int n0 = 0, k = 0; n0 < N; n0 += cf, ++k) {
+        Slot& s = g_ring.slot[k % kSlots];
+        // a slot is reused only after everything queued on its stream has drained (keeps device buffers private)
+        OFK_CUDA(cudaStreamSynchronize(s.st));
+        s.deliver();
+        const Chunk c(s, n0, std::min(cf, N - n0), frame_bytes, NB);
+        OFH_TRY(launch(c));
+        if (prev.cn) OFH_TRY(finish(prev));
+        prev = c;
+    }
+    OFH_TRY(finish(prev));
+    for (auto& s : g_ring.slot) {
+        OFK_CUDA(cudaStreamSynchronize(s.st));
+        s.deliver();
+    }
+    return OFK_OK;
+}
 
 }  // namespace
 
@@ -340,148 +421,44 @@ extern "C" int ofh_warp_t(const void* payload, int dtype, int C, int arith, cons
                           int mask_rule, int N, int H, int W, int device) {
     OFK_CHECK_ARG(flow != nullptr && N >= 0 && H > 0 && W > 0 && C >= 0, "ofh_warp_t: bad arguments");
     OFK_CHECK_ARG(dtype >= OFK_U8 && dtype <= OFK_F64, "ofh_warp_t: unknown dtype %d", dtype);
-    if (N == 0) return OFK_OK;
-    std::lock_guard<std::mutex> lk(g_ring.mu);
-    DeviceGuard restore_device;
-    const size_t px = (size_t)H * W, es = esize(dtype);
-    const size_t b_flow = px * 8, b_pay = px * C * es, b_m = px;
-    const size_t per_frame = pad256(b_flow) + 2 * pad256(b_pay) + 3 * pad256(b_m);
-    int cf = (int)(kChunkTarget / per_frame);
-    if (cf < 1) cf = 1;
-    if (cf > N) cf = N;
-    int rc = ring_prepare(device, per_frame * cf + 4096);
-    if (rc != OFK_OK) return rc;
-    DrainRing drain_on_exit;
-    struct Pending {
-        Slot* slot;
-        int n0, cn;
-        void* d_out;
-        uint8_t* d_om;
-    };
-    Pending prev = {};
-    bool have_prev = false;
-    auto download = [&](const Pending& p) -> int {
-        Slot& s = *p.slot;
-        if (C) OFH_COPY_OUT((char*)out + (size_t)p.n0 * b_pay, p.d_out, b_pay * p.cn);
-        if (p.d_om) OFH_COPY_OUT(out_mask + (size_t)p.n0 * px, p.d_om, b_m * p.cn);
-        return OFK_OK;
-    };
-    int chunk = 0;
-    for (int n0 = 0; n0 < N; n0 += cf, ++chunk) {
-        Slot& s = g_ring.slot[chunk % kSlots];
-        const int cn = (N - n0 < cf) ? (N - n0) : cf;
-        // a slot is reused only after everything queued on its stream has drained (keeps device buffers private)
-        OFK_CUDA(cudaStreamSynchronize(s.st));
-        s.used = 0;
-        float* d_flow = (float*)s.take(b_flow * cn);
-        void* d_pay = C ? s.take(b_pay * cn) : nullptr;
-        void* d_out = C ? s.take(b_pay * cn) : nullptr;
-        uint8_t* d_pm = payload_mask ? (uint8_t*)s.take(b_m * cn) : nullptr;
-        uint8_t* d_fm = flow_mask ? (uint8_t*)s.take(b_m * cn) : nullptr;
-        uint8_t* d_om = out_mask ? (uint8_t*)s.take(b_m * cn) : nullptr;
-        OFH_COPY_IN(d_flow, flow + (size_t)n0 * px * 2, b_flow * cn);
-        if (C) OFH_COPY_IN(d_pay, (const char*)payload + (size_t)n0 * b_pay, b_pay * cn);
-        if (d_pm) OFH_COPY_IN(d_pm, payload_mask + (size_t)n0 * px, b_m * cn);
-        if (d_fm) OFH_COPY_IN(d_fm, flow_mask + (size_t)n0 * px, b_m * cn);
-        rc = ofk_warp_t(d_pay, dtype, C, arith, d_flow, flow_sign, d_pm, d_fm, d_out, d_om, mask_rule, cn, H, W, H, W,
-                        0, 0, 1, (ofk_stream_t)s.st);
-        if (rc != OFK_OK) return rc;
-        // The download of a chunk is issued after the NEXT chunk has been uploaded and launched: with pageable user
-        // buffers a download blocks the host, and this order keeps the device busy meanwhile (with pinned buffers the
-        // order is irrelevant, every copy is asynchronous).
-        if (have_prev) {
-            rc = download(prev);
-            if (rc != OFK_OK) return rc;
-        }
-        prev = {&s, n0, cn, d_out, d_om};
-        have_prev = true;
-    }
-    if (have_prev) {
-        rc = download(prev);
-        if (rc != OFK_OK) return rc;
-    }
-    for (auto& s : g_ring.slot) OFK_CUDA(cudaStreamSynchronize(s.st));
-    return OFK_OK;
+    const size_t px = (size_t)H * W, b_pay = px * C * esize(dtype);
+    enum { kFlow, kPay, kOut, kPm, kFm, kOm };
+    return run_ring(
+        device, N, {px * 8, b_pay, b_pay, payload_mask ? px : 0, flow_mask ? px : 0, out_mask ? px : 0}, nullptr,
+        [&](const Chunk& c) {
+            OFH_TRY(c.in(kFlow, flow));
+            OFH_TRY(c.in(kPay, payload));
+            OFH_TRY(c.in(kPm, payload_mask));
+            OFH_TRY(c.in(kFm, flow_mask));
+            return ofk_warp_t(c.at(kPay), dtype, C, arith, c.at<float>(kFlow), flow_sign, c.at<uint8_t>(kPm),
+                              c.at<uint8_t>(kFm), c.at(kOut), c.at<uint8_t>(kOm), mask_rule, c.cn, H, W, H, W, 0, 0, 1,
+                              c.stream());
+        },
+        [&](const Chunk& c) {
+            OFH_TRY(c.out(out, kOut));
+            return c.out(out_mask, kOm);
+        });
 }
 
 extern "C" int ofh_combine3(const float* A, const uint8_t* Am, const float* B, const uint8_t* Bm, int ref, float thr,
                             float* out, uint8_t* out_mask, int* flags, int N, int H, int W, int device) {
     OFK_CHECK_ARG(A && B && out && out_mask && N >= 0 && H > 0 && W > 0, "ofh_combine3: bad arguments");
-    if (N == 0) return OFK_OK;
-    std::lock_guard<std::mutex> lk(g_ring.mu);
-    DeviceGuard restore_device;
-    const size_t px = (size_t)H * W;
-    const size_t b_flow = px * 8, b_m = px;
-    const size_t per_frame = 3 * pad256(b_flow) + 3 * pad256(b_m) + 256;
-    int cf = (int)(kChunkTarget / per_frame);
-    if (cf < 1) cf = 1;
-    if (cf > N) cf = N;
-    int rc = ring_prepare(device, per_frame * cf + 4096);
-    if (rc != OFK_OK) return rc;
-    DrainRing drain_on_exit;
-    struct Pending {
-        Slot* slot;
-        int n0, cn;
-        float* dO;
-        uint8_t* dOm;
-        int* dF;
-    };
-    Pending prev = {};
-    bool have_prev = false;
-    auto download = [&](const Pending& p) -> int {
-        Slot& s = *p.slot;
-        OFH_COPY_OUT(out + (size_t)p.n0 * px * 2, p.dO, b_flow * p.cn);
-        OFH_COPY_OUT(out_mask + (size_t)p.n0 * px, p.dOm, b_m * p.cn);
-        if (flags) {                                     // small: always through the slot's pinned staging words
-            OFK_CUDA(cudaMemcpyAsync(s.hflags, p.dF, sizeof(int) * 2 * p.cn, cudaMemcpyDeviceToHost, s.st));
-            s.flags_dst = flags + (size_t)p.n0 * 2;
-            s.flags_n = (size_t)2 * p.cn;
-        }
-        return OFK_OK;
-    };
-    int chunk = 0;
-    for (int n0 = 0; n0 < N; n0 += cf, ++chunk) {
-        Slot& s = g_ring.slot[chunk % kSlots];
-        const int cn = (N - n0 < cf) ? (N - n0) : cf;
-        OFK_CUDA(cudaStreamSynchronize(s.st));
-        s.deliver();
-        s.used = 0;
-        if (flags && s.hflags_cap < (size_t)2 * cf) {
-            if (s.hflags) OFK_CUDA(cudaFreeHost(s.hflags));
-            s.hflags = nullptr;
-            s.hflags_cap = 0;
-            OFK_CUDA(cudaHostAlloc((void**)&s.hflags, sizeof(int) * 2 * cf, cudaHostAllocDefault));
-            s.hflags_cap = (size_t)2 * cf;
-        }
-        float* dA = (float*)s.take(b_flow * cn);
-        float* dB = (float*)s.take(b_flow * cn);
-        float* dO = (float*)s.take(b_flow * cn);
-        uint8_t* dAm = Am ? (uint8_t*)s.take(b_m * cn) : nullptr;
-        uint8_t* dBm = Bm ? (uint8_t*)s.take(b_m * cn) : nullptr;
-        uint8_t* dOm = (uint8_t*)s.take(b_m * cn);
-        int* dF = (int*)s.take(sizeof(int) * 2 * cn);
-        OFH_COPY_IN(dA, A + (size_t)n0 * px * 2, b_flow * cn);
-        OFH_COPY_IN(dB, B + (size_t)n0 * px * 2, b_flow * cn);
-        if (dAm) OFH_COPY_IN(dAm, Am + (size_t)n0 * px, b_m * cn);
-        if (dBm) OFH_COPY_IN(dBm, Bm + (size_t)n0 * px, b_m * cn);
-        rc = ofk_combine3(dA, dAm, dB, dBm, ref, thr, dO, dOm, dF, cn, H, W, (ofk_stream_t)s.st);
-        if (rc != OFK_OK) return rc;
-        if (have_prev) {                                 // see ofh_warp_t: downloads trail the launches by one chunk
-            rc = download(prev);
-            if (rc != OFK_OK) return rc;
-        }
-        prev = {&s, n0, cn, dO, dOm, dF};
-        have_prev = true;
-    }
-    if (have_prev) {
-        rc = download(prev);
-        if (rc != OFK_OK) return rc;
-    }
-    for (auto& s : g_ring.slot) {
-        OFK_CUDA(cudaStreamSynchronize(s.st));
-        s.deliver();
-    }
-    return OFK_OK;
+    const size_t px = (size_t)H * W, b_flow = px * 8;
+    enum { kA, kB, kO, kAm, kBm, kOm, kF };
+    return run_ring(
+        device, N, {b_flow, b_flow, b_flow, Am ? px : 0, Bm ? px : 0, px, kFlagBytes}, flags,
+        [&](const Chunk& c) {
+            OFH_TRY(c.in(kA, A));
+            OFH_TRY(c.in(kB, B));
+            OFH_TRY(c.in(kAm, Am));
+            OFH_TRY(c.in(kBm, Bm));
+            return ofk_combine3(c.at<float>(kA), c.at<uint8_t>(kAm), c.at<float>(kB), c.at<uint8_t>(kBm), ref, thr,
+                                c.at<float>(kO), c.at<uint8_t>(kOm), c.at<int>(kF), c.cn, H, W, c.stream());
+        },
+        [&](const Chunk& c) {
+            OFH_TRY(c.out(out, kO));
+            return c.out(out_mask, kOm);
+        });
 }
 
 // The pair of calls a frame pipeline makes per batch -- `A.apply(image, return_valid_area=True)` and
@@ -495,108 +472,35 @@ extern "C" int ofh_apply_combine3(const void* image, int dtype, int C, int arith
                   "ofh_apply_combine3: bad arguments");
     OFK_CHECK_ARG(dtype >= OFK_U8 && dtype <= OFK_F64, "ofh_apply_combine3: unknown dtype %d", dtype);
     OFK_CHECK_ARG(ref == 's' || ref == 't', "ofh_apply_combine3: ref must be 's' or 't'");
-    if (N == 0) return OFK_OK;
-    std::lock_guard<std::mutex> lk(g_ring.mu);
-    DeviceGuard restore_device;
-    const size_t px = (size_t)H * W, es = esize(dtype);
-    const size_t b_flow = px * 8, b_m = px, b_img = px * C * es;
-    const size_t per_frame = 3 * pad256(b_flow) + 4 * pad256(b_m) + 2 * pad256(b_img) + 256;
-    int cf = (int)(kChunkTarget / per_frame);
-    if (cf < 1) cf = 1;
-    if (cf > N) cf = N;
-    int rc = ring_prepare(device, per_frame * cf + 8192);
-    if (rc != OFK_OK) return rc;
-    DrainRing drain_on_exit;
-    struct Pending {
-        Slot* slot;
-        int n0, cn;
-        void* dOi;
-        uint8_t* dOv;
-        float* dO;
-        uint8_t* dOm;
-        int* dF;
-    };
-    Pending prev = {};
-    bool have_prev = false;
-    auto download = [&](const Pending& p) -> int {
-        Slot& s = *p.slot;
-        OFH_COPY_OUT((char*)out_image + (size_t)p.n0 * b_img, p.dOi, b_img * p.cn);
-        if (p.dOv) OFH_COPY_OUT(out_valid + (size_t)p.n0 * px, p.dOv, b_m * p.cn);
-        OFH_COPY_OUT(out + (size_t)p.n0 * px * 2, p.dO, b_flow * p.cn);
-        OFH_COPY_OUT(out_mask + (size_t)p.n0 * px, p.dOm, b_m * p.cn);
-        if (flags) {
-            OFK_CUDA(cudaMemcpyAsync(s.hflags, p.dF, sizeof(int) * 2 * p.cn, cudaMemcpyDeviceToHost, s.st));
-            s.flags_dst = flags + (size_t)p.n0 * 2;
-            s.flags_n = (size_t)2 * p.cn;
-        }
-        return OFK_OK;
-    };
-    int chunk = 0;
-    for (int n0 = 0; n0 < N; n0 += cf, ++chunk) {
-        Slot& s = g_ring.slot[chunk % kSlots];
-        const int cn = (N - n0 < cf) ? (N - n0) : cf;
-        OFK_CUDA(cudaStreamSynchronize(s.st));
-        s.deliver();
-        s.used = 0;
-        if (flags && s.hflags_cap < (size_t)2 * cf) {
-            if (s.hflags) OFK_CUDA(cudaFreeHost(s.hflags));
-            s.hflags = nullptr;
-            s.hflags_cap = 0;
-            OFK_CUDA(cudaHostAlloc((void**)&s.hflags, sizeof(int) * 2 * cf, cudaHostAllocDefault));
-            s.hflags_cap = (size_t)2 * cf;
-        }
-        float* dA = (float*)s.take(b_flow * cn);
-        float* dB = (float*)s.take(b_flow * cn);
-        float* dO = (float*)s.take(b_flow * cn);
-        void* dI = s.take(b_img * cn);
-        void* dOi = s.take(b_img * cn);
-        uint8_t* dAm = Am ? (uint8_t*)s.take(b_m * cn) : nullptr;
-        uint8_t* dBm = Bm ? (uint8_t*)s.take(b_m * cn) : nullptr;
-        uint8_t* dOm = (uint8_t*)s.take(b_m * cn);
-        uint8_t* dOv = out_valid ? (uint8_t*)s.take(b_m * cn) : nullptr;
-        int* dF = (int*)s.take(sizeof(int) * 2 * cn);
-        OFH_COPY_IN(dA, A + (size_t)n0 * px * 2, b_flow * cn);
-        if (dAm) OFH_COPY_IN(dAm, Am + (size_t)n0 * px, b_m * cn);
-        OFH_COPY_IN(dI, (const char*)image + (size_t)n0 * b_img, b_img * cn);
-        // the image warp starts while B is still on its way
-        rc = ofk_warp_t(dI, dtype, C, arith, dA, ref == 't' ? -1.0f : 1.0f, nullptr, dOv ? dAm : nullptr, dOi, dOv,
-                        mask_rule, cn, H, W, H, W, 0, 0, 1, (ofk_stream_t)s.st);
-        if (rc != OFK_OK) return rc;
-        OFH_COPY_IN(dB, B + (size_t)n0 * px * 2, b_flow * cn);
-        if (dBm) OFH_COPY_IN(dBm, Bm + (size_t)n0 * px, b_m * cn);
-        rc = ofk_combine3(dA, dAm, dB, dBm, ref, thr, dO, dOm, dF, cn, H, W, (ofk_stream_t)s.st);
-        if (rc != OFK_OK) return rc;
-        if (have_prev) {                                 // see ofh_warp_t: downloads trail the launches by one chunk
-            rc = download(prev);
-            if (rc != OFK_OK) return rc;
-        }
-        prev = {&s, n0, cn, dOi, dOv, dO, dOm, dF};
-        have_prev = true;
-    }
-    if (have_prev) {
-        rc = download(prev);
-        if (rc != OFK_OK) return rc;
-    }
-    for (auto& s : g_ring.slot) {
-        OFK_CUDA(cudaStreamSynchronize(s.st));
-        s.deliver();
-    }
-    return OFK_OK;
+    const size_t px = (size_t)H * W, b_flow = px * 8, b_img = px * C * esize(dtype);
+    enum { kA, kB, kO, kI, kOi, kAm, kBm, kOm, kOv, kF };
+    return run_ring(
+        device, N,
+        {b_flow, b_flow, b_flow, b_img, b_img, Am ? px : 0, Bm ? px : 0, px, out_valid ? px : 0, kFlagBytes}, flags,
+        [&](const Chunk& c) {
+            OFH_TRY(c.in(kA, A));
+            OFH_TRY(c.in(kAm, Am));
+            OFH_TRY(c.in(kI, image));
+            // the image warp starts while B is still on its way
+            OFH_TRY(ofk_warp_t(c.at(kI), dtype, C, arith, c.at<float>(kA), ref == 't' ? -1.0f : 1.0f, nullptr,
+                               out_valid ? c.at<uint8_t>(kAm) : nullptr, c.at(kOi), c.at<uint8_t>(kOv), mask_rule,
+                               c.cn, H, W, H, W, 0, 0, 1, c.stream()));
+            OFH_TRY(c.in(kB, B));
+            OFH_TRY(c.in(kBm, Bm));
+            return ofk_combine3(c.at<float>(kA), c.at<uint8_t>(kAm), c.at<float>(kB), c.at<uint8_t>(kBm), ref, thr,
+                                c.at<float>(kO), c.at<uint8_t>(kOm), c.at<int>(kF), c.cn, H, W, c.stream());
+        },
+        [&](const Chunk& c) {
+            OFH_TRY(c.out(out_image, kOi));
+            OFH_TRY(c.out(out_valid, kOv));
+            OFH_TRY(c.out(out, kO));
+            return c.out(out_mask, kOm);
+        });
 }
 
 extern "C" int ofh_release(void) {
     std::lock_guard<std::mutex> lk(g_ring.mu);
     DeviceGuard restore_device;
-    if (g_ring.device >= 0) {
-        cudaSetDevice(g_ring.device);
-        for (auto& s : g_ring.slot) {
-            if (s.st) cudaStreamSynchronize(s.st);
-            if (s.dev) cudaFree(s.dev);
-            if (s.hflags) cudaFreeHost(s.hflags);
-            if (s.st) cudaStreamDestroy(s.st);
-            s = Slot();
-        }
-        g_ring.device = -1;
-    }
+    ring_free();
     return OFK_OK;
 }

@@ -48,6 +48,14 @@ def test_argument_errors_do_not_need_a_gpu(lib_path):
         _lib.call('ofk_warp_t', None, 0, 0, 0, None, -1.0, None, None, None, None, 0, 1, 4, 4, 4, 4, 0, 0, 1, None)
     with pytest.raises(_lib.OflibCudaError, match="ref must be"):
         _lib.call('ofk_combine3', 16, None, 16, None, ord('x'), 0.0, 16, 16, None, 1, 4, 4, None)
+    # host-buffer entry points: checked before the ring or a device is touched
+    with pytest.raises(_lib.OflibCudaError, match="ofh_warp_t: bad arguments"):
+        _lib.call('ofh_warp_t', 16, 0, 1, 0, None, -1.0, None, None, 16, None, 0, 1, 4, 4, 0)
+    with pytest.raises(_lib.OflibCudaError, match="ofh_combine3: bad arguments"):
+        _lib.call('ofh_combine3', 16, None, None, None, ord('t'), 0.0, 16, 16, None, 1, 4, 4, 0)
+    with pytest.raises(_lib.OflibCudaError, match="ofh_apply_combine3: ref must be"):
+        _lib.call('ofh_apply_combine3', 16, 0, 1, 0, 0, 16, None, 16, None, ord('x'), 0.0, 16, None, 16, 16, None, 1,
+                  4, 4, 0)
 
 
 def test_no_cpu_fallback_without_gpu(lib_path):

@@ -909,6 +909,70 @@ def test_host_buffer_api_with_plain_numpy_batches(of):
         same(m.view(np.uint8), dm.view(np.uint8))
 
 
+def test_host_buffer_apply_combine3_and_flags(of):
+    """ofh_apply_combine3 (batch.apply_combine_host) and the flags of ofh_combine3 / ofh_apply_combine3 give the bytes
+    of the device API: ref 't' and 's', with and without masks, pageable and pinned buffers, at one frame per chunk
+    (1080p: slots are reused, the last download trails) and at several frames per chunk with a short last chunk
+    (540x960). The ref 's' image warp samples at p + A[p], i.e. it is FlowBatch(-A, 't').apply."""
+    from oflibnumpy_b200 import _lib, _ops
+    from oflibnumpy_b200.batch import FlowBatch
+    rng = np.random.default_rng(23)
+    n, device = 5, of.device.get_device()
+
+    def u8(x):
+        return x.view(np.uint8) if x.dtype == np.bool_ else x
+
+    def ptr(x):
+        return None if x is None else x.ctypes.data
+
+    def pinned_copy(x, keep):
+        if x is None:
+            return None
+        p, handle = of.device.pinned_empty(x.shape, x.dtype)
+        keep.append(handle)
+        p[...] = x
+        return p
+
+    for h, w in ((1080, 1920), (540, 960)):
+        a = np.stack([_smooth_flow(rng, h, w, 20) for _ in range(n)])
+        b = np.stack([_smooth_flow(rng, h, w, 20) for _ in range(n)])
+        a[1] = 0                                              # zero operands: the early-exit flags must come back
+        b[3] = 0
+        img = rng.integers(0, 256, (n, h, w, 3), dtype=np.uint8)
+        arith, rule = _ops.promoted_rule(img.dtype, False)
+        for masked in (True, False):
+            am, bm = (rng.random((n, h, w)) > 0.02, rng.random((n, h, w)) > 0.02) if masked else (None, None)
+            for r in ('t', 's'):
+                d_img, d_valid = FlowBatch(a if r == 't' else -a, 't', am).apply(img, return_valid_area=True)
+                res, d_flags = FlowBatch(a, r, am).combine_with(FlowBatch(b, r, bm), 3, return_flags=True)
+                want = (d_img.numpy(), d_valid.numpy(), *res.numpy())
+                want_flags = d_flags.numpy()
+                assert (want_flags[1, 0], want_flags[3, 1]) == (0, 0) and want_flags[0].all()
+                for pinned in (False, True):
+                    ins, outs, keep = (a, b, img, am, bm), [np.empty_like(x) for x in want], []
+                    if pinned:
+                        ins, outs = [pinned_copy(x, keep) for x in ins], [pinned_copy(x, keep) for x in outs]
+                    got = of.batch.apply_combine_host(ins[0], ins[1], ins[2], r, ins[3], ins[4], out_images=outs[0],
+                                                      out_valid=outs[1].view(np.bool_), out=outs[2],
+                                                      out_masks=outs[3])
+                    for g, x in zip(got, want):
+                        same(u8(g), u8(x))
+                # flags and outputs of direct calls into plain numpy buffers; out_valid = NULL once
+                v, m, flags = np.empty_like(a), np.empty((n, h, w), np.bool_), np.full((n, 2), -1, np.int32)
+                _lib.call('ofh_combine3', a.ctypes.data, ptr(am), b.ctypes.data, ptr(bm), ord(r), 0.0, v.ctypes.data,
+                          m.ctypes.data, flags.ctypes.data, n, h, w, device)
+                for g, x in zip((v, m, flags), want[2:] + (want_flags,)):
+                    same(u8(g), u8(x))
+                o_img, v, m, flags = np.empty_like(img), np.empty_like(a), np.empty((n, h, w), np.bool_), \
+                    np.full((n, 2), -1, np.int32)
+                _lib.call('ofh_apply_combine3', img.ctypes.data, _ops.dtype_code(img.dtype), 3, arith, rule,
+                          a.ctypes.data, ptr(am), b.ctypes.data, ptr(bm), ord(r), 0.0, o_img.ctypes.data, None,
+                          v.ctypes.data, m.ctypes.data, flags.ctypes.data, n, h, w, device)
+                for g, x in zip((o_img, v, m, flags), (want[0],) + want[2:] + (want_flags,)):
+                    same(u8(g), u8(x))
+        _lib.call('ofh_release')                              # the next size starts from a fresh ring
+
+
 def test_torch_cuda_tensors_pass_through_zero_copy(of):
     """Optional PyTorch interop (north star): torch.cuda tensors are adopted through __cuda_array_interface__ without
     a copy -- as flow vectors / masks of Flow and FlowBatch -- and results are exported the same way."""
