@@ -184,12 +184,12 @@ int ofk_resize_flow(const float* vecs, const uint8_t* mask, float* out_vecs, uin
 /* out[i] = v[i] > thr (the `> .99` mask test of combine_with mode 2 / ref 't', flow_class.py:1410). */
 int ofk_greater(const float* v, float thr, uint8_t* out, size_t n, ofk_stream_t stream);
 
-/* Flow.visualise (flow_class.py:869-951), one frame per call.
+/* Flow.visualise (flow_class.py:869-951), one frame per call (the N = 1 case of ofk_visualise_batch's kernels).
  * ofk_vis_magnitude: mag[p] = magnitude of threshold_vectors(flow)[p] as cv2.cartToPolar computes it (float32);
  *   *max_out (device float) receives the maximum.
- * ofk_kth_smallest: exact order statistics of a NON-NEGATIVE float32 device array: out[q] (device) = the element of
- *   rank ranks_host[q] (0-based, host array, 1 <= n_ranks <= 4) in sorted order -- the values numpy.percentile
- *   interpolates between. ws: device workspace of ofk_kth_smallest_workspace(n_ranks) bytes.
+ * ofk_kth_smallest: exact order statistics of a NON-NEGATIVE float32 device array of n < 2^32 values: out[q] (device)
+ *   = the element of rank ranks_host[q] (0-based, host array, 1 <= n_ranks <= 4) in sorted order -- the values
+ *   numpy.percentile interpolates between. ws: device workspace of ofk_kth_smallest_workspace(n_ranks) bytes.
  * ofk_visualise: out uint8 [H,W,3]; mode 0 'hsv', 1 'rgb', 2 'bgr'; range_max = magnitude mapped to full saturation
  *   (the caller derives it from the 99th percentile / maximum as the reference does); mask may be NULL (all valid). */
 int ofk_vis_magnitude(const float* flow, float thr, float* mag, float* max_out, size_t n_pixels, ofk_stream_t stream);
@@ -198,6 +198,18 @@ int ofk_kth_smallest(const float* values, size_t n, const unsigned long long* ra
                      void* ws, size_t ws_bytes, ofk_stream_t stream);
 int ofk_visualise(const float* flow, const uint8_t* mask, float thr, int mode, int show_mask, int show_mask_borders,
                   float range_max, uint8_t* out, int H, int W, ofk_stream_t stream);
+
+/* Flow.visualise of N frames: frame n of out equals Flow(flow[n], ref, mask[n]).visualise(mode, show_mask,
+ * show_mask_borders, range_max). range_max > 0: that range for every frame; range_max == 0: the reference's default per
+ * frame, resolved on the device (numpy's float32 percentile(mag, 99) over all H*W magnitudes, mask ignored; if that is
+ * 0 the maximum, if that is 0 too then 1); < 0 or NaN: OFK_EINVAL. mask NULL = all valid. mode 0 hsv, 1 rgb, 2 bgr.
+ * out uint8 [N,H,W,3]. ws: ofk_visualise_batch_workspace(N,H,W) bytes, 4-byte aligned (256-byte aligned keeps the
+ * loads of each frame's magnitudes aligned), N times a per-frame amount (0 is fine when range_max > 0). A fixed number
+ * of launches whatever N (the frame index is folded into grid x, so N is not limited to 65535); H*W < 2^31. */
+size_t ofk_visualise_batch_workspace(int N, int H, int W);
+int ofk_visualise_batch(const float* flow, const uint8_t* mask, float thr, int mode, int show_mask,
+                        int show_mask_borders, float range_max, uint8_t* out, int N, int H, int W, void* ws,
+                        size_t ws_bytes, ofk_stream_t stream);
 
 /* Point tracking through an 's' flow with float points: replaces bilinear_interpolation + `pts + flow_vecs`
  * (utils.py:161-196,605,608). flow [H,W,2] (one frame), pts float64 [n][2] (row, col); out float64 [n][2];
@@ -304,6 +316,10 @@ int ofh_combine3(const float* A, const uint8_t* Am, const float* B, const uint8_
 int ofh_apply_combine3(const void* image, int dtype, int C, int arith, int mask_rule, const float* A, const uint8_t* Am,
                        const float* B, const uint8_t* Bm, int ref, float thr, void* out_image, uint8_t* out_valid,
                        float* out, uint8_t* out_mask, int* flags, int N, int H, int W, int device);
+/* ofk_visualise_batch on host buffers (flow [N,H,W,2], mask [N,H,W] or NULL, out uint8 [N,H,W,3]) through the ring;
+ * synchronous. */
+int ofh_visualise(const float* flow, const uint8_t* mask, float thr, int mode, int show_mask, int show_mask_borders,
+                  float range_max, uint8_t* out, int N, int H, int W, int device);
 /* All ofh_* calls leave the caller's current CUDA device unchanged. */
 /* release the internal ring (also done at process exit) */
 int ofh_release(void);

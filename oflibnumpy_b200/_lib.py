@@ -44,6 +44,8 @@ _SIGNATURES = {
     'ofk_kth_smallest_workspace': (_sz, [_i]),
     'ofk_kth_smallest': (_i, [_vp, _sz, _vp, _i, _vp, _vp, _sz, _vp]),
     'ofk_visualise': (_i, [_vp, _vp, _f, _i, _i, _i, _f, _vp, _i, _i, _vp]),
+    'ofk_visualise_batch_workspace': (_sz, [_i, _i, _i]),
+    'ofk_visualise_batch': (_i, [_vp, _vp, _f, _i, _i, _i, _f, _vp, _i, _i, _i, _vp, _sz, _vp]),
     'ofk_track_bilinear': (_i, [_vp, _vp, _sz, _i, _i, _vp, _vp, _vp]),
     'ofk_points_inside_area': (_i, [_vp, _sz, _i, _i, _vp, _vp]),
     'ofk_forward_s_workspace': (_sz, [_i, _i, _i]),
@@ -59,6 +61,7 @@ _SIGNATURES = {
     'ofh_warp_t': (_i, [_vp, _i, _i, _i, _vp, _f, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i]),
     'ofh_combine3': (_i, [_vp, _vp, _vp, _vp, _i, _f, _vp, _vp, _vp, _i, _i, _i, _i]),
     'ofh_apply_combine3': (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _f, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i]),
+    'ofh_visualise': (_i, [_vp, _vp, _f, _i, _i, _i, _f, _vp, _i, _i, _i, _i]),
     'ofh_release': (_i, []),
     'ofk_rt_device_count': (_i, [C.POINTER(_i)]),
     'ofk_rt_set_device': (_i, [_i]),
@@ -88,7 +91,8 @@ _SIGNATURES = {
     'ofk_rt_path_count': (C.c_ulonglong, [C.c_int]),
 }
 
-_NO_CHECK = {'ofk_last_error', 'ofk_version', 'ofk_forward_s_workspace', 'ofk_combine12_workspace', 'ofk_kth_smallest_workspace', 'ofk_rt_launch_count', 'ofk_rt_path_count'}
+_NO_CHECK = {'ofk_last_error', 'ofk_version', 'ofk_forward_s_workspace', 'ofk_combine12_workspace', 'ofk_kth_smallest_workspace',
+             'ofk_visualise_batch_workspace', 'ofk_rt_launch_count', 'ofk_rt_path_count'}
 
 _lib = None
 

@@ -228,6 +228,31 @@ def visualise(flow, mask, mode, show_mask, show_mask_borders, range_max, thr):
     return out.numpy()
 
 
+def vis_range_arg(range_max):
+    """The range_max argument of ofk_visualise_batch / ofh_visualise: 0 for None (each frame's default range, found
+    on the device), else the float32 value. A positive range that float32 cannot hold (rounds to 0) becomes -1, which
+    the library rejects as ofk_visualise rejects it, instead of silently taking the default range."""
+    if range_max is None:
+        return 0.0
+    r = float(np.float32(range_max))
+    return r if r != 0 else -1.0
+
+
+def visualise_batch(flow, mask, mode_code, show_mask, show_mask_borders, range_max, thr):
+    """Flow.visualise of every frame in one ofk_visualise_batch call: flow [N,H,W,2], mask [N,H,W] or None. With
+    range_max None the default range of each frame is found on the device (no read-back). Returns a device uint8
+    [N,H,W,3] array; asynchronous."""
+    n, h, w = flow.shape[:3]
+    out = DeviceArray.empty((n, h, w, 3), np.uint8)
+    ws, ws_bytes = None, 0
+    if range_max is None:
+        ws_bytes = _lib.call('ofk_visualise_batch_workspace', n, h, w)
+        ws = DeviceArray.empty((max(ws_bytes, 16),), np.uint8)
+    _lib.call('ofk_visualise_batch', flow.ptr, _p(mask), float(thr), mode_code, int(show_mask), int(show_mask_borders),
+              vis_range_arg(range_max), out.ptr, n, h, w, _p(ws), ws_bytes, dev.current_stream())
+    return out
+
+
 def points_inside_area(pts, shape):
     p = np.ascontiguousarray(pts, dtype=np.float64)
     d = DeviceArray.from_numpy(p)

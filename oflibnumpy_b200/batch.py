@@ -11,9 +11,11 @@ from . import _ops
 from . import device as dev
 from .device import DeviceArray
 from .flow import Flow
-from .validation import get_valid_ref, validate_shape, validate_transform_list, DEFAULT_THRESHOLD
+from .validation import get_valid_ref, validate_shape, validate_transform_list, validate_visualise_args, \
+    DEFAULT_THRESHOLD
 
-__all__ = ['FlowBatch', 'shard_range', 'apply_flow_host', 'combine_flows_host', 'apply_combine_host']
+__all__ = ['FlowBatch', 'shard_range', 'apply_flow_host', 'combine_flows_host', 'apply_combine_host',
+           'visualise_flows_host']
 
 
 def shard_range(n, rank, world):
@@ -247,6 +249,15 @@ class FlowBatch(object):
             return FlowBatch._wrap(out, 's', omask)
         return FlowBatch._wrap(self._negated(), 's', self.masks).switch_ref()
 
+    def visualise(self, mode, show_mask=None, show_mask_borders=None, range_max=None):
+        """Frame-wise ``Flow.visualise`` (flow_class.py:869-951) in one ofk_visualise_batch call: frame ``i`` is
+        ``self[i].visualise(mode, show_mask, show_mask_borders, range_max)``, bit for bit. The default range of each
+        frame (99th percentile of its magnitudes, else the maximum, else 1) is found on the device: no synchronisation,
+        no read-back. Returns a device uint8 array (N,H,W,3) (``.numpy()`` to download)."""
+        code, show_mask, show_mask_borders = validate_visualise_args(mode, show_mask, show_mask_borders, range_max)
+        return _ops.visualise_batch(self.vecs, self.masks, code, show_mask, show_mask_borders, range_max,
+                                    DEFAULT_THRESHOLD)
+
 
 # ---------------------------------------------------------------------------------------------------- host-buffer calls
 def _c(a, dtype=None):
@@ -383,3 +394,29 @@ def apply_combine_host(flows_1, flows_2, images, ref='t', masks_1=None, masks_2=
               DEFAULT_THRESHOLD if thresholded else 0.0, out_images.ctypes.data, out_valid.ctypes.data, out.ctypes.data,
               out_masks.ctypes.data, flags.ctypes.data, n, h, w, device)
     return out_images, out_valid, out, out_masks
+
+
+def visualise_flows_host(flows, mode, masks=None, show_mask=False, show_mask_borders=False, range_max=None, out=None,
+                         device=None):
+    """Batched ``Flow(flows[i], 't', masks[i]).visualise(mode, show_mask, show_mask_borders, range_max)`` on HOST
+    arrays through ofh_visualise: frames stream through the device ring, copies overlap the kernels, the default range
+    of each frame is found on the device. Pass pinned arrays (device.pinned_empty) for full-rate copies. Returns a
+    numpy uint8 array (N,H,W,3)."""
+    code, show_mask, show_mask_borders = validate_visualise_args(mode, show_mask, show_mask_borders, range_max)
+    flows = _c(flows, np.float32)
+    if flows.ndim != 4 or flows.shape[3] != 2:
+        raise ValueError("Error visualising flow: flows need shape (N,H,W,2)")
+    n, h, w = flows.shape[:3]
+    if masks is not None:
+        masks = _c(masks, np.bool_)
+        if masks.shape != (n, h, w):
+            raise ValueError("Error setting flow mask: Input has a different shape than the flow vectors")
+    if out is None:
+        out = np.empty((n, h, w, 3), np.uint8)
+    else:
+        _check_out(out, (n, h, w, 3), np.uint8, 'out')
+    device = dev.get_device() if device is None else device
+    _lib.call('ofh_visualise', flows.ctypes.data, None if masks is None else masks.ctypes.data, DEFAULT_THRESHOLD,
+              code, int(show_mask), int(show_mask_borders), _ops.vis_range_arg(range_max), out.ctypes.data, n, h, w,
+              device)
+    return out

@@ -498,6 +498,28 @@ extern "C" int ofh_apply_combine3(const void* image, int dtype, int C, int arith
         });
 }
 
+// Flow.visualise of N host frames: with the default range (range_max == 0) each chunk carries the magnitudes and
+// selection records of ofk_visualise_batch as a per-frame buffer that is never copied.
+extern "C" int ofh_visualise(const float* flow, const uint8_t* mask, float thr, int mode, int show_mask,
+                             int show_mask_borders, float range_max, uint8_t* out, int N, int H, int W, int device) {
+    OFK_CHECK_ARG(flow && out && N >= 0 && H > 0 && W > 0, "ofh_visualise: bad arguments");
+    OFK_CHECK_ARG((size_t)H * W < (1ull << 31), "ofh_visualise: a frame needs fewer than 2^31 pixels");
+    OFK_CHECK_ARG(mode >= 0 && mode <= 2, "ofh_visualise: mode must be 0 (hsv), 1 (rgb) or 2 (bgr)");
+    OFK_CHECK_ARG(range_max >= 0.f, "ofh_visualise: range_max must be positive, or 0 for the default range");
+    const size_t px = (size_t)H * W, b_ws = range_max > 0.f ? 0 : ofk_visualise_batch_workspace(1, H, W);
+    enum { kFlow, kMask, kOut, kWs };
+    return run_ring(
+        device, N, {px * 8, mask ? px : 0, px * 3, b_ws}, nullptr,
+        [&](const Chunk& c) {
+            OFH_TRY(c.in(kFlow, flow));
+            OFH_TRY(c.in(kMask, mask));
+            return ofk_visualise_batch(c.at<float>(kFlow), c.at<uint8_t>(kMask), thr, mode, show_mask,
+                                       show_mask_borders, range_max, c.at<uint8_t>(kOut), c.cn, H, W, c.at(kWs),
+                                       b_ws * c.cn, c.stream());
+        },
+        [&](const Chunk& c) { return c.out(out, kOut); });
+}
+
 extern "C" int ofh_release(void) {
     std::lock_guard<std::mutex> lk(g_ring.mu);
     DeviceGuard restore_device;

@@ -16,7 +16,7 @@ from . import _lib
 from . import _ops
 from . import device as dev
 from .device import DeviceArray
-from .validation import get_valid_ref, get_valid_padding, validate_shape, DEFAULT_THRESHOLD
+from .validation import get_valid_ref, get_valid_padding, validate_shape, validate_visualise_args, DEFAULT_THRESHOLD
 
 __all__ = ['Flow']
 
@@ -595,19 +595,7 @@ class Flow(object):
         """Flow as an rgb / bgr / hsv image (flow_class.py:869-951): hue = direction, saturation = magnitude scaled to
         `range_max` (default: 99th percentile of the magnitudes, found by radix selection on the device), optionally
         invalid areas greyed out and the mask outline in black. Returns a numpy uint8 array (H, W, 3)."""
-        show_mask = False if show_mask is None else show_mask
-        show_mask_borders = False if show_mask_borders is None else show_mask_borders
-        if not isinstance(show_mask, bool):
-            raise TypeError("Error visualising flow: Show_mask needs to be boolean")
-        if not isinstance(show_mask_borders, bool):
-            raise TypeError("Error visualising flow: Show_mask_borders needs to be boolean")
-        if range_max is not None:
-            if not isinstance(range_max, (float, int)):
-                raise TypeError("Error visualising flow: Range_max needs to be an integer or a float")
-            if range_max <= 0:
-                raise ValueError("Error visualising flow: Range_max needs to be larger than zero")
-        if mode not in ('hsv', 'rgb', 'bgr'):
-            raise ValueError("Error visualising flow: Mode needs to be either 'bgr', 'rgb', or 'hsv'")
+        _, show_mask, show_mask_borders = validate_visualise_args(mode, show_mask, show_mask_borders, range_max)
         return _ops.visualise(self._vd(), self._md(), mode, show_mask, show_mask_borders, range_max, DEFAULT_THRESHOLD)
 
     # ---- host-side presentation / estimation (SURVEY section 2 rows 19-20: not on the hot path, delegated)

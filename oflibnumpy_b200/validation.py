@@ -55,6 +55,28 @@ def validate_flow_array(flow, error_string=None, finite_on_device=False):
     return np.ascontiguousarray(flow, dtype=np.float32)
 
 
+VIS_MODES = {'hsv': 0, 'rgb': 1, 'bgr': 2}
+
+
+def validate_visualise_args(mode, show_mask, show_mask_borders, range_max):
+    """Checks of Flow.visualise (flow_class.py:893-905), shared by Flow.visualise, FlowBatch.visualise and
+    batch.visualise_flows_host. Returns (mode code, show_mask, show_mask_borders); None stands for False."""
+    show_mask = False if show_mask is None else show_mask
+    show_mask_borders = False if show_mask_borders is None else show_mask_borders
+    if not isinstance(show_mask, bool):
+        raise TypeError("Error visualising flow: Show_mask needs to be boolean")
+    if not isinstance(show_mask_borders, bool):
+        raise TypeError("Error visualising flow: Show_mask_borders needs to be boolean")
+    if range_max is not None:
+        if not isinstance(range_max, (float, int)):
+            raise TypeError("Error visualising flow: Range_max needs to be an integer or a float")
+        if range_max <= 0:
+            raise ValueError("Error visualising flow: Range_max needs to be larger than zero")
+    if mode not in ('hsv', 'rgb', 'bgr'):                    # a tuple: an unhashable mode raises ValueError too
+        raise ValueError("Error visualising flow: Mode needs to be either 'bgr', 'rgb', or 'hsv'")
+    return VIS_MODES[mode], show_mask, show_mask_borders
+
+
 def validate_transform_list(transform_list):
     """Checks of from_transforms (utils.py:363-388)."""
     pre = "Error creating flow from transforms: "
