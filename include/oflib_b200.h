@@ -50,6 +50,9 @@ extern "C" {
 #define OFK_U16 2
 #define OFK_F32 3
 #define OFK_F64 4
+/* point element types of ofk_track (besides OFK_F32 / OFK_F64) */
+#define OFK_I32 5
+#define OFK_I64 6
 
 /* interpolation arithmetic (OpenCV picks it from the dtype of the array handed to cv2.remap, which for Flow.apply is
  * the numpy promotion of payload||mask -- flow_class.py:615,644):
@@ -216,6 +219,29 @@ int ofk_visualise_batch(const float* flow, const uint8_t* mask, float thr, int m
  * bad (int32, device) is set to 1 if any point lies outside the flow area (the reference raises IndexError). */
 int ofk_track_bilinear(const float* flow, const double* pts, size_t n, int H, int W, double* out, int* bad,
                        ofk_stream_t stream);
+
+/* Flow.track (flow_class.py:755-795, utils.py:547-622) of N frames in one call: frame n of the outputs equals
+ * Flow(flow[n], ref, mask[n]).track(pts_n, int_out, get_valid_status, exact), bit for bit.
+ *   flow [N,H,W,2]; mask [N,H,W] or NULL (all valid), read for ref 's' status only; ref 's' or 't'.
+ *   exact != 0: s_exact_mode (ref 's' float points only: Flow.track looks integer points up whatever the mode).
+ *   flow_nonzero int32 [N] (device, ofk_nonzero_flags(flow, NULL, 1e-3)): frames with 0 pass their points through.
+ *   pts [N,P,2] (pts_shared = 0) or [P,2] for every frame (pts_shared != 0), (row, col), of pts_dtype OFK_F32, OFK_F64,
+ *     OFK_I32 or OFK_I64. Routes: ref 's' integer points look the vector up (numpy indexing: an index in [-H,-1] wraps),
+ *     ref 's' float points interpolate it bilinearly in float64, or with exact locate the point in the mesh of
+ *     ofk_mesh_sample on the undisplaced grid; ref 't' locates it in the mesh p - flow[p].
+ *   arith OFK_F32 or OFK_F64: the type of `pts + vector` (numpy's result type; OFK_F32 only for integer points on an
+ *     's' flow, i.e. numpy's int8/int16/uint8/uint16 points). out [N,P,2] of that type, or int32 with int_out != 0
+ *     (round half to even).
+ *   status uint8 [N,P] or NULL: valid_source at the rounded point, computed from flow and mask for ref 's' and gathered
+ *     from status_plane [N,H,W] (the valid_source plane) for ref 't'.
+ *   errors int32 [N] (device; the call zeroes it): bit 1 a float point on an 's' flow outside [0,H-1]x[0,W-1], bit 2 an
+ *     integer point on an 's' flow outside [-H,H-1]x[-W,W-1] (both only where flow_nonzero is set), bit 4 a rounded point
+ *     outside [-H,H-1]x[-W,W-1] with status. The reference raises IndexError in these cases; the call itself succeeds.
+ * One kernel launch whatever N (the frame is folded into the point index). The mesh routes need H, W >= 2 and
+ * H*W < 2^30. */
+int ofk_track(const float* flow, const uint8_t* mask, int ref, int exact, const int* flow_nonzero, const void* pts,
+              int pts_dtype, int pts_shared, int P, int arith, int int_out, void* out, const uint8_t* status_plane,
+              uint8_t* status, int* errors, int N, int H, int W, ofk_stream_t stream);
 
 /* points_inside_area (utils.py:283-295): pts float64 [n][2] (row, col) rounded half-even like numpy.round. */
 int ofk_points_inside_area(const double* pts, size_t n, int H, int W, uint8_t* out, ofk_stream_t stream);

@@ -6,7 +6,7 @@ import os
 from . import build as _build
 
 # enums of include/oflib_b200.h
-U8, I16, U16, F32, F64 = 0, 1, 2, 3, 4
+U8, I16, U16, F32, F64, I32, I64 = 0, 1, 2, 3, 4, 5, 6
 ARITH_NATIVE, ARITH_RINT = 0, 1
 RULE_STRICT, RULE_GT_HALF, RULE_GE_HALF = 0, 1, 2
 OP_ADD, OP_SUB, OP_MUL, OP_DIV, OP_POW = 0, 1, 2, 3, 4
@@ -47,6 +47,7 @@ _SIGNATURES = {
     'ofk_visualise_batch_workspace': (_sz, [_i, _i, _i]),
     'ofk_visualise_batch': (_i, [_vp, _vp, _f, _i, _i, _i, _f, _vp, _i, _i, _i, _vp, _sz, _vp]),
     'ofk_track_bilinear': (_i, [_vp, _vp, _sz, _i, _i, _vp, _vp, _vp]),
+    'ofk_track': (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
     'ofk_points_inside_area': (_i, [_vp, _sz, _i, _i, _vp, _vp]),
     'ofk_forward_s_workspace': (_sz, [_i, _i, _i]),
     'ofk_forward_s': (_i, [_vp, _i, _vp, _f, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _sz, _vp]),

@@ -347,6 +347,25 @@ def track_bilinear(flow, pts):
     return out.numpy(), bool(bad.numpy()[0])
 
 
+TRACK_PTS_CODES = {np.dtype('float32'): _lib.F32, np.dtype('float64'): _lib.F64, np.dtype('int32'): _lib.I32,
+                   np.dtype('int64'): _lib.I64}
+
+
+def track(flow, mask, ref, exact, flow_nonzero, pts, arith_dtype, int_out, status_plane=None, want_status=False):
+    """Flow.track of every frame in one ofk_track call: flow [N,H,W,2], pts device [N,P,2] or [P,2] of a
+    TRACK_PTS_CODES dtype. Returns device arrays (tracked [N,P,2] of arith_dtype or int32, status uint8 [N,P] or None,
+    error words int32 [N]); asynchronous."""
+    n, h, w = flow.shape[:3]
+    p = pts.shape[-2]
+    out = DeviceArray.empty((n, p, 2), np.int32 if int_out else arith_dtype)
+    status = DeviceArray.empty((n, p), np.uint8) if want_status else None
+    errors = DeviceArray.empty((n,), np.int32)
+    _lib.call('ofk_track', flow.ptr, _p(mask), ord(ref), int(exact), flow_nonzero.ptr, pts.ptr,
+              TRACK_PTS_CODES[pts.dtype], int(pts.ndim == 2), p, DTYPE_CODES[np.dtype(arith_dtype)], int(int_out),
+              out.ptr, _p(status_plane), _p(status), errors.ptr, n, h, w, dev.current_stream())
+    return out, status, errors
+
+
 def resize_flow(vecs, mask, fy, fx):
     """cv2.resize semantics: output size = round-half-even(size * scale) (ofk_resize_flow)."""
     n, h, w = (vecs if vecs is not None else mask).shape[:3]

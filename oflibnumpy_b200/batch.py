@@ -12,7 +12,7 @@ from . import device as dev
 from .device import DeviceArray
 from .flow import Flow
 from .validation import get_valid_ref, validate_shape, validate_transform_list, validate_visualise_args, \
-    DEFAULT_THRESHOLD
+    validate_track_args, validate_track_dtype, DEFAULT_THRESHOLD
 
 __all__ = ['FlowBatch', 'shard_range', 'apply_flow_host', 'combine_flows_host', 'apply_combine_host',
            'visualise_flows_host']
@@ -257,6 +257,88 @@ class FlowBatch(object):
         code, show_mask, show_mask_borders = validate_visualise_args(mode, show_mask, show_mask_borders, range_max)
         return _ops.visualise_batch(self.vecs, self.masks, code, show_mask, show_mask_borders, range_max,
                                     DEFAULT_THRESHOLD)
+
+    def track(self, pts, int_out=None, get_valid_status=None, s_exact_mode=None):
+        """Frame-wise ``Flow.track`` (flow_class.py:755-795) in one ofk_track call. ``pts`` (row, col) is (N,P,2), frame
+        ``i`` using ``pts[i]``, or (P,2), the same points in every frame; a numpy array or a device array
+        (``DeviceArray``, any ``__cuda_array_interface__`` exporter such as a torch.cuda tensor; float32, float64, int32
+        or int64). Frame ``i`` of the result is ``self[i].track(pts_i, int_out, False, s_exact_mode)`` bit for bit, in
+        the dtype ``Flow.track`` gives a frame with non-zero flow (integer points on an 's' flow:
+        ``np.result_type(pts.dtype, np.float32)``; otherwise float64; int32 with ``int_out``). Frames whose flow is zero
+        below the threshold hold their points converted to that dtype.
+
+        Returns a device array (N,P,2), and with ``get_valid_status`` also a device uint8 (N,P) of 0/1, the status
+        ``self[i].track(pts_i, get_valid_status=True)`` returns (``.numpy()`` to download, ``.view(bool)`` for numpy's
+        type). Ref 't' status reads the batch's valid_source plane (one forward resampling per frame).
+
+        Raises IndexError where a loop of ``Flow.track`` would, for the lowest such frame. Host points are range-tested
+        in numpy first: when they all pass, the call returns without synchronising. Otherwise, and always for device
+        points, the per-frame error words of the kernel are read back, which synchronises with the device."""
+        host = isinstance(pts, np.ndarray)
+        if not host and dev.is_device_array(pts):
+            pts = dev.as_device(pts)
+        n, (h, w) = len(self), self.shape
+        int_out, get_valid_status, s_exact_mode = validate_track_args(pts, int_out, get_valid_status, s_exact_mode, n)
+        validate_track_dtype(pts.dtype)
+        is_int = np.issubdtype(pts.dtype, np.integer)
+        lookup = self.ref == 's' and (is_int or not s_exact_mode)        # Flow.track looks integer points up
+        arith = np.result_type(pts.dtype, np.float32) if lookup and is_int else np.dtype(np.float64)
+        if host:
+            if pts.dtype not in _ops.TRACK_PTS_CODES:           # int8 ... uint16 -> int32 (arith float32 if lookup)
+                pts = pts.astype(np.int32 if is_int and pts.dtype.itemsize < 4 else
+                                 (np.int64 if is_int else np.float64))
+            bad = _track_range_fails(pts, lookup, is_int, get_valid_status, h, w)
+            dpts = DeviceArray.from_numpy(pts)
+        else:
+            if pts.dtype not in _ops.TRACK_PTS_CODES:
+                raise TypeError("Error tracking points: device points need dtype float32, float64, int32 or int64, not "
+                                "{}".format(pts.dtype))
+            bad, dpts = True, pts
+        p = pts.shape[-2]
+        if n == 0 or p == 0:
+            out = DeviceArray.empty((n, p, 2), np.int32 if int_out else arith)
+            return (out, DeviceArray.empty((n, p), np.uint8)) if get_valid_status else out
+        plane = self.valid_source() if get_valid_status and self.ref == 't' else None
+        out, status, errors = _ops.track(self.vecs, self.masks, self.ref, s_exact_mode, self._zero_flags(), dpts,
+                                         arith, int_out, plane, get_valid_status)
+        if bad:
+            _raise_track_error(errors.numpy(), h, w)
+        return (out, status) if get_valid_status else out
+
+
+def _track_range_fails(pts, lookup, is_int, status, h, w):
+    """True if a host point fails a range test of Flow.track (the tests ofk_track repeats per frame), which only
+    depend on the points and the frame size: float points on an 's' flow outside [0,H-1]x[0,W-1], integer points on an
+    's' flow outside [-H,H-1]x[-W,W-1], and with status the rounded points outside that range."""
+    r, c = pts[..., 0], pts[..., 1]
+    if lookup and is_int:
+        fails = (r < -h) | (r >= h) | (c < -w) | (c >= w)
+    elif lookup:
+        r, c = r.astype(np.float64), c.astype(np.float64)
+        fails = ~((0 <= r) & (r <= h - 1) & (0 <= c) & (c <= w - 1))
+    else:
+        fails = np.zeros(r.shape, bool)
+    if status:
+        with np.errstate(invalid='ignore'):                   # NaN and huge values become INT_MIN, as in Flow.track
+            ri, ci = np.round(r).astype('i'), np.round(c).astype('i')
+        fails |= (ri < -h) | (ri >= h) | (ci < -w) | (ci >= w)
+    return bool(fails.any())
+
+
+def _raise_track_error(errors, h, w):
+    """Raises the IndexError of the lowest frame whose error word (ofk_track) is set, as a loop of Flow.track would."""
+    flagged = np.flatnonzero(errors)
+    if flagged.size == 0:
+        return
+    i = int(flagged[0])
+    e = int(errors[i])
+    if e & 1:
+        raise IndexError("Some points are outside of the data area.")
+    if e & 2:
+        raise IndexError("Error tracking points: Pts of frame {} index outside of the flow field of shape {}".format(
+            i, (h, w)))
+    raise IndexError("Error tracking points: Rounded pts of frame {} for the valid status lie outside of the flow "
+                     "field of shape {}".format(i, (h, w)))
 
 
 # ---------------------------------------------------------------------------------------------------- host-buffer calls

@@ -7,6 +7,7 @@
 #include <algorithm>
 
 #include "ofk_common.cuh"
+#include "track_device.cuh"
 
 namespace ofk {
 
@@ -286,34 +287,17 @@ __global__ void __launch_bounds__(256) greater_kernel(const float* __restrict__ 
         out[i] = v[i] > thr ? 1 : 0;
 }
 
-// Flow vectors at float64 points (row, col) by exact bilinear interpolation with clipped neighbours, float64
-// arithmetic in the reference's operation order (utils.py:161-196); out = pts + (v, u). bad[0] is set when a point
-// lies outside [0,H-1]x[0,W-1] (the reference raises IndexError).
+// Flow vectors at float64 points (row, col) by exact bilinear interpolation (bilinear_track_point); out = pts + (v, u).
+// bad[0] is set when a point lies outside [0,H-1]x[0,W-1] (the reference raises IndexError).
 __global__ void __launch_bounds__(128) track_bilinear_kernel(const float* __restrict__ flow, const double* __restrict__ pts,
                                                              size_t n, int H, int W, double* __restrict__ out,
                                                              int* __restrict__ bad) {
     const float2* f = reinterpret_cast<const float2*>(flow);
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
-        const double r = pts[i * 2], c = pts[i * 2 + 1];
-        if (!(0 <= r && r <= H - 1) || !(0 <= c && c <= W - 1)) {
+        if (!bilinear_track_point(f, H, W, pts[i * 2], pts[i * 2 + 1], out[i * 2], out[i * 2 + 1])) {
             *bad = 1;
             out[i * 2] = out[i * 2 + 1] = 0.0;
-            continue;
         }
-        const int r0 = (int)floor(r), c0 = (int)floor(c);
-        const int r0c = min(max(r0, 0), H - 1), c0c = min(max(c0, 0), W - 1);
-        const int r1c = min(max(r0 + 1, 0), H - 1), c1c = min(max(c0 + 1, 0), W - 1);
-        const double wa = __dmul_rn((double)r1c - r, (double)c1c - c), wb = __dmul_rn((double)r1c - r, c - (double)c0c);
-        const double wc = __dmul_rn(r - (double)r0c, (double)c1c - c), wd = __dmul_rn(r - (double)r0c, c - (double)c0c);
-        const float2 a = f[(size_t)r0c * W + c0c], b = f[(size_t)r1c * W + c0c], cc = f[(size_t)r0c * W + c1c],
-                     d = f[(size_t)r1c * W + c1c];
-        // result = wa*data_a + wb*data_b + wc*data_c + wd*data_d, data in (v, u) order, no FMA contraction
-        const double dv = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(wa, (double)a.y), __dmul_rn(wb, (double)b.y)),
-                                              __dmul_rn(wc, (double)cc.y)), __dmul_rn(wd, (double)d.y));
-        const double du = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(wa, (double)a.x), __dmul_rn(wb, (double)b.x)),
-                                              __dmul_rn(wc, (double)cc.x)), __dmul_rn(wd, (double)d.x));
-        out[i * 2] = __dadd_rn(r, dv);
-        out[i * 2 + 1] = __dadd_rn(c, du);
     }
 }
 

@@ -29,6 +29,7 @@
 
 #include "ofk_common.cuh"
 #include "forward_irregular.cuh"
+#include "track_device.cuh"
 
 // ============================================================ order-independent resolve for folding fields (round 1)
 namespace ofk {
@@ -2201,6 +2202,48 @@ __device__ bool locate_in_cell(const float2* __restrict__ fl, int H, int W, floa
     return false;
 }
 
+// The triangle of the mesh p + sign * fl[p] that contains the query (qx, qy): a fixed-point walk towards the source
+// position, then an exact containment search in the rings of cells around it. On success fills the three vertex indices
+// and the barycentric weights.
+__device__ __forceinline__ bool mesh_locate(const float2* __restrict__ fl, int H, int W, float mesh_sign, int pos_f32,
+                                            double qx, double qy, int (&vidx)[3], double (&w)[3], double flip_tol) {
+    // fixed-point walk towards the source position p with p + sign*flow(p) = q (bilinear flow lookup, clamped)
+    double px = qx, py = qy;
+    for (int it = 0; it < 12; ++it) {
+        const double cx = fmin(fmax(px, 0.0), (double)(W - 1)), cy = fmin(fmax(py, 0.0), (double)(H - 1));
+        const int j0 = min((int)cx, W - 2 < 0 ? 0 : W - 2), i0 = min((int)cy, H - 2 < 0 ? 0 : H - 2);
+        const double a = cx - j0, b = cy - i0;
+        const int j1 = min(j0 + 1, W - 1), i1 = min(i0 + 1, H - 1);
+        const float2 f00 = __ldg(fl + i0 * W + j0), f01 = __ldg(fl + i0 * W + j1), f10 = __ldg(fl + i1 * W + j0),
+                     f11 = __ldg(fl + i1 * W + j1);
+        const double u = (1 - b) * ((1 - a) * f00.x + a * f01.x) + b * ((1 - a) * f10.x + a * f11.x);
+        const double v = (1 - b) * ((1 - a) * f00.y + a * f01.y) + b * ((1 - a) * f10.y + a * f11.y);
+        const double nx = qx - mesh_sign * u, ny = qy - mesh_sign * v;
+        const bool done = fabs(nx - px) < 1e-3 && fabs(ny - py) < 1e-3;
+        px = nx;
+        py = ny;
+        if (done) break;
+    }
+    bool hit = false;
+    const int ci = (int)floor(py), cj = (int)floor(px);
+    for (int ring = 0; ring <= 2 && !hit; ++ring) {
+        for (int di = -ring; di <= ring && !hit; ++di)
+            for (int dj = -ring; dj <= ring && !hit; ++dj) {
+                if (max(abs(di), abs(dj)) != ring) continue;
+                hit = locate_in_cell(fl, H, W, mesh_sign, pos_f32, ci + di, cj + dj, qx, qy, vidx, w, flip_tol);
+            }
+    }
+    return hit;
+}
+
+// channel c of the C-channel payload interpolated with the weights of mesh_locate
+__device__ __forceinline__ double mesh_interp(const float* __restrict__ pay, int C, const int (&vidx)[3],
+                                              const double (&w)[3], int c) {
+    return w[0] * (double)__ldg(pay + (size_t)vidx[0] * C + c) +
+           w[1] * (double)__ldg(pay + (size_t)vidx[1] * C + c) +
+           w[2] * (double)__ldg(pay + (size_t)vidx[2] * C + c);
+}
+
 __global__ void __launch_bounds__(128) mesh_sample_kernel(const float* __restrict__ mesh_flow, float mesh_sign,
                                                           int pos_f32, const float* __restrict__ payload, int C,
                                                           const uint8_t* __restrict__ payload_mask,
@@ -2231,34 +2274,9 @@ __global__ void __launch_bounds__(128) mesh_sample_kernel(const float* __restric
             qy = static_cast<double>(row) + static_cast<double>(query_sign * f.y);
         }
     }
-    // fixed-point walk towards the source position p with p + sign*flow(p) = q (bilinear flow lookup, clamped)
-    double px = qx, py = qy;
-    for (int it = 0; it < 12; ++it) {
-        const double cx = fmin(fmax(px, 0.0), (double)(W - 1)), cy = fmin(fmax(py, 0.0), (double)(H - 1));
-        const int j0 = min((int)cx, W - 2 < 0 ? 0 : W - 2), i0 = min((int)cy, H - 2 < 0 ? 0 : H - 2);
-        const double a = cx - j0, b = cy - i0;
-        const int j1 = min(j0 + 1, W - 1), i1 = min(i0 + 1, H - 1);
-        const float2 f00 = __ldg(fl + i0 * W + j0), f01 = __ldg(fl + i0 * W + j1), f10 = __ldg(fl + i1 * W + j0),
-                     f11 = __ldg(fl + i1 * W + j1);
-        const double u = (1 - b) * ((1 - a) * f00.x + a * f01.x) + b * ((1 - a) * f10.x + a * f11.x);
-        const double v = (1 - b) * ((1 - a) * f00.y + a * f01.y) + b * ((1 - a) * f10.y + a * f11.y);
-        const double nx = qx - mesh_sign * u, ny = qy - mesh_sign * v;
-        const bool done = fabs(nx - px) < 1e-3 && fabs(ny - py) < 1e-3;
-        px = nx;
-        py = ny;
-        if (done) break;
-    }
     int vidx[3];
     double w[3];
-    bool hit = false;
-    const int ci = (int)floor(py), cj = (int)floor(px);
-    for (int ring = 0; ring <= 2 && !hit; ++ring) {
-        for (int di = -ring; di <= ring && !hit; ++di)
-            for (int dj = -ring; dj <= ring && !hit; ++dj) {
-                if (max(abs(di), abs(dj)) != ring) continue;
-                hit = locate_in_cell(fl, H, W, mesh_sign, pos_f32, ci + di, cj + dj, qx, qy, vidx, w, flip_tol);
-            }
-    }
+    const bool hit = mesh_locate(fl, H, W, mesh_sign, pos_f32, qx, qy, vidx, w, flip_tol);
     const size_t o = (size_t)n * Q + k;
     if (found) found[o] = hit ? 1 : 0;
     float vals[4] = {0.f, 0.f, 0.f, 0.f};
@@ -2266,9 +2284,7 @@ __global__ void __launch_bounds__(128) mesh_sample_kernel(const float* __restric
     if (hit) {
         const float* pay = payload + fbase * C;
         for (int c = 0; c < C; ++c) {
-            const double val = w[0] * (double)__ldg(pay + (size_t)vidx[0] * C + c) +
-                               w[1] * (double)__ldg(pay + (size_t)vidx[1] * C + c) +
-                               w[2] * (double)__ldg(pay + (size_t)vidx[2] * C + c);
+            const double val = mesh_interp(pay, C, vidx, w, c);
             if (sub_from == nullptr) out[o * C + c] = (float)val;
             else vals[c & 3] = (float)val;
         }
@@ -2289,7 +2305,74 @@ __global__ void __launch_bounds__(128) mesh_sample_kernel(const float* __restric
     }
 }
 
+// ofk_track's mesh route: Flow.track for ref 't' (mesh p - flow[p]) and for float points on ref 's' with s_exact_mode
+// (mesh_sign = 0:
+// the undisplaced grid, the same vertex positions as the zero field Flow.track meshes), one thread per point of the
+// flat [N*P] index. The vector at the point is the barycentric interpolation of ofk_mesh_sample, rounded to float32 as
+// ofk_mesh_sample stores it; out = pts + (v, u) in float64, (0, 0) where no triangle contains the point (griddata's NaN
+// rows, utils.py:616-618), the points themselves in frames whose flow_nonzero is 0.
+template <typename PT>
+__global__ void __launch_bounds__(128) track_mesh_kernel(const float* __restrict__ flow,
+                                                         const uint8_t* __restrict__ mask, float mesh_sign,
+                                                         const int* __restrict__ flow_nonzero,
+                                                         const PT* __restrict__ pts, int pts_shared, int P,
+                                                         void* __restrict__ out, int int_out,
+                                                         const uint8_t* __restrict__ status_plane,
+                                                         uint8_t* __restrict__ status, int* __restrict__ errors, int H,
+                                                         int W, size_t total, double flip_tol) {
+    const size_t hw = (size_t)H * W;
+    for (size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x; k < total; k += (size_t)gridDim.x * blockDim.x) {
+        const size_t n = k / (size_t)P;
+        const size_t i = pts_shared ? k - n * P : k;
+        const PT r = pts[2 * i], c = pts[2 * i + 1];
+        const float* fn = flow + n * hw * 2;
+        const float2* fl = reinterpret_cast<const float2*>(fn);
+        if (flow_nonzero[n] == 0) {
+            store_passthrough<PT, double>(out, int_out, k, r, c);
+        } else {
+            const double qy = (double)r, qx = (double)c;
+            int vidx[3];
+            double w[3];
+            double orow = 0.0, ocol = 0.0;
+            if (mesh_locate(fl, H, W, mesh_sign, 0, qx, qy, vidx, w, flip_tol)) {
+                orow = __dadd_rn(qy, (double)(float)mesh_interp(fn, 2, vidx, w, 1));
+                ocol = __dadd_rn(qx, (double)(float)mesh_interp(fn, 2, vidx, w, 0));
+            }
+            store_tracked<double>(out, int_out, k, orow, ocol);
+        }
+        int err = 0;
+        if (status != nullptr)
+            track_status(r, c, fl, mask ? mask + n * hw : nullptr, status_plane ? status_plane + n * hw : nullptr, H, W,
+                         k, status, err);
+        if (err) atomicOr(errors + n, err);
+    }
+}
+
 }  // namespace legacy
+
+int launch_track_mesh(const float* flow, const uint8_t* mask, int ref, const int* flow_nonzero, const void* pts,
+                      int pts_dtype, int pts_shared, int P, void* out, int int_out, const uint8_t* status_plane,
+                      uint8_t* status, int* errors, int N, int H, int W, cudaStream_t st) {
+    const size_t total = (size_t)N * P;
+    const float mesh_sign = ref == 't' ? -1.0f : 0.0f;
+    const size_t blocks = std::min((total + 127) / 128, (size_t)sm_count() * 64);
+    const double tol = g_flip_tol.load();
+#define OFK_TRACK_MESH(T)                                                                                              \
+    legacy::track_mesh_kernel<T><<<(unsigned)blocks, 128, 0, st>>>(flow, mask, mesh_sign, flow_nonzero,               \
+                                                                   static_cast<const T*>(pts), pts_shared, P, out,     \
+                                                                   int_out, status_plane, status, errors, H, W, total, \
+                                                                   tol)
+    switch (pts_dtype) {
+        case OFK_F32: OFK_TRACK_MESH(float); break;
+        case OFK_F64: OFK_TRACK_MESH(double); break;
+        case OFK_I32: OFK_TRACK_MESH(int32_t); break;
+        default: OFK_TRACK_MESH(int64_t); break;
+    }
+#undef OFK_TRACK_MESH
+    OFK_LAUNCHED();
+    return OFK_OK;
+}
+
 }  // namespace ofk
 
 extern "C" int ofk_mesh_sample(const float* mesh_flow, float mesh_sign, int pos_f32, const float* payload, int C,

@@ -81,6 +81,18 @@ __device__ __forceinline__ QCoord quantise_fast(float X) {
     return q;
 }
 
+// "every tap with a non-zero weight lies inside the frame" for the sampling position (X, Y): the valid-area test of
+// valid_geom_vec4 (warp_t.cu) and of ofk_track's status (track_device.cuh).
+__device__ __forceinline__ unsigned strict_in_frame(float X, float Y, int H, int W) {
+    // clamping keeps the fast quantiser in range; a clamped coordinate is an integer outside [0, W-1] -> invalid
+    X = fminf(fmaxf(X, -2.0f), (float)(W + 1));
+    Y = fminf(fmaxf(Y, -2.0f), (float)(H + 1));
+    const QCoord qx = quantise_fast(X), qy = quantise_fast(Y);
+    const bool ok = qx.i >= 0 && qy.i >= 0 && (qx.i + 1 < W || (qx.f == 0 && qx.i < W)) &&
+                    (qy.i + 1 < H || (qy.f == 0 && qy.i < H));
+    return ok ? 1u : 0u;
+}
+
 // Absolute sampling coordinate: float32(sign*flow) + float32(grid), one rounding, as numpy's in-place
 // `field *= -1; field += arange` (utils.py:233-235).
 __device__ __forceinline__ float sample_coord(float flow_component, float sign, int grid) {

@@ -427,16 +427,6 @@ __global__ void __launch_bounds__(256) warp_t_u8x3(const uint8_t* __restrict__ p
 // valid_target (ref 't') / valid_source (ref 's'), flow_class.py:1148-1150,1179-1183: "every tap with a non-zero
 // weight lies inside the frame", AND the flow mask. Pure streaming (8 + 1 B/px in, 1 B/px out): 4 consecutive pixels
 // per thread, 2 x 16-byte flow loads, one 32-bit mask word in and out.
-__device__ __forceinline__ unsigned strict_in_frame(float X, float Y, int H, int W) {
-    // clamping keeps the fast quantiser in range; a clamped coordinate is an integer outside [0, W-1] -> invalid
-    X = fminf(fmaxf(X, -2.0f), (float)(W + 1));
-    Y = fminf(fmaxf(Y, -2.0f), (float)(H + 1));
-    const QCoord qx = quantise_fast(X), qy = quantise_fast(Y);
-    const bool ok = qx.i >= 0 && qy.i >= 0 && (qx.i + 1 < W || (qx.f == 0 && qx.i < W)) &&
-                    (qy.i + 1 < H || (qy.f == 0 && qy.i < H));
-    return ok ? 1u : 0u;
-}
-
 __global__ void __launch_bounds__(256) valid_geom_vec4(const float4* __restrict__ flow, float sign,
                                                        const uint32_t* __restrict__ fmask, uint32_t* __restrict__ out,
                                                        int H, int W, unsigned quads_per_frame) {

@@ -16,7 +16,8 @@ from . import _lib
 from . import _ops
 from . import device as dev
 from .device import DeviceArray
-from .validation import get_valid_ref, get_valid_padding, validate_shape, validate_visualise_args, DEFAULT_THRESHOLD
+from .validation import get_valid_ref, get_valid_padding, validate_shape, validate_visualise_args, \
+    validate_track_args, DEFAULT_THRESHOLD
 
 __all__ = ['Flow']
 
@@ -557,9 +558,7 @@ class Flow(object):
 
     def track(self, pts, int_out=None, get_valid_status=None, s_exact_mode=None):
         from .ops import _track_device
-        get_valid_status = False if get_valid_status is None else get_valid_status
-        if not isinstance(get_valid_status, bool):
-            raise TypeError("Error tracking points: Get_tracked needs to be a boolean")
+        int_out, get_valid_status, s_exact_mode = validate_track_args(pts, int_out, get_valid_status, s_exact_mode)
         warped = _track_device(self, pts, int_out, s_exact_mode)
         if get_valid_status:
             status = self.valid_source()[np.round(pts[..., 0]).astype('i'), np.round(pts[..., 1]).astype('i')]

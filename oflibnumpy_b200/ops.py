@@ -12,7 +12,7 @@ from . import _ops
 from .device import DeviceArray
 from .flow import Flow
 from .validation import (get_valid_ref, validate_shape, validate_flow_array, validate_transform_list,
-                         DEFAULT_THRESHOLD)
+                         validate_track_args, validate_track_dtype, DEFAULT_THRESHOLD)
 
 __all__ = ['apply_flow', 'combine_flows', 'invert_flow', 'switch_flow_ref', 'valid_target', 'valid_source',
            'get_flow_padding', 'from_matrix', 'from_transforms', 'matrix_from_transforms', 'matrix_from_transform',
@@ -212,19 +212,8 @@ def resize_flow(flow, scale):
 
 
 def _track_device(flow, pts, int_out, s_exact_mode):
-    """Point tracking (utils.py:547-622) on the device. `flow` is a Flow object."""
-    if not isinstance(pts, np.ndarray):
-        raise TypeError("Error tracking points: Pts needs to be a numpy array")
-    if pts.ndim != 2:
-        raise ValueError("Error tracking points: Pts needs to have shape N-2")
-    if pts.shape[1] != 2:
-        raise ValueError("Error tracking points: Pts needs to have shape N-2")
-    int_out = False if int_out is None else int_out
-    s_exact_mode = False if s_exact_mode is None else s_exact_mode
-    if not isinstance(int_out, bool):
-        raise TypeError("Error tracking points: Int_out needs to be a boolean")
-    if not isinstance(s_exact_mode, bool):
-        raise TypeError("Error tracking points: S_exact_mode needs to be a boolean")
+    """Point tracking (utils.py:547-622) on the device. `flow` is a Flow object; the arguments have passed
+    validate_track_args."""
     vecs = flow._vd()
     if int(_ops.nonzero_flags(vecs, None, DEFAULT_THRESHOLD)[0]) == 0:      # thresholded-zero flow: points unchanged
         warped = pts
@@ -235,7 +224,7 @@ def _track_device(flow, pts, int_out, s_exact_mode):
             d = vecs.numpy()[0][pts[:, 0], pts[:, 1], ::-1]
             warped = pts + d
         elif flow.ref == 's' and not np.issubdtype(pts.dtype, np.floating):
-            raise TypeError("Error tracking points: Pts numpy array needs to have a float or int dtype")
+            validate_track_dtype(pts.dtype)
         elif flow.ref == 's' and not s_exact_mode:
             warped, outside = _ops.track_bilinear(vecs, pts)
             if outside:
@@ -257,7 +246,9 @@ def _track_device(flow, pts, int_out, s_exact_mode):
 def track_pts(flow, ref, pts, int_out=None, s_exact_mode=None):
     """Warp points (N,2) given as (row, col) with a flow field (utils.py:547-622)."""
     flow = validate_flow_array(flow, "Error tracking points: ")
-    return _track_device(Flow(flow, ref), pts, int_out, s_exact_mode)
+    flow = Flow(flow, ref)
+    int_out, _, s_exact_mode = validate_track_args(pts, int_out, None, s_exact_mode)
+    return _track_device(flow, pts, int_out, s_exact_mode)
 
 
 def _combine2_t_device(a, b):

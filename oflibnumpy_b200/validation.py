@@ -77,6 +77,38 @@ def validate_visualise_args(mode, show_mask, show_mask_borders, range_max):
     return VIS_MODES[mode], show_mask, show_mask_borders
 
 
+def validate_track_args(pts, int_out, get_valid_status, s_exact_mode, batch_size=None):
+    """Checks of Flow.track (flow_class.py:755-795, utils.py:547-622), shared by Flow.track, track_pts and
+    FlowBatch.track. Returns (int_out, get_valid_status, s_exact_mode); None stands for False. With batch_size (a
+    FlowBatch's N), pts may also be a device array (``__cuda_array_interface__``) and of shape (N,P,2) as well as
+    (P,2)."""
+    get_valid_status = False if get_valid_status is None else get_valid_status
+    if not isinstance(get_valid_status, bool):
+        raise TypeError("Error tracking points: Get_tracked needs to be a boolean")
+    if not isinstance(pts, np.ndarray) and (batch_size is None or not hasattr(pts, '__cuda_array_interface__')):
+        raise TypeError("Error tracking points: Pts needs to be a numpy array")
+    if batch_size is None:
+        if len(pts.shape) != 2:
+            raise ValueError("Error tracking points: Pts needs to have shape N-2")
+        if pts.shape[1] != 2:
+            raise ValueError("Error tracking points: Pts needs to have shape N-2")
+    elif not (len(pts.shape) == 2 or (len(pts.shape) == 3 and pts.shape[0] == batch_size)) or pts.shape[-1] != 2:
+        raise ValueError("Error tracking points: Pts needs to have shape ({},P,2) or (P,2)".format(batch_size))
+    int_out = False if int_out is None else int_out
+    s_exact_mode = False if s_exact_mode is None else s_exact_mode
+    if not isinstance(int_out, bool):
+        raise TypeError("Error tracking points: Int_out needs to be a boolean")
+    if not isinstance(s_exact_mode, bool):
+        raise TypeError("Error tracking points: S_exact_mode needs to be a boolean")
+    return int_out, get_valid_status, s_exact_mode
+
+
+def validate_track_dtype(dtype):
+    """Point dtypes Flow.track accepts for an 's' flow (utils.py:600-602); FlowBatch.track applies it to both refs."""
+    if not (np.issubdtype(dtype, np.integer) or np.issubdtype(dtype, np.floating)):
+        raise TypeError("Error tracking points: Pts numpy array needs to have a float or int dtype")
+
+
 def validate_transform_list(transform_list):
     """Checks of from_transforms (utils.py:363-388)."""
     pre = "Error creating flow from transforms: "
