@@ -243,6 +243,27 @@ int ofk_track(const float* flow, const uint8_t* mask, int ref, int exact, const 
               int pts_dtype, int pts_shared, int P, int arith, int int_out, void* out, const uint8_t* status_plane,
               uint8_t* status, int* errors, int N, int H, int W, ofk_stream_t stream);
 
+/* Flow.matrix (flow_class.py:797-867) of N frames: a 3x3 float64 transform per frame fitted to the point pairs of the
+ * valid pixels, resolved on the device with no synchronisation.
+ *   flow [N,H,W,2]; mask [N,H,W] or NULL (all valid), read when masked != 0; ref 's' (src = grid, dst = grid + flow)
+ *     or 't' (src = grid - flow, dst = grid), grid = (column, row), coordinates rounded to float32.
+ *   dof 4 (similarity), 6 (affine) or 8 (homography); method OFK_FIT_RANSAC or OFK_FIT_LMEDS with `hypotheses`
+ *     minimal samples per frame (1 to 65536), or OFK_FIT_LMS (dof 8 only: every valid point).
+ *   thr: frames whose flow is zero below thr (on valid pixels when masked) give the identity.
+ *   out_mats float64 [N,3,3] (src -> dst; bottom row 0 0 1 for dof 4 and 6, H[2][2] = 1 for dof 8; all NaN for a
+ *     degenerate frame); out_inliers uint8 [N,H,W] 0/1 (the inliers of the selected hypothesis, the set the refinement
+ *     used) and out_counts int32 [N] (0 for zero and degenerate frames) may be NULL.
+ *   ws: ofk_fit_matrix_workspace(dof, method, hypotheses, N, H, W) bytes, 8-byte aligned (0 for bad arguments).
+ * Frame n of the outputs does not depend on the other frames of the batch, and repeated calls give identical outputs.
+ * A fixed number of launches whatever N; N <= 65535, H*W < 2^31. */
+#define OFK_FIT_LMS 0
+#define OFK_FIT_RANSAC 1
+#define OFK_FIT_LMEDS 2
+size_t ofk_fit_matrix_workspace(int dof, int method, int hypotheses, int N, int H, int W);
+int ofk_fit_matrix(const float* flow, const uint8_t* mask, int ref, int dof, int method, int hypotheses, float thr,
+                   int masked, double* out_mats, uint8_t* out_inliers, int* out_counts, int N, int H, int W, void* ws,
+                   size_t ws_bytes, ofk_stream_t stream);
+
 /* points_inside_area (utils.py:283-295): pts float64 [n][2] (row, col) rounded half-even like numpy.round. */
 int ofk_points_inside_area(const double* pts, size_t n, int H, int W, uint8_t* out, ofk_stream_t stream);
 

@@ -12,6 +12,8 @@ RULE_STRICT, RULE_GT_HALF, RULE_GE_HALF = 0, 1, 2
 OP_ADD, OP_SUB, OP_MUL, OP_DIV, OP_POW = 0, 1, 2, 3, 4
 PAD_CONSTANT, PAD_EDGE, PAD_SYMMETRIC = 0, 1, 2
 PAD_MODES = {'constant': PAD_CONSTANT, 'edge': PAD_EDGE, 'symmetric': PAD_SYMMETRIC}
+FIT_LMS, FIT_RANSAC, FIT_LMEDS = 0, 1, 2
+FIT_METHODS = {'lms': FIT_LMS, 'ransac': FIT_RANSAC, 'lmeds': FIT_LMEDS}
 
 
 class OflibCudaError(RuntimeError):
@@ -48,6 +50,8 @@ _SIGNATURES = {
     'ofk_visualise_batch': (_i, [_vp, _vp, _f, _i, _i, _i, _f, _vp, _i, _i, _i, _vp, _sz, _vp]),
     'ofk_track_bilinear': (_i, [_vp, _vp, _sz, _i, _i, _vp, _vp, _vp]),
     'ofk_track': (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
+    'ofk_fit_matrix_workspace': (_sz, [_i, _i, _i, _i, _i, _i]),
+    'ofk_fit_matrix': (_i, [_vp, _vp, _i, _i, _i, _i, _f, _i, _vp, _vp, _vp, _i, _i, _i, _vp, _sz, _vp]),
     'ofk_points_inside_area': (_i, [_vp, _sz, _i, _i, _vp, _vp]),
     'ofk_forward_s_workspace': (_sz, [_i, _i, _i]),
     'ofk_forward_s': (_i, [_vp, _i, _vp, _f, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _sz, _vp]),
@@ -93,7 +97,7 @@ _SIGNATURES = {
 }
 
 _NO_CHECK = {'ofk_last_error', 'ofk_version', 'ofk_forward_s_workspace', 'ofk_combine12_workspace', 'ofk_kth_smallest_workspace',
-             'ofk_visualise_batch_workspace', 'ofk_rt_launch_count', 'ofk_rt_path_count'}
+             'ofk_visualise_batch_workspace', 'ofk_fit_matrix_workspace', 'ofk_rt_launch_count', 'ofk_rt_path_count'}
 
 _lib = None
 

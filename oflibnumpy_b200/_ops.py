@@ -377,3 +377,18 @@ def resize_flow(vecs, mask, fy, fx):
     _lib.call('ofk_resize_flow', _p(vecs), _p(mask), _p(ov), _p(om), n, h, w, ho, wo, float(fy), float(fx),
               dev.current_stream())
     return ov, om
+
+
+def fit_matrix(flow, mask, ref, dof, method, hypotheses, thr, masked, want_inliers):
+    """Flow.matrix of every frame in one ofk_fit_matrix call: flow [N,H,W,2], mask [N,H,W]. Returns device arrays
+    (matrices float64 [N,3,3], inliers uint8 [N,H,W] or None, counts int32 [N]); asynchronous."""
+    n, h, w = flow.shape[:3]
+    code = _lib.FIT_METHODS[method]
+    mats = DeviceArray.empty((n, 3, 3), np.float64)
+    inliers = DeviceArray.empty((n, h, w), np.uint8) if want_inliers else None
+    counts = DeviceArray.empty((n,), np.int32)
+    ws_bytes = _lib.call('ofk_fit_matrix_workspace', dof, code, hypotheses, n, h, w)
+    ws = DeviceArray.empty((max(ws_bytes, 16),), np.uint8)
+    _lib.call('ofk_fit_matrix', flow.ptr, _p(mask), ord(ref), dof, code, hypotheses, float(thr), int(masked), mats.ptr,
+              _p(inliers), counts.ptr, n, h, w, ws.ptr, ws_bytes, dev.current_stream())
+    return mats, inliers, counts

@@ -12,7 +12,7 @@ from . import device as dev
 from .device import DeviceArray
 from .flow import Flow
 from .validation import get_valid_ref, validate_shape, validate_transform_list, validate_visualise_args, \
-    validate_track_args, validate_track_dtype, DEFAULT_THRESHOLD
+    validate_track_args, validate_track_dtype, validate_matrix_args, DEFAULT_THRESHOLD
 
 __all__ = ['FlowBatch', 'shard_range', 'apply_flow_host', 'combine_flows_host', 'apply_combine_host',
            'visualise_flows_host']
@@ -305,6 +305,26 @@ class FlowBatch(object):
             _raise_track_error(errors.numpy(), h, w)
         return (out, status) if get_valid_status else out
 
+
+    def matrix(self, dof=None, method=None, masked=None, *, hypotheses=None, return_inliers=False):
+        """Frame-wise ``Flow.matrix`` (flow_class.py:797-867) fitted on the device in one ofk_fit_matrix call: frame
+        ``i`` is the 3x3 transform from the src to the dst points of ``self[i]`` (ref 's': src = grid, dst = grid +
+        flow; ref 't': src = grid - flow, dst = grid; the valid pixels only when ``masked``) with ``dof`` 4
+        (similarity), 6 (affine) or 8 (homography) and ``method`` 'lms', 'ransac' or 'lmeds'; the defaults are the
+        reference's (8, 'ransac', True). 'ransac' and 'lmeds' score ``hypotheses`` (default 1024) minimal samples per
+        frame and refine the best on its inliers (reprojection error at most 3 px for 'ransac', the LMedS threshold
+        from the median otherwise); 'lms' fits every valid point. No synchronisation and no read-back.
+
+        Returns a device float64 array (N,3,3) (``.numpy()`` to download): the bottom row is [0, 0, 1] for dof 4 and 6,
+        H[2,2] = 1 for dof 8. A frame whose flow is zero below the threshold gives the identity; a degenerate frame (too
+        few valid points, no non-degenerate sample, a singular refinement) gives NaN. With ``return_inliers`` also a
+        device uint8 (N,H,W) of 0/1, the inliers the refinement used, and a device int32 (N,) of their counts (0 for
+        zero and degenerate frames). The hypotheses come from a fixed counter-based generator: frame ``i`` does not
+        depend on the rest of the batch, and two calls give the same result."""
+        dof, method, masked, hypotheses = validate_matrix_args(dof, method, masked, hypotheses)
+        mats, inliers, counts = _ops.fit_matrix(self.vecs, self.masks, self.ref, dof, method, hypotheses,
+                                                DEFAULT_THRESHOLD, masked, return_inliers)
+        return (mats, inliers, counts) if return_inliers else mats
 
 def _track_range_fails(pts, lookup, is_int, status, h, w):
     """True if a host point fails a range test of Flow.track (the tests ofk_track repeats per frame), which only

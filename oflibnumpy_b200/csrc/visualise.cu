@@ -21,7 +21,7 @@
 #include <algorithm>
 #include <cmath>
 
-#include "ofk_common.cuh"
+#include "radix_select.cuh"
 
 namespace ofk {
 namespace vis {
@@ -46,11 +46,8 @@ __device__ __forceinline__ float fast_atan2_deg(float y, float x) {
 }
 
 // ------------------------------------------------------------------------------------------------ radix selection
-// Digits of the 32-bit pattern: bits 31..20 (pass 0), 19..10 (pass 1), 9..0 (pass 2). Non-negative floats order like
-// their bit patterns.
-constexpr int kBins0 = 4096, kBins12 = 1024, kMaxRanks = 4;
-__host__ __device__ constexpr int pass_shift(int pass) { return pass == 0 ? 20 : (pass == 1 ? 10 : 0); }
-__host__ __device__ constexpr int pass_bins(int pass) { return pass == 0 ? kBins0 : kBins12; }
+// (digits, histogram helpers: radix_select.cuh)
+constexpr int kMaxRanks = 4;
 
 // Per-frame selection record: head, then the histograms (pass 0: one, shared by every rank since no prefix is fixed
 // yet; passes 1 and 2: one per rank). Zeroed before the magnitude / first histogram pass.
@@ -79,26 +76,6 @@ struct Select {
     int nq;
     __device__ SelectHead* head(size_t n) const { return reinterpret_cast<SelectHead*>(base + n * stride); }
 };
-
-// Adds one to sh[bin] for the lanes with `active`. When all active lanes of the warp share one bin (thresholded flows
-// put most pixels of a frame into bin 0) that is one atomic for the warp instead of 32 colliding ones. Called by all
-// 32 lanes.
-__device__ __forceinline__ void hist_add(unsigned int* sh, unsigned int bin, bool active) {
-    const unsigned int act = __ballot_sync(0xffffffffu, active);
-    if (act == 0) return;
-    const int leader = __ffs(act) - 1;
-    const unsigned int lead_bin = __shfl_sync(0xffffffffu, bin, leader);
-    if (__all_sync(0xffffffffu, !active || bin == lead_bin)) {
-        if ((int)(threadIdx.x & 31) == leader) atomicAdd(sh + lead_bin, (unsigned int)__popc(act));
-    } else if (active) {
-        atomicAdd(sh + bin, 1u);
-    }
-}
-
-__device__ __forceinline__ void flush_hist(const unsigned int* sh, unsigned int* g, int bins) {
-    for (int k = threadIdx.x; k < bins; k += blockDim.x)
-        if (sh[k]) atomicAdd(g + k, sh[k]);
-}
 
 constexpr int kUnroll = 4;   // elements per thread and loop trip, strided by the block (coalesced)
 

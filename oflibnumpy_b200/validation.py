@@ -1,6 +1,8 @@
 """Argument validators of the public API. Types of exception and message texts are the reference's
 (utils.py:25-88 of oflibnumpy) because they are part of the drop-in contract; the checks run on the host before any
 device call."""
+import warnings
+
 import numpy as np
 
 DEFAULT_THRESHOLD = 1e-3  # utils.py:22
@@ -127,3 +129,29 @@ def validate_transform_list(transform_list):
                              .format(t[0], expected[t[0]], len(t) - 1))
         if not all(isinstance(item, (float, int)) for item in t[1:]):
             raise ValueError(pre + "Transform values for '{}' need to be integers or floats".format(t[0]))
+
+
+def validate_matrix_args(dof, method, masked, hypotheses):
+    """Checks of Flow.matrix (flow_class.py:797-867) plus the hypothesis count of FlowBatch.matrix. Returns (dof, method,
+    masked, hypotheses) with the reference's defaults for None (8, 'ransac', True) and 1024 hypotheses. 'lms' with dof
+    4 or 6 warns and becomes 'ransac', as in the reference (only findHomography has a plain least-squares method)."""
+    pre = "Error fitting transformation matrix to flow: "
+    dof = 8 if dof is None else dof
+    method = 'ransac' if method is None else method
+    masked = True if masked is None else masked
+    hypotheses = 1024 if hypotheses is None else hypotheses
+    if dof not in (4, 6, 8):
+        raise ValueError(pre + "Dof needs to be 4, 6 or 8")
+    if method not in ('lms', 'ransac', 'lmeds'):
+        raise ValueError(pre + "Method needs to be 'lms', 'ransac', or 'lmeds'")
+    if not isinstance(masked, bool):
+        raise TypeError(pre + "Masked needs to be boolean")
+    if isinstance(hypotheses, bool) or not isinstance(hypotheses, int):
+        raise TypeError(pre + "Hypotheses needs to be an integer")
+    if not 1 <= hypotheses <= 65536:
+        raise ValueError(pre + "Hypotheses needs to be between 1 and 65536")
+    if method == 'lms' and dof != 8:
+        warnings.warn("Method 'lms' (least mean squares) not supported for fitting a transformation matrix with 4 or 6 "
+                      "degrees of freedom to the flow. Method 'ransac' used instead.")
+        method = 'ransac'
+    return dof, method, masked, hypotheses
