@@ -264,6 +264,26 @@ int ofk_fit_matrix(const float* flow, const uint8_t* mask, int ref, int dof, int
                    int masked, double* out_mats, uint8_t* out_inliers, int* out_counts, int N, int H, int W, void* ws,
                    size_t ws_bytes, ofk_stream_t stream);
 
+/* Accumulation of clips of flows to their keyframe: mode-3 composition (ofk_combine3) folded over each clip, with the
+ * early exits of combine_with at every step. The batch flow [S*L,H,W,2], mask [S*L,H,W] (0/1, required) is S clips
+ * of L consecutive frames B_0 .. B_{L-1}, clip-major. "Zero" is the masked zero test of a whole frame at thr (as in
+ * ofk_nonzero_flags); self is tested first, as in combine_with.
+ *   ref 's' (left fold, frame 0 -> frame k+1 on frame 0's grid): C_0 = B_0; for k = 1 .. L-1:
+ *     C_{k-1} zero -> C_k = B_k;  else B_k zero -> C_k = C_{k-1};
+ *     else C_k(p) = C_{k-1}(p) + Q(B_k, p + C_{k-1}(p)), mask C_{k-1}m(p) & strict(B_k mask at the taps).
+ *   ref 't' (right fold, frame j -> frame L on frame L's grid): D_{L-1} = B_{L-1}; for j = L-2 .. 0:
+ *     B_j zero -> D_j = D_{j+1};  else D_{j+1} zero -> D_j = B_j;
+ *     else D_j(p) = D_{j+1}(p) + Q(B_j, p - D_{j+1}(p)), mask D_{j+1}m(p) & strict(B_j mask at the taps).
+ * Q is the cv2.remap sample of ofk_combine3: every frame is byte-identical to the loop of ofk_combine3 calls.
+ *   cumulative != 0: out [S*L,H,W,2], out_mask [S*L,H,W], frame s*L+k = C_k ('s') or D_k ('t');
+ *   cumulative == 0: out [S,H,W,2], out_mask [S,H,W], the whole-clip composite C_{L-1} ('s') or D_0 ('t').
+ * flow and out 8-byte aligned; ws: ofk_accumulate_workspace(S, L) bytes, 4-byte aligned (0 for bad arguments).
+ * S*L <= 65535, H and W below 32768, frame offsets 64-bit. A fixed number of launches whatever S and L: a state that
+ * is zero by cancellation is found after the walk and its clip redone by one CTA (slow, exact). */
+size_t ofk_accumulate_workspace(int S, int L);
+int ofk_accumulate(const float* flow, const uint8_t* mask, int ref, float thr, int S, int L, int H, int W,
+                   int cumulative, float* out, uint8_t* out_mask, void* ws, size_t ws_bytes, ofk_stream_t stream);
+
 /* points_inside_area (utils.py:283-295): pts float64 [n][2] (row, col) rounded half-even like numpy.round. */
 int ofk_points_inside_area(const double* pts, size_t n, int H, int W, uint8_t* out, ofk_stream_t stream);
 

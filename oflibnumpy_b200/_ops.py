@@ -392,3 +392,17 @@ def fit_matrix(flow, mask, ref, dof, method, hypotheses, thr, masked, want_inlie
     _lib.call('ofk_fit_matrix', flow.ptr, _p(mask), ord(ref), dof, code, hypotheses, float(thr), int(masked), mats.ptr,
               _p(inliers), counts.ptr, n, h, w, ws.ptr, ws_bytes, dev.current_stream())
     return mats, inliers, counts
+
+
+def accumulate(flow, mask, ref, thr, s, l, cumulative):
+    """Mode-3 composition folded over S clips of L frames in one ofk_accumulate call: flow [S*L,H,W,2], mask [S*L,H,W].
+    Returns device arrays (vecs [S*L or S,H,W,2] float32, masks uint8 of the same frames); asynchronous."""
+    h, w = flow.shape[1:3]
+    n_out = s * l if cumulative else s
+    out = DeviceArray.empty((n_out, h, w, 2), np.float32)
+    omask = DeviceArray.empty((n_out, h, w), np.uint8)
+    ws_bytes = _lib.call('ofk_accumulate_workspace', s, l)
+    ws = DeviceArray.empty((max(ws_bytes, 16),), np.uint8)
+    _lib.call('ofk_accumulate', flow.ptr, mask.ptr, ord(ref), float(thr), s, l, h, w, int(cumulative), out.ptr,
+              omask.ptr, ws.ptr, ws_bytes, dev.current_stream())
+    return out, omask

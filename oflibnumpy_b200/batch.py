@@ -12,7 +12,7 @@ from . import device as dev
 from .device import DeviceArray
 from .flow import Flow
 from .validation import get_valid_ref, validate_shape, validate_transform_list, validate_visualise_args, \
-    validate_track_args, validate_track_dtype, validate_matrix_args, DEFAULT_THRESHOLD
+    validate_track_args, validate_track_dtype, validate_matrix_args, validate_accumulate_args, DEFAULT_THRESHOLD
 
 __all__ = ['FlowBatch', 'shard_range', 'apply_flow_host', 'combine_flows_host', 'apply_combine_host',
            'visualise_flows_host']
@@ -325,6 +325,31 @@ class FlowBatch(object):
         mats, inliers, counts = _ops.fit_matrix(self.vecs, self.masks, self.ref, dof, method, hypotheses,
                                                 DEFAULT_THRESHOLD, masked, return_inliers)
         return (mats, inliers, counts) if return_inliers else mats
+
+    def accumulate(self, clip_length=None, cumulative=True, thresholded=False):
+        """Mode-3 composition (``combine_with(., 3)``) folded over clips, in one ofk_accumulate call. The N frames are
+        N / ``clip_length`` clips of L = ``clip_length`` consecutive frames (default: one clip of all N), clip-major:
+        frame ``s*L + k`` is step k of clip s. Clips are independent.
+
+        ref 's', the left fold: C_0 = B_0, C_k = C_{k-1}.combine_with(B_k, 3), the flow from frame 0 to frame k+1 on
+        frame 0's grid. ref 't', the right fold: D_{L-1} = B_{L-1}, D_j = B_j.combine_with(D_{j+1}, 3), the flow from
+        frame j to frame L on frame L's grid. Every step takes combine_with's early exits ("zero" is ``is_zero(
+        thresholded, masked=True)`` of the whole frame, self tested first), so each result frame equals, vectors and
+        mask byte for byte, the loop ``acc = F[0]; acc = acc.combine_with(F[k], 3, thresholded)`` ('s') or
+        ``acc = F[L-1]; acc = F[j].combine_with(acc, 3, thresholded)`` ('t').
+
+        Returns a device-resident FlowBatch of the same ref, without synchronisation or read-back: with ``cumulative``
+        N frames in the input's layout (frame ``s*L + k`` is C_k, resp. D_k), otherwise N / L frames, the whole-clip
+        composite (C_{L-1}, resp. D_0). Frames are always new arrays, also where an exit returns an input."""
+        n, (h, w) = len(self), self.shape
+        clip = validate_accumulate_args(clip_length, cumulative, thresholded, n)
+        if n == 0:
+            return FlowBatch._wrap(DeviceArray.empty((0, h, w, 2), np.float32), self.ref,
+                                   DeviceArray.empty((0, h, w), np.uint8))
+        v, m = _ops.accumulate(self.vecs, self.masks, self.ref, DEFAULT_THRESHOLD if thresholded else 0.0, n // clip,
+                               clip, cumulative)
+        return FlowBatch._wrap(v, self.ref, m)
+
 
 def _track_range_fails(pts, lookup, is_int, status, h, w):
     """True if a host point fails a range test of Flow.track (the tests ofk_track repeats per frame), which only

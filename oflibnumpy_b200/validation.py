@@ -155,3 +155,20 @@ def validate_matrix_args(dof, method, masked, hypotheses):
                       "degrees of freedom to the flow. Method 'ransac' used instead.")
         method = 'ransac'
     return dof, method, masked, hypotheses
+
+
+def validate_accumulate_args(clip_length, cumulative, thresholded, batch_size):
+    """Checks of FlowBatch.accumulate. Returns the clip length L: ``clip_length``, or the whole batch for None (1 for
+    an empty batch)."""
+    pre = "Error accumulating flows: "
+    if not isinstance(cumulative, bool):
+        raise TypeError(pre + "Cumulative needs to be a boolean")
+    if not isinstance(thresholded, bool):
+        raise TypeError(pre + "Thresholded needs to be a boolean")
+    if clip_length is None:
+        return max(batch_size, 1)
+    if isinstance(clip_length, bool) or not isinstance(clip_length, (int, np.integer)) or clip_length < 1 or \
+            batch_size % clip_length != 0:
+        raise ValueError(pre + "Clip_length needs to be a positive integer that divides the batch size {}, not {!r}"
+                         .format(batch_size, clip_length))
+    return int(clip_length)
