@@ -2,6 +2,7 @@
 // the zero / finite tests (flow_class.py:78-79,1230-1245; utils.py:298-316,527-544), Flow.pad (:508-526), the extent
 // reduction of get_padding (:1197-1228) and points_inside_area (utils.py:283-295). All HBM-bound; 128-bit accesses,
 // grid-stride loops sized to the SM count.
+#include <float.h>
 #include <math.h>
 
 #include <algorithm>
@@ -71,6 +72,17 @@ __device__ __forceinline__ R apply_op(int op, R a, R s) {
     }
 }
 
+// float32 ** python scalar: numpy sends the exponents 1, -1, 0, 0.5 and 2 to positive / reciprocal / ones_like / sqrt /
+// square (fast_scalar_power), all correctly rounded; every other exponent goes to a float32 pow that is not.
+__device__ __forceinline__ float pow_f32(float a, float s) {
+    if (s == 2.f) return __fmul_rn(a, a);
+    if (s == 0.5f) return __fsqrt_rn(a);
+    if (s == -1.f) return __fdiv_rn(1.f, a);
+    if (s == 1.f) return a;
+    if (s == 0.f) return 1.f;
+    return powf(a, s);
+}
+
 __global__ void __launch_bounds__(256) scale_kernel(int op, const float* __restrict__ A, double su, double sv,
                                                     int in_f64, float* __restrict__ out, size_t npix) {
     const size_t tid = (size_t)blockIdx.x * blockDim.x + threadIdx.x, nth = (size_t)gridDim.x * blockDim.x;
@@ -81,6 +93,9 @@ __global__ void __launch_bounds__(256) scale_kernel(int op, const float* __restr
         if (in_f64) {
             r.x = (float)apply_op<double>(op, (double)a.x, su);
             r.y = (float)apply_op<double>(op, (double)a.y, sv);
+        } else if (op == OFK_OP_POW) {
+            r.x = pow_f32(a.x, fu);
+            r.y = pow_f32(a.y, fv);
         } else {
             r.x = apply_op<float>(op, a.x, fu);
             r.y = apply_op<float>(op, a.y, fv);
@@ -117,13 +132,14 @@ __global__ void __launch_bounds__(256) finite_kernel(const float* __restrict__ d
     if (__syncthreads_or(bad) && threadIdx.x == 0) *flag = 1;
 }
 
-// float atomic min/max through the ordered-int trick
+// float atomic min/max through the ordered-int trick. The branch is on the sign bit, not on v >= 0: -0.0 is >= 0 but
+// as a signed int it is INT_MIN, which would beat every negative value already stored.
 __device__ __forceinline__ void atomic_min_f(float* addr, float v) {
-    if (v >= 0.f) atomicMin(reinterpret_cast<int*>(addr), __float_as_int(v));
+    if (__float_as_int(v) >= 0) atomicMin(reinterpret_cast<int*>(addr), __float_as_int(v));
     else atomicMax(reinterpret_cast<unsigned int*>(addr), __float_as_uint(v));
 }
 __device__ __forceinline__ void atomic_max_f(float* addr, float v) {
-    if (v >= 0.f) atomicMax(reinterpret_cast<int*>(addr), __float_as_int(v));
+    if (__float_as_int(v) >= 0) atomicMax(reinterpret_cast<int*>(addr), __float_as_int(v));
     else atomicMin(reinterpret_cast<unsigned int*>(addr), __float_as_uint(v));
 }
 
@@ -229,54 +245,91 @@ __global__ void __launch_bounds__(256) crop_kernel(const uint8_t* __restrict__ i
         dst[i] = src[i];
 }
 
-// cv2.resize(INTER_LINEAR) of a flow field and its mask (utils.py:493-524, flow_class.py:491-506): half-pixel-centre
-// mapping, edge clamp, float32 coefficients; horizontal pass then vertical pass like OpenCV's separable kernel.
-// Vectors are scaled per axis afterwards; the mask is the resized float mask rounded half-even (0.5 -> 0).
-__device__ __forceinline__ void resize_coord(int d, double scale, int n, int& s0, int& s1, float& f) {
-    float fx = (float)((d + 0.5) * scale - 0.5);
+// cv2.resize(INTER_LINEAR) of a flow field and its mask (utils.py:493-524, flow_class.py:491-506), bit for bit with
+// OpenCV's generic float path (resize.cpp): half-pixel-centre mapping, float32 coefficients, horizontal pass then
+// vertical pass, no FMA. Vectors are scaled per axis afterwards; the mask is the resized float mask rounded half-even
+// (0.5 -> 0). OpenCV's border rules differ per axis: a column outside [0, W-1] is clamped together with its weight,
+// a row outside [0, H-1] only has its index clamped, so a border row is S*(1-fy) + S*fy, which may differ from S.
+enum { RESIZE_LINEAR = 0, RESIZE_AREA2 = 1, RESIZE_COPY = 2 };
+
+__device__ __forceinline__ void resize_coord(int d, double scale, int n, bool clamp_weight, int& s0, int& s1,
+                                             float& f) {
+    float fx = (float)__dadd_rn(__dmul_rn(d + 0.5, scale), -0.5);  // not contracted to an FMA, as in OpenCV
     int sx = (int)floorf(fx);
     fx -= sx;
-    if (sx < 0) { fx = 0.f; sx = 0; }
-    if (sx >= n - 1) { fx = 0.f; sx = n - 1; }
-    s0 = sx;
-    s1 = min(sx + 1, n - 1);
+    if (clamp_weight) {
+        if (sx < 0) { fx = 0.f; sx = 0; }
+        if (sx >= n - 1) { fx = 0.f; sx = n - 1; }
+        s0 = sx;
+        s1 = min(sx + 1, n - 1);
+    } else {
+        s0 = min(max(sx, 0), n - 1);
+        s1 = min(max(sx + 1, 0), n - 1);
+    }
     f = fx;
+}
+
+// One output value from the four taps (00, 01 along x; 10, 11 one row down).
+// RESIZE_LINEAR: bilinear blend. RESIZE_AREA2: OpenCV turns INTER_LINEAR at an exact 1/2 x 1/2 scale into INTER_AREA's
+// fast path, sum = 0 + (((s00 + s01) + s10) + s11) times 0.25 where the 2x2 block is inside the image; an output whose
+// block is cut by the right or bottom edge of an odd-sized input averages the taps it has, summed in the same order.
+__device__ __forceinline__ float resize_tap(int mode, float s00, float s01, float s10, float s11, float a0, float a1,
+                                            float b0, float b1, bool has_x1, bool has_y1) {
+    if (mode == RESIZE_LINEAR) {
+        const float r0 = __fadd_rn(__fmul_rn(s00, a0), __fmul_rn(s01, a1));
+        const float r1 = __fadd_rn(__fmul_rn(s10, a0), __fmul_rn(s11, a1));
+        return __fadd_rn(__fmul_rn(r0, b0), __fmul_rn(r1, b1));
+    }
+    if (mode == RESIZE_COPY) return s00;
+    if (has_x1 && has_y1)
+        return __fmul_rn(__fadd_rn(0.f, __fadd_rn(__fadd_rn(__fadd_rn(s00, s01), s10), s11)), 0.25f);
+    float sum = __fadd_rn(0.f, s00);
+    if (has_x1) sum = __fadd_rn(sum, s01);
+    if (has_y1) sum = __fadd_rn(sum, s10);
+    return __fdiv_rn(sum, (float)(1 + has_x1 + has_y1));
 }
 
 __global__ void __launch_bounds__(256) resize_kernel(const float* __restrict__ vecs, const uint8_t* __restrict__ mask,
                                                      float* __restrict__ ov, uint8_t* __restrict__ om, int H, int W,
-                                                     int Ho, int Wo, double scale_x, double scale_y, float mul_u,
-                                                     float mul_v) {
+                                                     int Ho, int Wo, int mode, double scale_x, double scale_y,
+                                                     float mul_u, float mul_v) {
     const int x = blockIdx.x * 32 + (threadIdx.x & 31);
     const int y = blockIdx.y * 8 + (threadIdx.x >> 5);
     const int n = blockIdx.z;
     if (x >= Wo || y >= Ho) return;
     int x0, x1, y0, y1;
-    float fx, fy;
-    resize_coord(x, scale_x, W, x0, x1, fx);
-    resize_coord(y, scale_y, H, y0, y1, fy);
+    float fx = 0.f, fy = 0.f;
+    bool has_x1 = true, has_y1 = true;
+    if (mode == RESIZE_LINEAR) {
+        resize_coord(x, scale_x, W, true, x0, x1, fx);
+        resize_coord(y, scale_y, H, false, y0, y1, fy);
+    } else if (mode == RESIZE_AREA2) {
+        x0 = 2 * x;
+        y0 = 2 * y;
+        has_x1 = x0 + 1 < W;
+        has_y1 = y0 + 1 < H;
+        x1 = has_x1 ? x0 + 1 : x0;
+        y1 = has_y1 ? y0 + 1 : y0;
+    } else {
+        x0 = x1 = x;
+        y0 = y1 = y;
+    }
     const float a0 = 1.f - fx, a1 = fx, b0 = 1.f - fy, b1 = fy;
     const size_t fb = (size_t)n * H * W, ob = ((size_t)n * Ho + y) * Wo + x;
     if (ov != nullptr) {
         const float2* f = reinterpret_cast<const float2*>(vecs) + fb;
         const float2 s00 = f[(size_t)y0 * W + x0], s01 = f[(size_t)y0 * W + x1], s10 = f[(size_t)y1 * W + x0],
                      s11 = f[(size_t)y1 * W + x1];
-        const float r0u = __fadd_rn(__fmul_rn(s00.x, a0), __fmul_rn(s01.x, a1));
-        const float r1u = __fadd_rn(__fmul_rn(s10.x, a0), __fmul_rn(s11.x, a1));
-        const float r0v = __fadd_rn(__fmul_rn(s00.y, a0), __fmul_rn(s01.y, a1));
-        const float r1v = __fadd_rn(__fmul_rn(s10.y, a0), __fmul_rn(s11.y, a1));
         float2 o;
-        o.x = __fmul_rn(__fadd_rn(__fmul_rn(r0u, b0), __fmul_rn(r1u, b1)), mul_u);
-        o.y = __fmul_rn(__fadd_rn(__fmul_rn(r0v, b0), __fmul_rn(r1v, b1)), mul_v);
+        o.x = __fmul_rn(resize_tap(mode, s00.x, s01.x, s10.x, s11.x, a0, a1, b0, b1, has_x1, has_y1), mul_u);
+        o.y = __fmul_rn(resize_tap(mode, s00.y, s01.y, s10.y, s11.y, a0, a1, b0, b1, has_x1, has_y1), mul_v);
         reinterpret_cast<float2*>(ov)[ob] = o;
     }
     if (om != nullptr) {
         const uint8_t* m = mask + fb;
         const float m00 = m[(size_t)y0 * W + x0], m01 = m[(size_t)y0 * W + x1], m10 = m[(size_t)y1 * W + x0],
                     m11 = m[(size_t)y1 * W + x1];
-        const float r0 = __fadd_rn(__fmul_rn(m00, a0), __fmul_rn(m01, a1));
-        const float r1 = __fadd_rn(__fmul_rn(m10, a0), __fmul_rn(m11, a1));
-        const float v = __fadd_rn(__fmul_rn(r0, b0), __fmul_rn(r1, b1));
+        const float v = resize_tap(mode, m00, m01, m10, m11, a0, a1, b0, b1, has_x1, has_y1);
         om[ob] = rintf(v) == 1.0f ? 1 : 0;
     }
 }
@@ -518,9 +571,15 @@ extern "C" int ofk_resize_flow(const float* vecs, const uint8_t* mask, float* ou
     OFK_CHECK_ARG(!out_vecs || ((((uintptr_t)vecs | (uintptr_t)out_vecs) & 7) == 0), "ofk_resize_flow: vecs must be 8-byte aligned");
     if (N == 0) return OFK_OK;
     OFK_CHECK_ARG(N <= 65535, "ofk_resize_flow: N too large");
+    // cv::resize: an output of the input's size is a copy; INTER_LINEAR at an inverse scale of exactly 2 on both axes
+    // (|1/f - 2| < DBL_EPSILON) is INTER_AREA's fast path
+    const double sx = 1.0 / fx, sy = 1.0 / fy;
+    const int mode = (Ho == H && Wo == W)                                           ? RESIZE_COPY
+                     : (fabs(sx - 2.0) < DBL_EPSILON && fabs(sy - 2.0) < DBL_EPSILON) ? RESIZE_AREA2
+                                                                                      : RESIZE_LINEAR;
     dim3 grid((Wo + 31) / 32, (Ho + 7) / 8, N);
     resize_kernel<<<grid, 256, 0, as_stream(stream)>>>(out_vecs ? vecs : nullptr, out_mask ? mask : nullptr, out_vecs,
-                                                      out_mask, H, W, Ho, Wo, 1.0 / fx, 1.0 / fy, (float)fx, (float)fy);
+                                                      out_mask, H, W, Ho, Wo, mode, sx, sy, (float)fx, (float)fy);
     OFK_LAUNCHED();
     return OFK_OK;
 }

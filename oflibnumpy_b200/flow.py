@@ -330,6 +330,8 @@ class Flow(object):
             if self.shape != other.shape:
                 raise ValueError("Error {} flow: {} flow objects are not the same shape".format(name, whom))
             v, m = _ops.addsub(op, self._vd(), self._md(), other._vd(), other._md())
+            if not _ops.all_finite(v):      # the sum of two finite float32 fields can overflow
+                raise ValueError("Error setting flow vectors: Input contains NaN, Inf or -Inf values")
             return Flow._wrap(v, self._ref, m)
         if self.shape != other.shape[:2] or other.ndim != 3 or other.shape[2] != 2:
             raise ValueError("Error {} flow: {} numpy array needs to have the same shape as the flow "
