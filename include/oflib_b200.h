@@ -284,6 +284,27 @@ size_t ofk_accumulate_workspace(int S, int L);
 int ofk_accumulate(const float* flow, const uint8_t* mask, int ref, float thr, int S, int L, int H, int W,
                    int cumulative, float* out, uint8_t* out_mask, void* ws, size_t ws_bytes, ofk_stream_t stream);
 
+/* ofk_accumulate with the fold chosen for either ref: fold 'l' (left) or 'r' (right). The early exits depend on the
+ * fold only, as in the loop of combine_with:
+ *   fold 'l': A_0 = B_0; for k = 1 .. L-1: A_k = A_{k-1} (+) B_k, i.e. A_{k-1} zero -> B_k; else B_k zero -> A_{k-1};
+ *     else ref 's': A_k(p) = A_{k-1}(p) + Q(B_k, p + A_{k-1}(p)), mask A_{k-1}m(p) & strict(B_k mask at the taps);
+ *          ref 't': A_k(p) = B_k(p) + Q(A_{k-1}, p - B_k(p)), mask B_km(p) & strict(A_{k-1} mask at the taps).
+ *   fold 'r': A_{L-1} = B_{L-1}; for j = L-2 .. 0: A_j = B_j (+) A_{j+1}, i.e. B_j zero -> A_{j+1}; else A_{j+1} zero
+ *     -> B_j; else ref 's': A_j(p) = B_j(p) + Q(A_{j+1}, p + B_j(p)), mask B_jm(p) & strict(A_{j+1} mask at the taps);
+ *          ref 't': A_j(p) = A_{j+1}(p) + Q(B_j, p - A_{j+1}(p)), mask A_{j+1}m(p) & strict(B_j mask at the taps).
+ * ('s', 'l') and ('t', 'r') are exactly ofk_accumulate. ('t', 'l') gives the flow from frame 0 to frame k+1 on frame
+ * k+1's grid (apply it to frame 0 to warp the keyframe into frame k+1); ('s', 'r') the flow from frame j to frame L
+ * on frame j's grid. Outputs and cumulative as for ofk_accumulate: frame s*L+k = A_k, or one frame per clip, A_{L-1}
+ * (fold 'l') or A_0 (fold 'r').
+ * ws: ofk_accumulate_fold_workspace(ref, fold, S, L, H, W, cumulative) bytes (0 for bad arguments), 8-byte aligned for
+ * ('t', 'l') and ('s', 'r'), 4-byte aligned otherwise. Limits as for ofk_accumulate. ('t', 'l') and ('s', 'r') sample
+ * the composite of the previous step, so they run one launch per step for all S clips (L launches when cumulative,
+ * max(L-1, 1) otherwise, plus 2 for the zero flags), with exact exits and no repair. */
+size_t ofk_accumulate_fold_workspace(int ref, int fold, int S, int L, int H, int W, int cumulative);
+int ofk_accumulate_fold(const float* flow, const uint8_t* mask, int ref, int fold, float thr, int S, int L, int H,
+                        int W, int cumulative, float* out, uint8_t* out_mask, void* ws, size_t ws_bytes,
+                        ofk_stream_t stream);
+
 /* points_inside_area (utils.py:283-295): pts float64 [n][2] (row, col) rounded half-even like numpy.round. */
 int ofk_points_inside_area(const double* pts, size_t n, int H, int W, uint8_t* out, ofk_stream_t stream);
 

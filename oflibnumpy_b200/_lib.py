@@ -54,6 +54,8 @@ _SIGNATURES = {
     'ofk_fit_matrix': (_i, [_vp, _vp, _i, _i, _i, _i, _f, _i, _vp, _vp, _vp, _i, _i, _i, _vp, _sz, _vp]),
     'ofk_accumulate_workspace': (_sz, [_i, _i]),
     'ofk_accumulate': (_i, [_vp, _vp, _i, _f, _i, _i, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
+    'ofk_accumulate_fold_workspace': (_sz, [_i, _i, _i, _i, _i, _i, _i]),
+    'ofk_accumulate_fold': (_i, [_vp, _vp, _i, _i, _f, _i, _i, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
     'ofk_points_inside_area':(_i, [_vp, _sz, _i, _i, _vp, _vp]),
     'ofk_forward_s_workspace': (_sz, [_i, _i, _i]),
     'ofk_forward_s': (_i, [_vp, _i, _vp, _f, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _sz, _vp]),
@@ -100,7 +102,7 @@ _SIGNATURES = {
 
 _NO_CHECK = {'ofk_last_error', 'ofk_version', 'ofk_forward_s_workspace', 'ofk_combine12_workspace', 'ofk_kth_smallest_workspace',
              'ofk_visualise_batch_workspace', 'ofk_fit_matrix_workspace', 'ofk_accumulate_workspace',
-             'ofk_rt_launch_count', 'ofk_rt_path_count'}
+             'ofk_accumulate_fold_workspace', 'ofk_rt_launch_count', 'ofk_rt_path_count'}
 
 _lib = None
 

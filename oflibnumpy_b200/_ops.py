@@ -394,15 +394,16 @@ def fit_matrix(flow, mask, ref, dof, method, hypotheses, thr, masked, want_inlie
     return mats, inliers, counts
 
 
-def accumulate(flow, mask, ref, thr, s, l, cumulative):
-    """Mode-3 composition folded over S clips of L frames in one ofk_accumulate call: flow [S*L,H,W,2], mask [S*L,H,W].
-    Returns device arrays (vecs [S*L or S,H,W,2] float32, masks uint8 of the same frames); asynchronous."""
+def accumulate(flow, mask, ref, thr, s, l, cumulative, fold):
+    """Mode-3 composition folded ('left' or 'right') over S clips of L frames in one ofk_accumulate_fold call: flow
+    [S*L,H,W,2], mask [S*L,H,W]. Returns device arrays (vecs [S*L or S,H,W,2] float32, masks uint8 of the same
+    frames); asynchronous."""
     h, w = flow.shape[1:3]
     n_out = s * l if cumulative else s
     out = DeviceArray.empty((n_out, h, w, 2), np.float32)
     omask = DeviceArray.empty((n_out, h, w), np.uint8)
-    ws_bytes = _lib.call('ofk_accumulate_workspace', s, l)
+    ws_bytes = _lib.call('ofk_accumulate_fold_workspace', ord(ref), ord(fold[0]), s, l, h, w, int(cumulative))
     ws = DeviceArray.empty((max(ws_bytes, 16),), np.uint8)
-    _lib.call('ofk_accumulate', flow.ptr, mask.ptr, ord(ref), float(thr), s, l, h, w, int(cumulative), out.ptr,
-              omask.ptr, ws.ptr, ws_bytes, dev.current_stream())
+    _lib.call('ofk_accumulate_fold', flow.ptr, mask.ptr, ord(ref), ord(fold[0]), float(thr), s, l, h, w,
+              int(cumulative), out.ptr, omask.ptr, ws.ptr, ws_bytes, dev.current_stream())
     return out, omask

@@ -326,28 +326,39 @@ class FlowBatch(object):
                                                 DEFAULT_THRESHOLD, masked, return_inliers)
         return (mats, inliers, counts) if return_inliers else mats
 
-    def accumulate(self, clip_length=None, cumulative=True, thresholded=False):
-        """Mode-3 composition (``combine_with(., 3)``) folded over clips, in one ofk_accumulate call. The N frames are
-        N / ``clip_length`` clips of L = ``clip_length`` consecutive frames (default: one clip of all N), clip-major:
-        frame ``s*L + k`` is step k of clip s. Clips are independent.
+    def accumulate(self, clip_length=None, cumulative=True, thresholded=False, fold=None):
+        """Mode-3 composition (``combine_with(., 3)``) folded over clips, in one ofk_accumulate_fold call. The N frames
+        are N / ``clip_length`` clips of L = ``clip_length`` consecutive frames (default: one clip of all N),
+        clip-major: frame ``s*L + k`` is step k of clip s. Clips are independent.
 
-        ref 's', the left fold: C_0 = B_0, C_k = C_{k-1}.combine_with(B_k, 3), the flow from frame 0 to frame k+1 on
-        frame 0's grid. ref 't', the right fold: D_{L-1} = B_{L-1}, D_j = B_j.combine_with(D_{j+1}, 3), the flow from
-        frame j to frame L on frame L's grid. Every step takes combine_with's early exits ("zero" is ``is_zero(
-        thresholded, masked=True)`` of the whole frame, self tested first), so each result frame equals, vectors and
-        mask byte for byte, the loop ``acc = F[0]; acc = acc.combine_with(F[k], 3, thresholded)`` ('s') or
-        ``acc = F[L-1]; acc = F[j].combine_with(acc, 3, thresholded)`` ('t').
+        ``fold='left'``: A_0 = B_0, A_k = A_{k-1}.combine_with(B_k, 3), the loop ``acc = F[0]; acc =
+        acc.combine_with(F[k], 3, thresholded)``. For ref 's' A_k is the flow from frame 0 to frame k+1 on frame 0's
+        grid; for ref 't' the flow from frame 0 to frame k+1 on frame k+1's grid, so that ``A_k.apply(frame 0)`` warps
+        the keyframe into frame k+1 (keyframe or label propagation).
+        ``fold='right'``: A_{L-1} = B_{L-1}, A_j = B_j.combine_with(A_{j+1}, 3), the loop ``acc = F[L-1]; acc =
+        F[j].combine_with(acc, 3, thresholded)``. For ref 't' A_j is the flow from frame j to frame L on frame L's
+        grid; for ref 's' the flow from frame j to frame L on frame j's grid: where each pixel of frame j ends up in
+        the last frame.
+        ``fold=None`` is 'left' for ref 's' and 'right' for ref 't'.
+
+        Every step takes combine_with's early exits ("zero" is ``is_zero(thresholded, masked=True)`` of the whole
+        frame, self tested first), so each result frame equals the loop, vectors and mask byte for byte. ('s', 'left')
+        and ('t', 'right') walk each tile through the clip in a fixed number of launches; ('t', 'left') and ('s',
+        'right') sample the previous composite at every step and make one launch per step for all clips.
 
         Returns a device-resident FlowBatch of the same ref, without synchronisation or read-back: with ``cumulative``
-        N frames in the input's layout (frame ``s*L + k`` is C_k, resp. D_k), otherwise N / L frames, the whole-clip
-        composite (C_{L-1}, resp. D_0). Frames are always new arrays, also where an exit returns an input."""
+        N frames in the input's layout (frame ``s*L + k`` is A_k), otherwise N / L frames, the whole-clip composite
+        (A_{L-1} for the left fold, A_0 for the right). Frames are always new arrays, also where an exit returns an
+        input."""
         n, (h, w) = len(self), self.shape
-        clip = validate_accumulate_args(clip_length, cumulative, thresholded, n)
+        clip = validate_accumulate_args(clip_length, cumulative, thresholded, n, fold=fold)
         if n == 0:
             return FlowBatch._wrap(DeviceArray.empty((0, h, w, 2), np.float32), self.ref,
                                    DeviceArray.empty((0, h, w), np.uint8))
+        if fold is None:
+            fold = 'left' if self.ref == 's' else 'right'
         v, m = _ops.accumulate(self.vecs, self.masks, self.ref, DEFAULT_THRESHOLD if thresholded else 0.0, n // clip,
-                               clip, cumulative)
+                               clip, cumulative, fold)
         return FlowBatch._wrap(v, self.ref, m)
 
 

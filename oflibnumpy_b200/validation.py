@@ -157,7 +157,7 @@ def validate_matrix_args(dof, method, masked, hypotheses):
     return dof, method, masked, hypotheses
 
 
-def validate_accumulate_args(clip_length, cumulative, thresholded, batch_size):
+def validate_accumulate_args(clip_length, cumulative, thresholded, batch_size, fold=None):
     """Checks of FlowBatch.accumulate. Returns the clip length L: ``clip_length``, or the whole batch for None (1 for
     an empty batch)."""
     pre = "Error accumulating flows: "
@@ -165,6 +165,8 @@ def validate_accumulate_args(clip_length, cumulative, thresholded, batch_size):
         raise TypeError(pre + "Cumulative needs to be a boolean")
     if not isinstance(thresholded, bool):
         raise TypeError(pre + "Thresholded needs to be a boolean")
+    if fold is not None and not (isinstance(fold, str) and fold in ('left', 'right')):
+        raise ValueError(pre + "Fold needs to be 'left' or 'right', not {!r}".format(fold))
     if clip_length is None:
         return max(batch_size, 1)
     if isinstance(clip_length, bool) or not isinstance(clip_length, (int, np.integer)) or clip_length < 1 or \
