@@ -305,6 +305,26 @@ int ofk_accumulate_fold(const float* flow, const uint8_t* mask, int ref, int fol
                         int W, int cumulative, float* out, uint8_t* out_mask, void* ws, size_t ws_bytes,
                         ofk_stream_t stream);
 
+/* Forward-backward consistency check (Sundaram, Brox & Keutzer, ECCV 2010): occlusion masks of a pair of flows in one
+ * pass. F [N,H,W,2] is the forward flow (frame 1 -> frame 2), G [N,H,W,2] the backward flow (frame 2 -> frame 1), both
+ * of reference ref ('s' or 't'); the result is on F's grid. For every pixel p of frame n, in float32 with every
+ * operation rounded on its own (no FMA contraction):
+ *   sign = +1 ('s') or -1 ('t');  w = F[p];  (su, sv) = Q(G, p + sign * w)   (the cv2.remap sample of ofk_combine3)
+ *   valid = Fm[p] & strict(Gm at the taps)                                     (the mask ofk_combine3 writes)
+ *   ru = wu + su;  rv = wv + sv;  lhs = ru*ru + rv*rv
+ *   rhs = alpha1 * ((wu*wu + wv*wv) + (su*su + sv*sv)) + alpha2
+ *   out[p] = valid & (lhs < rhs);  out_valid[p] = valid
+ * (ru, rv) and valid are the vectors and mask of ofk_combine3(F, G, 's') for ref 's' and of ofk_combine3(G, F, 't')
+ * for ref 't'. There are no early exits: zero flows go through the same formula (with alpha2 = 0 a zero pair is not
+ * consistent, since 0 < 0 is false). Sundaram et al. use alpha1 = 0.01, alpha2 = 0.5.
+ *   Fm / Gm: uint8 0/1 masks, both given or both NULL (all valid). out, out_valid: uint8 [N,H,W]; out_valid may be
+ *   NULL. F and G 8-byte aligned. alpha1, alpha2 finite and >= 0. N <= 65535, H and W below 32768, H*W below 2^30.
+ * One launch whatever N: the TMA kernel of ofk_combine3 with a consistency epilogue where W % 16 == 0 and the operands
+ * are 16-byte aligned, else the gather (rows) kernel of ofk_combine3 with the same epilogue; OFK_C3_WS=0 forces the
+ * latter. Every argument is checked before any device work. */
+int ofk_consistency(const float* F, const uint8_t* Fm, const float* G, const uint8_t* Gm, int ref, float alpha1,
+                    float alpha2, uint8_t* out, uint8_t* out_valid, int N, int H, int W, ofk_stream_t stream);
+
 /* points_inside_area (utils.py:283-295): pts float64 [n][2] (row, col) rounded half-even like numpy.round. */
 int ofk_points_inside_area(const double* pts, size_t n, int H, int W, uint8_t* out, ofk_stream_t stream);
 
@@ -447,10 +467,12 @@ unsigned long long ofk_rt_launch_count(void);
  * kernels): which = 0 ofk_combine3 / TMA kernel, 1 ofk_combine3 / gather kernels, 2 ofk_warp_t / TMA kernels,
  * 3 ofk_warp_t / gather kernels. which = 4 / 5: inside the TMA kernels of ofk_combine3 / ofk_warp_t, how many
  * (warp, tile) pairs fetched taps from global memory because the tile's box did not cover them (discontinuous or noisy
- * flows); read synchronously from the current device. which = 6..9: ofk_forward_s, pixels outside the regular mesh
+ * flows); read synchronously from the current device. Counter 4 also counts ofk_consistency's TMA kernel, which is the
+ * same kernel. which = 6..9: ofk_forward_s, pixels outside the regular mesh
  * since process start: 6 located in a bridging / pocket triangle, 7 found outside the hull by the search, 8 searches
  * that did not terminate (treated as outside; expected 0), 9 rejected by the per-frame hull polygon, 10 pixels handed
- * to the warp-cooperative pocket pass, 11 its work items. */
+ * to the warp-cooperative pocket pass, 11 its work items. which = 12 / 13: ofk_consistency calls that ran the TMA
+ * kernel / the gather (rows) kernel. */
 unsigned long long ofk_rt_path_count(int which);
 
 #if defined(__GNUC__)

@@ -56,6 +56,7 @@ _SIGNATURES = {
     'ofk_accumulate': (_i, [_vp, _vp, _i, _f, _i, _i, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
     'ofk_accumulate_fold_workspace': (_sz, [_i, _i, _i, _i, _i, _i, _i]),
     'ofk_accumulate_fold': (_i, [_vp, _vp, _i, _i, _f, _i, _i, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
+    'ofk_consistency': (_i, [_vp, _vp, _vp, _vp, _i, _f, _f, _vp, _vp, _i, _i, _i, _vp]),
     'ofk_points_inside_area':(_i, [_vp, _sz, _i, _i, _vp, _vp]),
     'ofk_forward_s_workspace': (_sz, [_i, _i, _i]),
     'ofk_forward_s': (_i, [_vp, _i, _vp, _f, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _sz, _vp]),

@@ -407,3 +407,16 @@ def accumulate(flow, mask, ref, thr, s, l, cumulative, fold):
     _lib.call('ofk_accumulate_fold', flow.ptr, mask.ptr, ord(ref), ord(fold[0]), float(thr), s, l, h, w,
               int(cumulative), out.ptr, omask.ptr, ws.ptr, ws_bytes, dev.current_stream())
     return out, omask
+
+
+def consistency(f, fm, g, gm, ref, alpha_1, alpha_2, want_valid):
+    """Forward-backward consistency of every frame in one ofk_consistency call: forward flow f and backward flow g
+    [N,H,W,2] with masks [N,H,W]. Returns device uint8 arrays (consistent [N,H,W], valid [N,H,W] or None);
+    asynchronous, no launch for N = 0."""
+    n, h, w = f.shape[:3]
+    out = DeviceArray.empty((n, h, w), np.uint8)
+    valid = DeviceArray.empty((n, h, w), np.uint8) if want_valid else None
+    if n:
+        _lib.call('ofk_consistency', f.ptr, _p(fm), g.ptr, _p(gm), ord(ref), float(np.float32(alpha_1)),
+                  float(np.float32(alpha_2)), out.ptr, _p(valid), n, h, w, dev.current_stream())
+    return out, valid

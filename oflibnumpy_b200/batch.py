@@ -12,7 +12,8 @@ from . import device as dev
 from .device import DeviceArray
 from .flow import Flow
 from .validation import get_valid_ref, validate_shape, validate_transform_list, validate_visualise_args, \
-    validate_track_args, validate_track_dtype, validate_matrix_args, validate_accumulate_args, DEFAULT_THRESHOLD
+    validate_track_args, validate_track_dtype, validate_matrix_args, validate_accumulate_args, \
+    validate_consistency_args, DEFAULT_THRESHOLD
 
 __all__ = ['FlowBatch', 'shard_range', 'apply_flow_host', 'combine_flows_host', 'apply_combine_host',
            'visualise_flows_host']
@@ -360,6 +361,29 @@ class FlowBatch(object):
         v, m = _ops.accumulate(self.vecs, self.masks, self.ref, DEFAULT_THRESHOLD if thresholded else 0.0, n // clip,
                                clip, cumulative, fold)
         return FlowBatch._wrap(v, self.ref, m)
+
+    def consistent_with(self, other, alpha_1=None, alpha_2=None, return_valid_area=False):
+        """Forward-backward consistency check (Sundaram, Brox & Keutzer, ECCV 2010) of this batch, the forward flows
+        (frame 1 -> frame 2), with ``other``, the backward flows (frame 2 -> frame 1) of the same shape and ref, in one
+        ofk_consistency launch. For every pixel p, with w = self[p] and s = other sampled at p + w (ref 's') or p - w
+        (ref 't') the way ``combine_with(., 3)`` samples it:
+
+            consistent = valid & (|w + s|^2 < alpha_1 (|w|^2 + |s|^2) + alpha_2)
+
+        in float32, every operation rounded on its own; the defaults are alpha_1 = 0.01 and alpha_2 = 0.5. The result
+        is on self's grid: for ref 's' frame 1's, where 1 means the pixel of frame 1 is visible in frame 2; for ref 't'
+        frame 2's, where 1 means the pixel of frame 2 has a consistent source in frame 1. ``valid`` is the mask of
+        ``self.combine_with(other, 3)`` for ref 's' and of ``other.combine_with(self, 3)`` for ref 't' (self's mask
+        and other's mask at the taps, which must lie inside the frame); ``w + s`` are the vectors of that composition.
+        There are no early exits: zero flows go through the same formula, so with alpha_2 = 0 a zero pair is not
+        consistent (0 < 0 is false).
+
+        Returns a device uint8 array (N,H,W) of 0/1 (``.numpy()`` to download), and with ``return_valid_area`` also
+        ``valid``; the pixels occluded in the frame are ``valid & ~consistent``. No synchronisation, no read-back."""
+        a1, a2 = validate_consistency_args(self, other, alpha_1, alpha_2, return_valid_area, FlowBatch)
+        out, valid = _ops.consistency(self.vecs, self.masks, other.vecs, other.masks, self.ref, a1, a2,
+                                      return_valid_area)
+        return (out, valid) if return_valid_area else out
 
 
 def _track_range_fails(pts, lookup, is_int, status, h, w):

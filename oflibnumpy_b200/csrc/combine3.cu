@@ -7,6 +7,7 @@
 // warp (remap of vecs||mask) -> Flow construction -> add -> mask AND, i.e. five full-frame passes plus two masked
 // zero tests; here one kernel reads both operands once (27 B/px algorithmic) and also produces the zero-test flags
 // that gate the reference's early exits (flow_class.py:1338-1354), which a second tiny kernel applies on the device.
+#include <float.h>
 #include <stdlib.h>
 
 #include "combine3_device.cuh"
@@ -68,11 +69,15 @@ __device__ __forceinline__ void load_tile(TileIn& in, const float2* __restrict__
     }
 }
 
-template <bool REF_T, bool MASKS, bool FULL>
+// EPI (combine3_device.cuh): EPI_COMPOSE writes O and Om; EPI_CONSIST writes the consistency byte to Om and, if Ov
+// is not NULL, the valid byte to Ov (O is not used).
+template <bool REF_T, bool MASKS, bool FULL, int EPI = EPI_COMPOSE>
 __device__ __forceinline__ void process_tile(const TileIn& cur, const float2* __restrict__ G,
                                              const uint8_t* __restrict__ Gm, float2* __restrict__ O,
                                              uint8_t* __restrict__ Om, unsigned x, float Xg, unsigned y0, float tz,
-                                             int H, int W, unsigned& nzP, unsigned& nzG) {
+                                             int H, int W, unsigned& nzP, unsigned& nzG,
+                                             const EpiArgs<EPI>& epi = EpiArgs<EPI>{},
+                                             uint8_t* __restrict__ Ov = nullptr) {
     const float sign = REF_T ? -1.0f : 1.0f;
     // phase 1: zero tests and quantised sample coordinates of all rows (no control flow)
     float X[4], Y[4];
@@ -140,12 +145,18 @@ __device__ __forceinline__ void process_tile(const TileIn& cur, const float2* __
             const unsigned y = y0 + j;
             if (FULL || y < (unsigned)H) {
                 const unsigned idx = y * (unsigned)W + x;
-                float2 o;
-                o.x = __fadd_rn(cur.p[j].x, su[j]);
-                o.y = __fadd_rn(cur.p[j].y, sv[j]);
-                asm volatile("st.global.L1::no_allocate.v2.f32 [%0], {%1,%2};" ::"l"(O + idx), "f"(o.x), "f"(o.y)
-                             : "memory");
-                Om[idx] = (uint8_t)(cur.pmv[j] & strict[j]);
+                if constexpr (EPI == EPI_CONSIST) {
+                    const unsigned v = cur.pmv[j] & strict[j];
+                    Om[idx] = (uint8_t)(v & fb_consistent(cur.p[j].x, cur.p[j].y, su[j], sv[j], epi.a1, epi.a2));
+                    if (Ov != nullptr) Ov[idx] = (uint8_t)v;
+                } else {
+                    float2 o;
+                    o.x = __fadd_rn(cur.p[j].x, su[j]);
+                    o.y = __fadd_rn(cur.p[j].y, sv[j]);
+                    asm volatile("st.global.L1::no_allocate.v2.f32 [%0], {%1,%2};" ::"l"(O + idx), "f"(o.x), "f"(o.y)
+                                 : "memory");
+                    Om[idx] = (uint8_t)(cur.pmv[j] & strict[j]);
+                }
             }
         }
     }
@@ -175,12 +186,15 @@ struct TileIter {
     }
 };
 
-template <bool REF_T, bool MASKS, int MINB>
+// EPI_CONSIST (ofk_consistency): omask receives the consistency byte, epi.valid (if set) the valid byte; out is not
+// used and flags must be NULL.
+template <bool REF_T, bool MASKS, int MINB, int EPI = EPI_COMPOSE>
 __global__ void __launch_bounds__(256, MINB) combine3_rows(const float* __restrict__ A, const uint8_t* __restrict__ Am,
                                                            const float* __restrict__ B, const uint8_t* __restrict__ Bm,
                                                            float thr, float* __restrict__ out,
                                                            uint8_t* __restrict__ omask, int* __restrict__ flags, int H,
-                                                           int W, int tiles_x, int tiles_y, int N) {
+                                                           int W, int tiles_x, int tiles_y, int N,
+                                                           const EpiArgs<EPI> epi = EpiArgs<EPI>{}) {
     // zero test as one compare per component: |c| >= t with t = thr, or the smallest denormal for the exact test
     const float tz = thr > 0.f ? thr : 1.401298464e-45f;
     const unsigned lane = threadIdx.x & 31, wrp = threadIdx.x >> 5;
@@ -213,13 +227,25 @@ __global__ void __launch_bounds__(256, MINB) combine3_rows(const float* __restri
             load_tile<MASKS, false>(nxt, Pb + fb2, Gb + fb2, Pmb + fb2, Gmb + fb2, (unsigned)it.tx * 32 + lane,
                                     (unsigned)it.ty * 32 + wrp * 4, H, W);
         }
-        float2* O = reinterpret_cast<float2*>(out) + fbase;
-        uint8_t* Om = omask + fbase;
-        const float Xg = static_cast<float>(x);
-        if (full)
-            process_tile<REF_T, MASKS, true>(cur, Gb + fbase, Gmb + fbase, O, Om, x, Xg, y0, tz, H, W, nzP, nzG);
-        else
-            process_tile<REF_T, MASKS, false>(cur, Gb + fbase, Gmb + fbase, O, Om, x, Xg, y0, tz, H, W, nzP, nzG);
+        if constexpr (EPI == EPI_CONSIST) {
+            uint8_t* Om = omask + fbase;
+            uint8_t* Ov = epi.valid != nullptr ? epi.valid + fbase : nullptr;
+            const float Xg = static_cast<float>(x);
+            if (full)
+                process_tile<REF_T, MASKS, true, EPI>(cur, Gb + fbase, Gmb + fbase, nullptr, Om, x, Xg, y0, tz, H, W, nzP,
+                                                      nzG, epi, Ov);
+            else
+                process_tile<REF_T, MASKS, false, EPI>(cur, Gb + fbase, Gmb + fbase, nullptr, Om, x, Xg, y0, tz, H, W,
+                                                       nzP, nzG, epi, Ov);
+        } else {
+            float2* O = reinterpret_cast<float2*>(out) + fbase;
+            uint8_t* Om = omask + fbase;
+            const float Xg = static_cast<float>(x);
+            if (full)
+                process_tile<REF_T, MASKS, true>(cur, Gb + fbase, Gmb + fbase, O, Om, x, Xg, y0, tz, H, W, nzP, nzG);
+            else
+                process_tile<REF_T, MASKS, false>(cur, Gb + fbase, Gmb + fbase, O, Om, x, Xg, y0, tz, H, W, nzP, nzG);
+        }
         // publish the zero-test result when this CTA leaves the frame (clamped duplicates of partial tiles repeat
         // pixels of the same frame, so they cannot create false positives)
         if (flags != nullptr && (!more || it.n != n)) {
@@ -327,6 +353,8 @@ int launch_combine3_ws(const float* P, const uint8_t* Pm, const float* G, const 
                        float* out, uint8_t* omask, int N, int H, int W, cudaStream_t st);
 int launch_c3_zero_flags(const float* A, const uint8_t* Am, const float* B, const uint8_t* Bm, float thr, int* flags,
                          int N, int H, int W, cudaStream_t st);
+int launch_consistency_ws(const float* F, const uint8_t* Fm, const float* G, const uint8_t* Gm, float sign, float a1,
+                          float a2, uint8_t* out, uint8_t* out_valid, int N, int H, int W, cudaStream_t st);
 bool c3_ws_enabled();
 }
 
@@ -410,5 +438,56 @@ extern "C" int ofk_combine3(const float* A, const uint8_t* Am, const float* B, c
         combine3_fixup<<<dim3(bx, N), 256, 0, st>>>(A, Am, B, Bm, flags, out, out_mask, frame);
         OFK_LAUNCHED();
     }
+    return OFK_OK;
+}
+
+// Forward-backward consistency of F (forward) and G (backward): one launch of the TMA kernel or of the rows kernel with
+// the consistency epilogue; no zero tests, no early exits.
+extern "C" int ofk_consistency(const float* F, const uint8_t* Fm, const float* G, const uint8_t* Gm, int ref,
+                               float alpha1, float alpha2, uint8_t* out, uint8_t* out_valid, int N, int H, int W,
+                               ofk_stream_t stream) {
+    OFK_CHECK_ARG(F && G && out, "ofk_consistency: NULL pointer (F=%p G=%p out=%p)", (void*)F, (void*)G, (void*)out);
+    OFK_CHECK_ARG((Fm == nullptr) == (Gm == nullptr), "ofk_consistency: Fm and Gm must both be given or both be NULL");
+    OFK_CHECK_ARG(ref == 's' || ref == 't', "ofk_consistency: ref must be 's' or 't', got %d", ref);
+    OFK_CHECK_ARG(alpha1 >= 0.f && alpha1 <= FLT_MAX && alpha2 >= 0.f && alpha2 <= FLT_MAX,
+                  "ofk_consistency: alpha1 and alpha2 must be finite and >= 0 (alpha1=%g alpha2=%g)", (double)alpha1,
+                  (double)alpha2);
+    OFK_CHECK_ARG(N >= 0 && H > 0 && W > 0 && H < 32768 && W < 32768 && (long long)H * W < (1ll << 30),
+                  "ofk_consistency: bad shape N=%d H=%d W=%d (H and W below 32768, H*W below 2^30)", N, H, W);
+    OFK_CHECK_ARG(N <= 65535, "ofk_consistency: N=%d exceeds 65535 frames per call", N);
+    OFK_CHECK_ARG(((reinterpret_cast<uintptr_t>(F) | reinterpret_cast<uintptr_t>(G)) & 7) == 0,
+                  "ofk_consistency: F and G must be 8-byte aligned (F=%p G=%p)", (void*)F, (void*)G);
+    if (N == 0) return OFK_OK;
+    cudaStream_t st = as_stream(stream);
+    const float sign = ref == 't' ? -1.0f : 1.0f;
+    // the TMA kernel where the tensor maps accept the operands (W % 16 == 0, 16-byte aligned), else the rows kernel
+    int ws = 0;
+    if (c3_ws_enabled()) {
+        ws = launch_consistency_ws(F, Fm, G, Gm, sign, alpha1, alpha2, out, out_valid, N, H, W, st);
+        if (ws < 0) return ws;
+    }
+    g_consistency_paths[ws == 1 ? 0 : 1].fetch_add(1, std::memory_order_relaxed);
+    if (ws == 1) return OFK_OK;
+    EpiArgs<EPI_CONSIST> epi;
+    epi.a1 = alpha1;
+    epi.a2 = alpha2;
+    epi.valid = out_valid;
+    const int tiles_x = (W + 31) / 32, tiles_y = (H + 31) / 32;
+    long long grid = (long long)sm_count() * 2;   // every CTA co-resident, as the composition's default
+    if (grid > (long long)tiles_x * tiles_y * N) grid = (long long)tiles_x * tiles_y * N;
+    // combine3_rows reads P = B, G = A for REF_T, P = A, G = B otherwise: here P is always F
+#define OFK_CONS(RT, MK)                                                                                          \
+    combine3_rows<RT, MK, 2, EPI_CONSIST><<<(unsigned)grid, 256, 0, st>>>(RT ? G : F, RT ? Gm : Fm, RT ? F : G, \
+                                                                          RT ? Fm : Gm, 0.f, nullptr, out,     \
+                                                                          nullptr, H, W, tiles_x, tiles_y, N, epi)
+    if (Fm != nullptr) {
+        if (ref == 't') OFK_CONS(true, true);
+        else OFK_CONS(false, true);
+    } else {
+        if (ref == 't') OFK_CONS(true, false);
+        else OFK_CONS(false, false);
+    }
+#undef OFK_CONS
+    OFK_LAUNCHED();
     return OFK_OK;
 }

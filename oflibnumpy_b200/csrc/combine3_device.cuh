@@ -5,6 +5,33 @@
 
 namespace ofk {
 
+// Epilogues of the sampling kernels (c3_ws_kernel, combine3_rows): what a pixel writes once s = Q(G, p + sign*P[p])
+// and its validity (P mask & strict G mask at the taps) are known.
+constexpr int EPI_SAMPLE = 0;    // out = s, mask = valid                    (Flow.apply of a flow, ofk_warp_t)
+constexpr int EPI_COMPOSE = 1;   // out = P + s, mask = valid                (ofk_combine3)
+constexpr int EPI_CONSIST = 2;   // out = valid & fb_consistent(P, s), one byte; optionally valid (ofk_consistency)
+
+// Kernel arguments of an epilogue: none for sample and compose, so that their kernels keep their code.
+template <int EPI>
+struct EpiArgs {};
+template <>
+struct EpiArgs<EPI_CONSIST> {
+    float a1, a2;
+    uint8_t* valid;   // NULL: the valid byte is not written
+};
+
+// Forward-backward consistency (Sundaram, Brox & Keutzer, ECCV 2010) of w = P[p] and the sampled backward flow s:
+//   |w + s|^2 < a1 (|w|^2 + |s|^2) + a2
+// in float32, every operation rounded on its own (no FMA contraction), in this order.
+__device__ __forceinline__ unsigned fb_consistent(float wu, float wv, float su, float sv, float a1, float a2) {
+    const float ru = __fadd_rn(wu, su), rv = __fadd_rn(wv, sv);
+    const float lhs = __fadd_rn(__fmul_rn(ru, ru), __fmul_rn(rv, rv));
+    const float ww = __fadd_rn(__fmul_rn(wu, wu), __fmul_rn(wv, wv));
+    const float ss = __fadd_rn(__fmul_rn(su, su), __fmul_rn(sv, sv));
+    const float rhs = __fadd_rn(__fmul_rn(a1, __fadd_rn(ww, ss)), a2);
+    return lhs < rhs ? 1u : 0u;
+}
+
 struct SampleResult {
     float u, v;
     int strict;

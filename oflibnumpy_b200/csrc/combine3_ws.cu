@@ -25,6 +25,7 @@
 
 #include <type_traits>
 
+#include "combine3_device.cuh"
 #include "ws_common.cuh"
 
 namespace ofk {
@@ -94,17 +95,49 @@ __device__ __forceinline__ void quant(float X, int& i, int& f) {
     f = bits & 31;
 }
 
+// What pixel j of this thread writes (EPI_* of combine3_device.cuh): p = P[p], s = Q(G, ...) packed, v = its validity
+// byte. The consistency epilogue writes its byte over the P mask tile (the mask store) and keeps the valid byte in vb.
+template <int EPI>
+__device__ __forceinline__ void epilogue(float2* prow, uint8_t* mrow, int j, uint64_t p, uint64_t s, unsigned v,
+                                         unsigned& vb, const EpiArgs<EPI>& epi) {
+    if constexpr (EPI == EPI_CONSIST) {
+        const float2 w = unpack2(p), q = unpack2(s);
+        mrow[j * TS] = (uint8_t)(v & fb_consistent(w.x, w.y, q.x, q.y, epi.a1, epi.a2));
+        vb = v;
+    } else {
+        *reinterpret_cast<uint64_t*>(prow + j * TS) = EPI == EPI_COMPOSE ? add2(p, s) : s;
+        mrow[j * TS] = (uint8_t)v;
+    }
+}
+// The consistency epilogue's valid bytes go out through the vector map slot, staged in the warp's own 4 P vector rows
+// (4 x 32 bytes from the start of its first row). Lanes overwrite vectors of other lanes there, so the warp first makes
+// sure that every lane has read its vectors. prow: this lane's first pixel in the P stage.
+template <int EPI>
+__device__ __forceinline__ void stage_valid(float2* prow, const unsigned (&vb)[4], const EpiArgs<EPI>& epi) {
+    if constexpr (EPI == EPI_CONSIST) {
+        __syncwarp();
+        if (epi.valid != nullptr) {
+            const unsigned lane = threadIdx.x & 31;
+            uint8_t* vrow = reinterpret_cast<uint8_t*>(prow - lane) + lane;
+#pragma unroll
+            for (int j = 0; j < 4; ++j) vrow[j * TS] = (uint8_t)vb[j];
+        }
+    }
+}
+
 // The global-tap path (out of line, see mixed_rows): taps of a warp's 4 x 32 pixels, all requested before the first
 // use -- from the box for the pixels it covers, from global memory for the others, predicated per tap on "inside the
 // frame" (zero border, mask invalid outside) -- then validity, release of the box, blend: one memory round trip per
 // warp and tile and the same arithmetic as the main path, so the result never depends on the box estimate.
-template <bool MASKS, bool ADD, class BStage>
+template <bool MASKS, int EPI, class BStage>
 __device__ __forceinline__ void sample_rows_mixed(const BStage& bs, float2* prow, uint8_t* mrow, const uint64_t (&p)[4],
                                             const unsigned (&pm)[4], const int (&dx)[4], const int (&dy)[4],
                                             const int (&fa)[4], const int (&fb)[4], int4 info, int n,
                                             const float2* __restrict__ G, const uint8_t* __restrict__ Gm, int H, int W,
-                                            uint64_t negzero2, uint64_t* bempty, uint32_t* sink, unsigned lane) {
+                                            uint64_t negzero2, uint64_t* bempty, uint32_t* sink, unsigned lane,
+                                            const EpiArgs<EPI>& epi) {
     const uint64_t one2 = pack2(1.0f, 1.0f);
+    unsigned vb[4];
     uint64_t t[4][4];
     unsigned m[4][4];
 #pragma unroll
@@ -168,9 +201,9 @@ __device__ __forceinline__ void sample_rows_mixed(const BStage& bs, float2* prow
         accv = add2(accv, mul2_nofuse(t[j][1], mul2(fa2, nb2), negzero2));
         accv = add2(accv, mul2_nofuse(t[j][2], mul2(na2, fb2), negzero2));
         accv = add2(accv, mul2_nofuse(t[j][3], mul2(fa2, fb2), negzero2));
-        *reinterpret_cast<uint64_t*>(prow + j * TS) = ADD ? add2(p[j], accv) : accv;
-        mrow[j * TS] = (uint8_t)(strict[j] & 1u);
+        epilogue<EPI>(prow, mrow, j, p[j], accv, strict[j] & 1u, vb[j], epi);
     }
+    stage_valid<EPI>(prow, vb, epi);
 }
 
 // this thread's four pixels of a tile: operand values, sample positions relative to the box, 1/32-px fractions;
@@ -203,10 +236,17 @@ __device__ __forceinline__ bool prepare_rows(const float2* prow, const uint8_t* 
 // preparation from shared memory and samples with sample_rows_mixed.
 static __device__ unsigned long long g_mixed_warp_tiles;   // test hook: how often the out-of-line path ran (per warp and tile)
 
-template <bool MASKS, bool ADD, class SM>
+// (epi: the EpiArgs of the consistency epilogue, nothing otherwise, so that the other kernels keep their calls)
+template <int EPI>
+__device__ __forceinline__ EpiArgs<EPI> epi_args() { return EpiArgs<EPI>{}; }
+template <int EPI>
+__device__ __forceinline__ EpiArgs<EPI> epi_args(const EpiArgs<EPI>& e) { return e; }
+
+template <bool MASKS, int EPI, class SM, class... E>
 __device__ __noinline__ void mixed_rows(typename SM::PStage* ps, const typename SM::BStage* bs, uint64_t* bempty,
                                         uint32_t* sink, int4 info, int4 tile, const float2* __restrict__ G,
-                                        const uint8_t* __restrict__ Gm, float sign, int H, int W, uint64_t negzero2) {
+                                        const uint8_t* __restrict__ Gm, float sign, int H, int W, uint64_t negzero2,
+                                        E... epi) {
     const unsigned lane = threadIdx.x & 31, wrp = threadIdx.x >> 5;
     if (lane == 0) atomicAdd(&g_mixed_warp_tiles, 1ull);
     float2* prow = ps->p + ((int)wrp * 4 * TS + lane);
@@ -216,17 +256,20 @@ __device__ __noinline__ void mixed_rows(typename SM::PStage* ps, const typename 
     int dx[4], dy[4], fa[4], fb[4];
     prepare_rows<MASKS>(prow, mrow, sign, (float)(tile.x + (int)lane), (float)(tile.y + (int)wrp * 4), info, p, pm, dx, dy,
                         fa, fb);
-    sample_rows_mixed<MASKS, ADD>(*bs, prow, mrow, p, pm, dx, dy, fa, fb, info, tile.z, G, Gm, H, W, negzero2, bempty,
-                                        sink, lane);
+    sample_rows_mixed<MASKS, EPI>(*bs, prow, mrow, p, pm, dx, dy, fa, fb, info, tile.z, G, Gm, H, W, negzero2, bempty,
+                                  sink, lane, epi_args<EPI>(epi...));
 }
 
-// ADD: out = P + Q(G, ...) (composition); otherwise out = Q(G, ...) alone (Flow.apply of a flow: ofk_warp_t, float32 x2)
-template <bool MASKS, bool ADD, int NP, int NB, int LA, int PW>
+// EPI (combine3_device.cuh): EPI_COMPOSE out = P + Q(G, ...) (composition); EPI_SAMPLE out = Q(G, ...) alone (Flow.apply
+// of a flow: ofk_warp_t, float32 x2); EPI_CONSIST the consistency byte through maps.om and, when epi.valid is set, the
+// valid byte through maps.ov (a uint8 map then); no vector store.
+template <bool MASKS, int EPI, int NP, int NB, int LA, int PW>
 __global__ void __launch_bounds__((NCW + PW) * 32, 2) c3_ws_kernel(const __grid_constant__ Maps maps,
                                                                const float2* __restrict__ G,
                                                                const uint8_t* __restrict__ Gm, float sign,
                                                                int H, int W, unsigned tiles_x, unsigned tiles_per_frame,
-                                                               unsigned total_tiles, uint64_t negzero2) {
+                                                               unsigned total_tiles, uint64_t negzero2,
+                                                               const EpiArgs<EPI> epi) {
     // a P stage is released one tile late (its rows double as the staging buffer of the output store)
     static_assert(NP >= NB + LA + 1, "P stages must outlive the box pipeline and the output store");
     using SM = Smem<NP, NB>;
@@ -380,6 +423,7 @@ __global__ void __launch_bounds__((NCW + PW) * 32, 2) c3_ws_kernel(const __grid_
             // [-2^16, 2^16], so such a pixel can never pass the box test (frames are smaller than 32768).
             ok = ok && (unsigned)dx[j] < (unsigned)(BW - 1) && (unsigned)dy[j] < (unsigned)(BH - 1);
         }
+        unsigned vb[4];   // valid bytes of the consistency epilogue
         if (__all_sync(0xffffffffu, ok)) {
             uint64_t t[4][4];
             unsigned m[4][4];
@@ -425,9 +469,9 @@ __global__ void __launch_bounds__((NCW + PW) * 32, 2) c3_ws_kernel(const __grid_
                 accv = add2(accv, mul2_nofuse(t[j][1], mul2(fa2, nb2), negzero2));
                 accv = add2(accv, mul2_nofuse(t[j][2], mul2(na2, fb2), negzero2));
                 accv = add2(accv, mul2_nofuse(t[j][3], mul2(fa2, fb2), negzero2));
-                *reinterpret_cast<uint64_t*>(prow + j * TS) = ADD ? add2(p[j], accv) : accv;
-                mrow[j * TS] = (uint8_t)(strict[j] & 1u);
+                epilogue<EPI>(prow, mrow, j, p[j], accv, strict[j] & 1u, vb[j], epi);
             }
+            stage_valid<EPI>(prow, vb, epi);
         } else {
             // Some pixel of this warp is not covered by the box. Along the frame border that is the rule (the box is
             // clamped to the frame): those pixels sample nothing but the zero border. Pixels that need taps from inside
@@ -441,7 +485,12 @@ __global__ void __launch_bounds__((NCW + PW) * 32, 2) c3_ws_kernel(const __grid_
                 need_global = need_global || !(inbox || ix < -1 || iy < -1 || ix >= W || iy >= H);
             }
             if (__any_sync(0xffffffffu, need_global)) {
-                mixed_rows<MASKS, ADD, SM>(&ps, &bs, &sm.bempty[b], &sm.sink[wrp], info, tile, G, Gm, sign, H, W, negzero2);
+                if constexpr (EPI == EPI_CONSIST)
+                    mixed_rows<MASKS, EPI, SM>(&ps, &bs, &sm.bempty[b], &sm.sink[wrp], info, tile, G, Gm, sign, H, W,
+                                               negzero2, epi);
+                else
+                    mixed_rows<MASKS, EPI, SM>(&ps, &bs, &sm.bempty[b], &sm.sink[wrp], info, tile, G, Gm, sign, H, W,
+                                               negzero2);
             } else {
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
@@ -470,9 +519,16 @@ __global__ void __launch_bounds__((NCW + PW) * 32, 2) c3_ws_kernel(const __grid_
                         sv = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(t00.y, f00), __fmul_rn(t01.y, f01)),
                                                  __fmul_rn(t10.y, f10)), __fmul_rn(t11.y, f11));
                     }
-                    prow[j * TS] = ADD ? make_float2(__fadd_rn(pv.x, su), __fadd_rn(pv.y, sv)) : make_float2(su, sv);
-                    mrow[j * TS] = (uint8_t)(pm[j] & strict & 1u);
+                    if constexpr (EPI == EPI_CONSIST) {
+                        vb[j] = pm[j] & strict & 1u;
+                        mrow[j * TS] = (uint8_t)(vb[j] & fb_consistent(pv.x, pv.y, su, sv, epi.a1, epi.a2));
+                    } else {
+                        prow[j * TS] = EPI == EPI_COMPOSE ? make_float2(__fadd_rn(pv.x, su), __fadd_rn(pv.y, sv))
+                                                          : make_float2(su, sv);
+                        mrow[j * TS] = (uint8_t)(pm[j] & strict & 1u);
+                    }
                 }
+                stage_valid<EPI>(prow, vb, epi);
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&sm.bempty[b]);
             }
@@ -483,8 +539,10 @@ __global__ void __launch_bounds__((NCW + PW) * 32, 2) c3_ws_kernel(const __grid_
         // (issued under elect.sync: the compiler moves the operands to uniform registers without a waterfall loop)
         const int u_tx = tx0, u_ty = ty0 + (int)wrp * 4, u_n = n;
         const uint32_t u_src = smem_u32(ps.p + (int)wrp * 4 * TS), u_srcm = smem_u32(ps.pm + (int)wrp * 4 * TS);
+        bool vec_store = true;
+        if constexpr (EPI == EPI_CONSIST) vec_store = epi.valid != nullptr;
         if (elect_one()) {
-            tma_store_3d_u(&maps.ov, u_src, u_tx, u_ty, u_n);
+            if (vec_store) tma_store_3d_u(&maps.ov, u_src, u_tx, u_ty, u_n);
             tma_store_3d_u(&maps.om, u_srcm, u_tx, u_ty, u_n);
             bulk_commit();
             if (prev_s >= 0) {
@@ -603,24 +661,26 @@ int launch_c3_zero_flags(const float* A, const uint8_t* Am, const float* B, cons
     return OFK_OK;
 }
 
-// Returns 1 if the kernel was launched, 0 if the configuration is not eligible (caller uses the rows kernel),
-// negative OFK_E* on error. P/G are the pointwise / gathered operands, sign = -1 ('t') or +1 ('s').
-int launch_combine3_ws(const float* P, const uint8_t* Pm, const float* G, const uint8_t* Gm, float sign, bool add,
-                       float* out, uint8_t* omask, int N, int H, int W, cudaStream_t st) {
-    using namespace c3ws;
-    const bool masks = Pm != nullptr && Gm != nullptr;
-    if ((Pm == nullptr) != (Gm == nullptr)) return 0;
-    if (W % 16 != 0) return 0;   // 16-byte row pitch of the uint8 tensors (output mask always, input masks if given)
-    if (H >= 32768 || W >= 32768) return 0;
-    Maps maps;
-    if (!make_map3(&maps.p, P, 8, W, H, N, TS, TS) || !make_map3(&maps.gb, G, 8, W, H, N, BW, BH) ||
-        !make_map3(&maps.ov, out, 8, W, H, N, TS, 4) || !make_map3(&maps.om, omask, 1, W, H, N, TS, 4))
-        return 0;
-    if (masks) {
-        if (!make_map3(&maps.pm, Pm, 1, W, H, N, TS, TS) || !make_map3(&maps.gmb, Gm, 1, W, H, N, BMW, BH)) return 0;
+namespace c3ws {
+// Maps of the pointwise operand, its mask and the gathered operand and its mask; false if an operand does not fit the
+// TMA kernel (caller uses the rows kernel)
+static bool input_maps(Maps& maps, const float* P, const uint8_t* Pm, const float* G, const uint8_t* Gm, int N, int H,
+                       int W) {
+    if ((Pm == nullptr) != (Gm == nullptr)) return false;
+    if (W % 16 != 0) return false;   // 16-byte row pitch of the uint8 tensors (output mask always, input masks if given)
+    if (H >= 32768 || W >= 32768) return false;
+    if (!make_map3(&maps.p, P, 8, W, H, N, TS, TS) || !make_map3(&maps.gb, G, 8, W, H, N, BW, BH)) return false;
+    if (Pm != nullptr) {
+        if (!make_map3(&maps.pm, Pm, 1, W, H, N, TS, TS) || !make_map3(&maps.gmb, Gm, 1, W, H, N, BMW, BH)) return false;
     } else {
         maps.pm = maps.gmb = maps.p;
     }
+    return true;
+}
+
+template <bool MK, int EPI>
+static int launch_ws(const Maps& maps, const float* G, const uint8_t* Gm, float sign, int N, int H, int W,
+                     const EpiArgs<EPI>& epi, cudaStream_t st) {
     const unsigned tx = (W + TS - 1) / TS, ty = (H + TS - 1) / TS;
     if ((double)tx * ty * N >= 4.0e9) return 0;
     const unsigned total = tx * ty * (unsigned)N;
@@ -628,28 +688,60 @@ int launch_combine3_ws(const float* P, const uint8_t* Pm, const float* G, const 
     if (grid > total) grid = total;
     grid = ws::cap_ctas(grid);
     const size_t smem = sizeof(Smem<WS_NP, WS_NB>);
-#define OFK_WS(MK, AD)                                                                                                  \
-    do {                                                                                                              \
-        static std::atomic<bool> attr_done_dev[64];   /* the attribute is per device; racing threads set it twice */ \
-        int dev_ = 0;                                                                                                 \
-        if (cudaGetDevice(&dev_) != cudaSuccess || dev_ < 0 || dev_ >= 64) return 0;                                  \
-        std::atomic<bool>& attr_done = attr_done_dev[dev_];                                                           \
-        if (!attr_done) {                                                                                             \
-            if (cudaFuncSetAttribute(c3_ws_kernel<MK, AD, WS_NP, WS_NB, WS_LA, WS_PW>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                     (int)smem) != cudaSuccess) {                                                     \
-                cudaGetLastError();                                                                                   \
-                return 0;                                                                                             \
-            }                                                                                                         \
-            attr_done = true;                                                                                         \
-        }                                                                                                             \
-        c3_ws_kernel<MK, AD, WS_NP, WS_NB, WS_LA, WS_PW><<<grid, (NCW + WS_PW) * 32, smem, st>>>(                                    \
-            maps, (const float2*)G, Gm, sign, H, W, tx, tx * ty, total, 0x8000000080000000ull);                       \
-    } while (0)
-    if (masks) { if (add) OFK_WS(true, true); else OFK_WS(true, false); }
-    else { if (add) OFK_WS(false, true); else OFK_WS(false, false); }
-#undef OFK_WS
+    static std::atomic<bool> attr_done_dev[64];   // the attribute is per device; racing threads set it twice
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return 0;
+    std::atomic<bool>& attr_done = attr_done_dev[dev];
+    if (!attr_done) {
+        if (cudaFuncSetAttribute(c3_ws_kernel<MK, EPI, WS_NP, WS_NB, WS_LA, WS_PW>,
+                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
+            cudaGetLastError();
+            return 0;
+        }
+        attr_done = true;
+    }
+    c3_ws_kernel<MK, EPI, WS_NP, WS_NB, WS_LA, WS_PW><<<grid, (NCW + WS_PW) * 32, smem, st>>>(
+        maps, (const float2*)G, Gm, sign, H, W, tx, tx * ty, total, 0x8000000080000000ull, epi);
     OFK_LAUNCHED();
     return 1;
+}
+}  // namespace c3ws
+
+// Returns 1 if the kernel was launched, 0 if the configuration is not eligible (caller uses the rows kernel),
+// negative OFK_E* on error. P/G are the pointwise / gathered operands, sign = -1 ('t') or +1 ('s').
+int launch_combine3_ws(const float* P, const uint8_t* Pm, const float* G, const uint8_t* Gm, float sign, bool add,
+                       float* out, uint8_t* omask, int N, int H, int W, cudaStream_t st) {
+    using namespace c3ws;
+    Maps maps;
+    if (!input_maps(maps, P, Pm, G, Gm, N, H, W) || !make_map3(&maps.ov, out, 8, W, H, N, TS, 4) ||
+        !make_map3(&maps.om, omask, 1, W, H, N, TS, 4))
+        return 0;
+    const EpiArgs<EPI_COMPOSE> compose{};
+    const EpiArgs<EPI_SAMPLE> sample{};
+    if (Pm != nullptr) return add ? launch_ws<true>(maps, G, Gm, sign, N, H, W, compose, st)
+                                  : launch_ws<true>(maps, G, Gm, sign, N, H, W, sample, st);
+    return add ? launch_ws<false>(maps, G, Gm, sign, N, H, W, compose, st)
+               : launch_ws<false>(maps, G, Gm, sign, N, H, W, sample, st);
+}
+
+// The consistency check of ofk_consistency through the TMA kernel: P = F, G = G, out / out_valid uint8 [N,H,W]
+// (out_valid may be NULL). Returns as launch_combine3_ws.
+int launch_consistency_ws(const float* F, const uint8_t* Fm, const float* G, const uint8_t* Gm, float sign, float a1,
+                          float a2, uint8_t* out, uint8_t* out_valid, int N, int H, int W, cudaStream_t st) {
+    using namespace c3ws;
+    Maps maps;
+    if (!input_maps(maps, F, Fm, G, Gm, N, H, W) || !make_map3(&maps.om, out, 1, W, H, N, TS, 4)) return 0;
+    if (out_valid != nullptr) {
+        if (!make_map3(&maps.ov, out_valid, 1, W, H, N, TS, 4)) return 0;
+    } else {
+        maps.ov = maps.om;   // not used
+    }
+    EpiArgs<EPI_CONSIST> epi;
+    epi.a1 = a1;
+    epi.a2 = a2;
+    epi.valid = out_valid;
+    return Fm != nullptr ? launch_ws<true>(maps, G, Gm, sign, N, H, W, epi, st)
+                         : launch_ws<false>(maps, G, Gm, sign, N, H, W, epi, st);
 }
 
 }  // namespace ofk

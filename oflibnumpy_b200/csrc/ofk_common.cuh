@@ -13,6 +13,7 @@ namespace ofk {
 void set_error(const char* fmt, ...);
 extern std::atomic<unsigned long long> g_launches;
 extern std::atomic<unsigned long long> g_paths[4];   // see ofk_rt_path_count
+extern std::atomic<unsigned long long> g_consistency_paths[2];   // ofk_consistency: TMA kernel, rows kernel
 int staged_copy(void* dst, const void* src, size_t bytes, bool to_device, cudaStream_t user);   // staging.cu
 unsigned long long c3_ws_mixed_count();               // combine3_ws.cu
 unsigned long long warp_ws_mixed_count();             // warp_t_ws.cu

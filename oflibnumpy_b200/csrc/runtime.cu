@@ -14,6 +14,7 @@ namespace ofk {
 static thread_local char t_error[512] = "";
 std::atomic<unsigned long long> g_launches{0};
 std::atomic<unsigned long long> g_paths[4];
+std::atomic<unsigned long long> g_consistency_paths[2];
 
 void set_error(const char* fmt, ...) {
     va_list ap;
@@ -45,6 +46,7 @@ extern "C" unsigned long long ofk_rt_path_count(int which) {
     if (which >= 0 && which < 4) return g_paths[which].load();
     if (which == 4) return c3_ws_mixed_count();      // synchronous reads of device counters (current device)
     if (which == 5) return warp_ws_mixed_count();
+    if (which == 12 || which == 13) return g_consistency_paths[which - 12].load();
     if (which >= 6 && which <= 21) return forward_s_stat(which - 6);
     return 0ull;
 }

@@ -17,7 +17,7 @@ from . import _ops
 from . import device as dev
 from .device import DeviceArray
 from .validation import get_valid_ref, get_valid_padding, validate_shape, validate_visualise_args, \
-    validate_track_args, DEFAULT_THRESHOLD
+    validate_track_args, validate_consistency_args, DEFAULT_THRESHOLD
 
 __all__ = ['Flow']
 
@@ -686,6 +686,17 @@ class Flow(object):
         # sequence behind ofk_combine12, including the zero-flow tests inside switch_ref and apply_flow
         v, m = _ops.combine12(mode, self._ref, self._vd(), self._md(), flow._vd(), flow._md())
         return Flow._wrap(v, self._ref, m)
+
+    def consistent_with(self, flow, alpha_1=None, alpha_2=None, return_valid_area=None):
+        """Forward-backward consistency check of this flow (forward, frame 1 -> frame 2) with ``flow`` (backward, frame
+        2 -> frame 1): ``FlowBatch.consistent_with`` of the one frame, through the same call. Returns a numpy bool
+        array (H,W), and with ``return_valid_area`` also the valid area."""
+        return_valid_area = False if return_valid_area is None else return_valid_area
+        a1, a2 = validate_consistency_args(self, flow, alpha_1, alpha_2, return_valid_area, Flow)
+        out, valid = _ops.consistency(self._vd(), self._md(), flow._vd(), flow._md(), self._ref, a1, a2,
+                                      return_valid_area)
+        out = out.numpy()[0].view(np.bool_)
+        return (out, valid.numpy()[0].view(np.bool_)) if return_valid_area else out
 
 
 def _ones_mask(shape):

@@ -1,6 +1,7 @@
 """Argument validators of the public API. Types of exception and message texts are the reference's
 (utils.py:25-88 of oflibnumpy) because they are part of the drop-in contract; the checks run on the host before any
 device call."""
+import numbers
 import warnings
 
 import numpy as np
@@ -174,3 +175,33 @@ def validate_accumulate_args(clip_length, cumulative, thresholded, batch_size, f
         raise ValueError(pre + "Clip_length needs to be a positive integer that divides the batch size {}, not {!r}"
                          .format(batch_size, clip_length))
     return int(clip_length)
+
+
+def validate_consistency_args(flow, other, alpha_1, alpha_2, return_valid_area, flow_type):
+    """Checks of Flow.consistent_with / FlowBatch.consistent_with: ``other`` an instance of ``flow_type`` of the same
+    shape and reference as ``flow``, alphas real, finite and non-negative (also once rounded to float32, the precision
+    of the check), ``return_valid_area`` a boolean. Returns (alpha_1, alpha_2) as floats, with the defaults of Sundaram
+    et al. (0.01, 0.5) for None."""
+    pre = "Error checking flow consistency: "
+    if not isinstance(other, flow_type):
+        raise TypeError(pre + "Flow need to be of type '{}'".format(flow_type.__name__))
+    def full_shape(f):   # (N, H, W) of a FlowBatch, (H, W) of a Flow
+        return ((len(f),) if hasattr(f, '__len__') else ()) + tuple(f.shape)
+
+    if full_shape(flow) != full_shape(other):
+        raise ValueError(pre + "Flow fields need to have the same shape")
+    if flow.ref != other.ref:
+        raise ValueError(pre + "Flow fields need to have the same reference")
+    alphas = []
+    for name, a, default in (('Alpha_1', alpha_1, 0.01), ('Alpha_2', alpha_2, 0.5)):
+        a = default if a is None else a
+        ok = not isinstance(a, (bool, np.bool_)) and isinstance(a, numbers.Real)
+        if ok:
+            with np.errstate(over='ignore'):
+                ok = bool(np.isfinite(float(a)) and float(a) >= 0 and np.isfinite(np.float32(a)))
+        if not ok:
+            raise ValueError(pre + "{} needs to be a non-negative finite number, not {!r}".format(name, a))
+        alphas.append(float(a))
+    if not isinstance(return_valid_area, bool):
+        raise TypeError(pre + "Return_valid_area needs to be a boolean")
+    return alphas[0], alphas[1]
