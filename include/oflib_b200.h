@@ -102,6 +102,14 @@ int ofk_version(void);
 int ofk_warp_t(const void* payload, int dtype, int C, int arith, const float* flow, float flow_sign,
                const uint8_t* payload_mask, const uint8_t* flow_mask, void* out, uint8_t* out_mask, int mask_rule,
                int N, int H, int W, int Hs, int Ws, int top, int left, int cut, ofk_stream_t stream);
+/* ofk_warp_t_ex: flow_nonzero (int32 [N], device, e.g. from ofk_nonzero_flags(flow, NULL, 1e-3)) or NULL; frames
+ * with 0 get the payload itself (its flow-frame window when cut) like apply_flow's early return for a flow that is zero
+ * below the threshold (utils.py:215-216). out_mask is the same either way. Integer payloads do not need the flags:
+ * identity taps reproduce them exactly; float payloads do (NaN / Inf on a zero-weight tap, -0.0). */
+int ofk_warp_t_ex(const void* payload, int dtype, int C, int arith, const float* flow, float flow_sign,
+                  const uint8_t* payload_mask, const uint8_t* flow_mask, const int* flow_nonzero, void* out,
+                  uint8_t* out_mask, int mask_rule, int N, int H, int W, int Hs, int Ws, int top, int left, int cut,
+                  ofk_stream_t stream);
 
 /* Fused flow composition, mode 3: replaces `flow + flow.apply(self)` (ref 't', flow_class.py:1422) and
  * `self + self.invert('t').apply(flow)` (ref 's', :1418) including the zero-flow early exits (:1338-1354):

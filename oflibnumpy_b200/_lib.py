@@ -26,6 +26,8 @@ _SIGNATURES = {
     'ofk_last_error': (C.c_char_p, []),
     'ofk_version': (_i, []),
     'ofk_warp_t': (_i, [_vp, _i, _i, _i, _vp, _f, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
+    'ofk_warp_t_ex': (_i, [_vp, _i, _i, _i, _vp, _f, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i,
+                           _vp]),
     'ofk_combine3': (_i, [_vp, _vp, _vp, _vp, _i, _f, _vp, _vp, _vp, _i, _i, _i, _vp]),
     'ofk_valid_geom_t': (_i, [_vp, _f, _vp, _vp, _i, _i, _i, _vp]),
     'ofk_from_matrix': (_i, [_vp, _i, _f, _vp, _i, _i, _i, _vp]),

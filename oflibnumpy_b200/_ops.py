@@ -10,6 +10,7 @@ import numpy as np
 from . import _lib
 from . import device as dev
 from .device import DeviceArray
+from .validation import DEFAULT_THRESHOLD
 
 DTYPE_CODES = {np.dtype('uint8'): _lib.U8, np.dtype('int16'): _lib.I16, np.dtype('uint16'): _lib.U16,
                np.dtype('float32'): _lib.F32, np.dtype('float64'): _lib.F64}
@@ -49,7 +50,9 @@ def promoted_rule(payload_dtype, mask_is_bool):
 
 def warp_t(flow, sign, payload=None, payload_mask=None, flow_mask=None, want_mask=False, arith=_lib.ARITH_NATIVE,
            rule=_lib.RULE_STRICT, placement=None, cut=True):
-    """Backward warp (ofk_warp_t). placement = (top, left) of the flow frame inside the payload frame."""
+    """Backward warp (ofk_warp_t_ex). placement = (top, left) of the flow frame inside the payload frame. Frames of a
+    float payload whose flow is zero below the threshold pass the payload through, as apply_flow does
+    (utils.py:215-216), decided on the device; integer payloads come out of the identity taps unchanged anyway."""
     n, h, w = flow.shape[:3]
     if payload is not None:
         hs, ws, c = payload.shape[1:4]
@@ -61,8 +64,11 @@ def warp_t(flow, sign, payload=None, payload_mask=None, flow_mask=None, want_mas
     ho, wo = (h, w) if cut else (hs, ws)
     out = DeviceArray.empty((n, ho, wo, c), payload.dtype) if payload is not None else None
     omask = DeviceArray.empty((n, ho, wo), np.uint8) if want_mask else None
-    _lib.call('ofk_warp_t', _p(payload), code, c, arith, flow.ptr, float(sign), _p(payload_mask), _p(flow_mask),
-              _p(out), _p(omask), rule, n, h, w, hs, ws, top, left, 1 if cut else 0, dev.current_stream())
+    nz = None
+    if payload is not None and n and code in (_lib.F32, _lib.F64):
+        nz = nonzero_flags_device(flow, None, DEFAULT_THRESHOLD)
+    _lib.call('ofk_warp_t_ex', _p(payload), code, c, arith, flow.ptr, float(sign), _p(payload_mask), _p(flow_mask),
+              _p(nz), _p(out), _p(omask), rule, n, h, w, hs, ws, top, left, 1 if cut else 0, dev.current_stream())
     return out, omask
 
 

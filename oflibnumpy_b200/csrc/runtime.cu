@@ -214,7 +214,7 @@ namespace {
 constexpr int kSlots = 3;
 constexpr size_t kChunkTarget = 48u << 20;  // ~48 MiB of traffic per chunk keeps PCIe busy without hoarding HBM
 constexpr size_t kFlagBytes = 2 * sizeof(int);  // per frame: the zero flags of ofk_combine3
-constexpr int kMaxBuffers = 10;             // device buffers of one chunk (ofh_apply_combine3 has the most)
+constexpr int kMaxBuffers = 11;             // device buffers of one chunk (ofh_apply_combine3 has the most)
 
 struct Slot {
     cudaStream_t st = nullptr;
@@ -424,17 +424,24 @@ extern "C" int ofh_warp_t(const void* payload, int dtype, int C, int arith, cons
     OFK_CHECK_ARG(flow != nullptr && N >= 0 && H > 0 && W > 0 && C >= 0, "ofh_warp_t: bad arguments");
     OFK_CHECK_ARG(dtype >= OFK_U8 && dtype <= OFK_F64, "ofh_warp_t: unknown dtype %d", dtype);
     const size_t px = (size_t)H * W, b_pay = px * C * esize(dtype);
-    enum { kFlow, kPay, kOut, kPm, kFm, kOm };
+    // float payloads need apply_flow's pass-through of zero flows (ofk_warp_t_ex); integer payloads come out of the
+    // identity taps unchanged
+    const bool pass = C > 0 && (dtype == OFK_F32 || dtype == OFK_F64);
+    enum { kFlow, kPay, kOut, kPm, kFm, kOm, kNz };
     return run_ring(
-        device, N, {px * 8, b_pay, b_pay, payload_mask ? px : 0, flow_mask ? px : 0, out_mask ? px : 0}, nullptr,
+        device, N,
+        {px * 8, b_pay, b_pay, payload_mask ? px : 0, flow_mask ? px : 0, out_mask ? px : 0, pass ? sizeof(int) : 0},
+        nullptr,
         [&](const Chunk& c) {
             OFH_TRY(c.in(kFlow, flow));
             OFH_TRY(c.in(kPay, payload));
             OFH_TRY(c.in(kPm, payload_mask));
             OFH_TRY(c.in(kFm, flow_mask));
-            return ofk_warp_t(c.at(kPay), dtype, C, arith, c.at<float>(kFlow), flow_sign, c.at<uint8_t>(kPm),
-                              c.at<uint8_t>(kFm), c.at(kOut), c.at<uint8_t>(kOm), mask_rule, c.cn, H, W, H, W, 0, 0, 1,
-                              c.stream());
+            if (pass) OFH_TRY(ofk_nonzero_flags(c.at<float>(kFlow), nullptr, 1e-3f, c.at<int>(kNz), c.cn, H, W,
+                                                c.stream()));
+            return ofk_warp_t_ex(c.at(kPay), dtype, C, arith, c.at<float>(kFlow), flow_sign, c.at<uint8_t>(kPm),
+                                 c.at<uint8_t>(kFm), c.at<int>(kNz), c.at(kOut), c.at<uint8_t>(kOm), mask_rule, c.cn,
+                                 H, W, H, W, 0, 0, 1, c.stream());
         },
         [&](const Chunk& c) {
             OFH_TRY(c.out(out, kOut));
@@ -475,18 +482,23 @@ extern "C" int ofh_apply_combine3(const void* image, int dtype, int C, int arith
     OFK_CHECK_ARG(dtype >= OFK_U8 && dtype <= OFK_F64, "ofh_apply_combine3: unknown dtype %d", dtype);
     OFK_CHECK_ARG(ref == 's' || ref == 't', "ofh_apply_combine3: ref must be 's' or 't'");
     const size_t px = (size_t)H * W, b_flow = px * 8, b_img = px * C * esize(dtype);
-    enum { kA, kB, kO, kI, kOi, kAm, kBm, kOm, kOv, kF };
+    const bool pass = dtype == OFK_F32 || dtype == OFK_F64;    // zero-flow pass-through, as in ofh_warp_t
+    enum { kA, kB, kO, kI, kOi, kAm, kBm, kOm, kOv, kNz, kF };
     return run_ring(
         device, N,
-        {b_flow, b_flow, b_flow, b_img, b_img, Am ? px : 0, Bm ? px : 0, px, out_valid ? px : 0, kFlagBytes}, flags,
+        {b_flow, b_flow, b_flow, b_img, b_img, Am ? px : 0, Bm ? px : 0, px, out_valid ? px : 0,
+         pass ? sizeof(int) : 0, kFlagBytes},
+        flags,
         [&](const Chunk& c) {
             OFH_TRY(c.in(kA, A));
             OFH_TRY(c.in(kAm, Am));
             OFH_TRY(c.in(kI, image));
+            if (pass) OFH_TRY(ofk_nonzero_flags(c.at<float>(kA), nullptr, 1e-3f, c.at<int>(kNz), c.cn, H, W,
+                                                c.stream()));
             // the image warp starts while B is still on its way
-            OFH_TRY(ofk_warp_t(c.at(kI), dtype, C, arith, c.at<float>(kA), ref == 't' ? -1.0f : 1.0f, nullptr,
-                               out_valid ? c.at<uint8_t>(kAm) : nullptr, c.at(kOi), c.at<uint8_t>(kOv), mask_rule,
-                               c.cn, H, W, H, W, 0, 0, 1, c.stream()));
+            OFH_TRY(ofk_warp_t_ex(c.at(kI), dtype, C, arith, c.at<float>(kA), ref == 't' ? -1.0f : 1.0f, nullptr,
+                                  out_valid ? c.at<uint8_t>(kAm) : nullptr, c.at<int>(kNz), c.at(kOi),
+                                  c.at<uint8_t>(kOv), mask_rule, c.cn, H, W, H, W, 0, 0, 1, c.stream()));
             OFH_TRY(c.in(kB, B));
             OFH_TRY(c.in(kBm, Bm));
             return ofk_combine3(c.at<float>(kA), c.at<uint8_t>(kAm), c.at<float>(kB), c.at<uint8_t>(kBm), ref, thr,

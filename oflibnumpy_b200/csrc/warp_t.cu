@@ -8,6 +8,8 @@
 //   warp_t_u8x3    the image case: both horizontal taps of a row come from one aligned 64-bit load, the horizontal
 //                  blend runs on packed bytes (dp4a), rounding is integer, 96-byte rows are stored as 24 words.
 //   warp_t_generic 1 pixel per thread, any channel count / dtype / padding offsets / unaligned pointers.
+#include <algorithm>
+
 #include "ofk_common.cuh"
 #include "warp_t_device.cuh"
 
@@ -445,6 +447,24 @@ __global__ void __launch_bounds__(256) valid_geom_vec4(const float4* __restrict_
     st_stream_u32(out + q, v & m);
 }
 
+// apply_flow returns its target untouched for a flow that is zero below the threshold (utils.py:215-216). The warp's
+// identity taps reproduce that for integer payloads but not for floats: NaN / Inf on a zero-weight tap poison the
+// result, and -0.0 next to a positive value comes out as +0. Frames whose flag is 0 get the payload copied over the
+// warp's output (bit for bit: E is an unsigned type of the element size). The valid area needs no repair: with identity
+// taps it already is the mask that went in, ANDed with the flow mask.
+template <typename E>
+__global__ void __launch_bounds__(256) warp_t_passthrough(const E* __restrict__ payload, const int* __restrict__ nz,
+                                                          E* __restrict__ out, int Ho, long long rowlen,
+                                                          long long src_row, long long src_off, long long src_frame) {
+    const int n = blockIdx.z;
+    if (nz[n]) return;
+    const E* src = payload + n * src_frame + src_off;
+    E* dst = out + (long long)n * Ho * rowlen;
+    for (long long y = blockIdx.y; y < Ho; y += gridDim.y)
+        for (long long i = blockIdx.x * 256ll + threadIdx.x; i < rowlen; i += gridDim.x * 256ll)
+            dst[y * rowlen + i] = src[y * src_row + i];
+}
+
 template <typename T, int C, int AR>
 static int launch_rows(const void* payload, const float* flow, float sign, const uint8_t* pmask, const uint8_t* fmask,
                        void* out, uint8_t* omask, int rule, int N, int H, int W, cudaStream_t st) {
@@ -590,6 +610,33 @@ extern "C" int ofk_warp_t(const void* payload, int dtype, int C, int arith, cons
         default: OFK_GEN(double, AR_F64);
     }
 #undef OFK_GEN
+}
+
+extern "C" int ofk_warp_t_ex(const void* payload, int dtype, int C, int arith, const float* flow, float flow_sign,
+                             const uint8_t* payload_mask, const uint8_t* flow_mask, const int* flow_nonzero, void* out,
+                             uint8_t* out_mask, int mask_rule, int N, int H, int W, int Hs, int Ws, int top, int left,
+                             int cut, ofk_stream_t stream) {
+    const int rc = ofk_warp_t(payload, dtype, C, arith, flow, flow_sign, payload_mask, flow_mask, out, out_mask,
+                              mask_rule, N, H, W, Hs, Ws, top, left, cut, stream);
+    if (rc != OFK_OK || flow_nonzero == nullptr || C == 0 || N == 0) return rc;
+    const int Ho = cut ? H : Hs;
+    const long long rowlen = (long long)(cut ? W : Ws) * C, src_row = (long long)Ws * C;
+    const long long src_off = cut ? (long long)top * src_row + (long long)left * C : 0;
+    dim3 grid((unsigned)std::min<long long>((rowlen + 255) / 256, 8), (unsigned)std::min(Ho, 64), N);
+    cudaStream_t st = as_stream(stream);
+#define OFK_PASS(E)                                                                                                \
+    warp_t_passthrough<E><<<grid, 256, 0, st>>>(static_cast<const E*>(payload), flow_nonzero, static_cast<E*>(out), \
+                                                Ho, rowlen, src_row, src_off, (long long)Hs * src_row)
+    switch (dtype) {
+        case OFK_U8: OFK_PASS(uint8_t); break;
+        case OFK_I16:
+        case OFK_U16: OFK_PASS(uint16_t); break;
+        case OFK_F32: OFK_PASS(uint32_t); break;
+        default: OFK_PASS(unsigned long long); break;
+    }
+#undef OFK_PASS
+    OFK_LAUNCHED();
+    return OFK_OK;
 }
 
 extern "C" int ofk_valid_geom_t(const float* flow, float flow_sign, const uint8_t* flow_mask, uint8_t* out, int N,
