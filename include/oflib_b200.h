@@ -333,6 +333,31 @@ int ofk_accumulate_fold(const float* flow, const uint8_t* mask, int ref, int fol
 int ofk_consistency(const float* F, const uint8_t* Fm, const float* G, const uint8_t* Gm, int ref, float alpha1,
                     float alpha2, uint8_t* out, uint8_t* out_valid, int N, int H, int W, ofk_stream_t stream);
 
+/* Error metrics of N estimated flows est [N,H,W,2] against their ground truth truth [N,H,W,2] (same grid; the ref is
+ * not used). Evaluated pixels: est_mask & truth_mask & region (uint8 0/1 [N,H,W] each, NULL = all valid). For every
+ * pixel, with (ue, ve) = est[p], (ug, vg) = truth[p], in float32 with every operation rounded on its own (no FMA
+ * contraction):
+ *   du = ue - ug;  dv = ve - vg;  d2 = du*du + dv*dv;  epe = sqrt(d2)          (correctly rounded sqrt)
+ *   mg = sqrt(ug*ug + vg*vg)
+ *   fl = epe > 3 && epe / mg > 0.05f                                           (KITTI 2015 Fl; mg = 0 -> inf)
+ *   out_k = epe > k for k = 1, 3, 5;  band = 0 if mg < 10, 1 if mg < 40, else 2  (Sintel s0-10 / s10-40 / s40+)
+ *   cz = ue*vg - ve*ug;  cr = sqrt(d2 + cz*cz);  dot = (1 + ue*ug) + ve*vg
+ *   ae = atan2f(cr, dot) * 57.29578f   (degrees: the angle between (ue, ve, 1) and (ug, vg, 1), Barron et al.; 0 for a
+ *                                       perfect estimate)
+ * Results per frame n over its evaluated pixels:
+ *   counts int64 [N,8] = {evaluated, fl, out_1, out_3, out_5, band 0, band 1, band 2}
+ *   sums float64 [N,5] = {epe, ae, epe over band 0, band 1, band 2}: the float32 values added in float64, per fixed
+ *     block of 8192 pixels, then over the blocks in order, so a frame's rows do not depend on the batch it is in.
+ *   epe float32 [N,H,W] or NULL: the EPE of every pixel, evaluated or not.
+ * Inputs whose squares overflow give inf (and NaN where inf meets inf) as float32 arithmetic does.
+ * est and truth 8-byte aligned (16 for vector loads), ws: ofk_evaluate_workspace(N, H, W) bytes, 8-byte aligned (0 for
+ * bad arguments). N <= 65535, H*W < 2^31. Every argument is checked before any device work. Two launches whatever N
+ * (per-block partials, then one fixed-order pass per frame), none for N = 0. */
+size_t ofk_evaluate_workspace(int N, int H, int W);
+int ofk_evaluate(const float* est, const uint8_t* est_mask, const float* truth, const uint8_t* truth_mask,
+                 const uint8_t* region, float* epe, long long* counts, double* sums, int N, int H, int W, void* ws,
+                 size_t ws_bytes, ofk_stream_t stream);
+
 /* points_inside_area (utils.py:283-295): pts float64 [n][2] (row, col) rounded half-even like numpy.round. */
 int ofk_points_inside_area(const double* pts, size_t n, int H, int W, uint8_t* out, ofk_stream_t stream);
 
@@ -436,6 +461,10 @@ int ofh_apply_combine3(const void* image, int dtype, int C, int arith, int mask_
  * synchronous. */
 int ofh_visualise(const float* flow, const uint8_t* mask, float thr, int mode, int show_mask, int show_mask_borders,
                   float range_max, uint8_t* out, int N, int H, int W, int device);
+/* ofk_evaluate on host buffers through the ring; synchronous. Only the per-frame rows (104 bytes per frame) and, if
+ * epe is not NULL, the EPE map come back. */
+int ofh_evaluate(const float* est, const uint8_t* est_mask, const float* truth, const uint8_t* truth_mask,
+                 const uint8_t* region, float* epe, long long* counts, double* sums, int N, int H, int W, int device);
 /* All ofh_* calls leave the caller's current CUDA device unchanged. */
 /* release the internal ring (also done at process exit) */
 int ofh_release(void);

@@ -59,6 +59,8 @@ _SIGNATURES = {
     'ofk_accumulate_fold_workspace': (_sz, [_i, _i, _i, _i, _i, _i, _i]),
     'ofk_accumulate_fold': (_i, [_vp, _vp, _i, _i, _f, _i, _i, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
     'ofk_consistency': (_i, [_vp, _vp, _vp, _vp, _i, _f, _f, _vp, _vp, _i, _i, _i, _vp]),
+    'ofk_evaluate_workspace': (_sz, [_i, _i, _i]),
+    'ofk_evaluate': (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _sz, _vp]),
     'ofk_points_inside_area':(_i, [_vp, _sz, _i, _i, _vp, _vp]),
     'ofk_forward_s_workspace': (_sz, [_i, _i, _i]),
     'ofk_forward_s': (_i, [_vp, _i, _vp, _f, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _sz, _vp]),
@@ -74,6 +76,7 @@ _SIGNATURES = {
     'ofh_combine3': (_i, [_vp, _vp, _vp, _vp, _i, _f, _vp, _vp, _vp, _i, _i, _i, _i]),
     'ofh_apply_combine3': (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _f, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i]),
     'ofh_visualise': (_i, [_vp, _vp, _f, _i, _i, _i, _f, _vp, _i, _i, _i, _i]),
+    'ofh_evaluate': (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i]),
     'ofh_release': (_i, []),
     'ofk_rt_device_count': (_i, [C.POINTER(_i)]),
     'ofk_rt_set_device': (_i, [_i]),
@@ -105,7 +108,7 @@ _SIGNATURES = {
 
 _NO_CHECK = {'ofk_last_error', 'ofk_version', 'ofk_forward_s_workspace', 'ofk_combine12_workspace', 'ofk_kth_smallest_workspace',
              'ofk_visualise_batch_workspace', 'ofk_fit_matrix_workspace', 'ofk_accumulate_workspace',
-             'ofk_accumulate_fold_workspace', 'ofk_rt_launch_count', 'ofk_rt_path_count'}
+             'ofk_accumulate_fold_workspace', 'ofk_evaluate_workspace', 'ofk_rt_launch_count', 'ofk_rt_path_count'}
 
 _lib = None
 

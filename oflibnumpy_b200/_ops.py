@@ -426,3 +426,19 @@ def consistency(f, fm, g, gm, ref, alpha_1, alpha_2, want_valid):
         _lib.call('ofk_consistency', f.ptr, _p(fm), g.ptr, _p(gm), ord(ref), float(np.float32(alpha_1)),
                   float(np.float32(alpha_2)), out.ptr, _p(valid), n, h, w, dev.current_stream())
     return out, valid
+
+
+def evaluate(est, est_mask, truth, truth_mask, region, want_epe):
+    """Error metrics of every frame in one ofk_evaluate call: estimates and truth [N,H,W,2], masks and region [N,H,W]
+    or None. Returns device arrays (counts int64 [N,8], sums float64 [N,5], EPE map float32 [N,H,W] or None);
+    asynchronous, no launch for N = 0."""
+    n, h, w = est.shape[:3]
+    counts = DeviceArray.empty((n, 8), np.int64)
+    sums = DeviceArray.empty((n, 5), np.float64)
+    epe = DeviceArray.empty((n, h, w), np.float32) if want_epe else None
+    if n:
+        ws_bytes = _lib.call('ofk_evaluate_workspace', n, h, w)
+        ws = DeviceArray.empty((ws_bytes,), np.uint8)
+        _lib.call('ofk_evaluate', est.ptr, _p(est_mask), truth.ptr, _p(truth_mask), _p(region), _p(epe), counts.ptr,
+                  sums.ptr, n, h, w, ws.ptr, ws_bytes, dev.current_stream())
+    return counts, sums, epe

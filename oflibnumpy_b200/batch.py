@@ -13,10 +13,10 @@ from .device import DeviceArray
 from .flow import Flow
 from .validation import get_valid_ref, validate_shape, validate_transform_list, validate_visualise_args, \
     validate_track_args, validate_track_dtype, validate_matrix_args, validate_accumulate_args, \
-    validate_consistency_args, DEFAULT_THRESHOLD
+    validate_consistency_args, validate_evaluate_args, DEFAULT_THRESHOLD
 
-__all__ = ['FlowBatch', 'shard_range', 'apply_flow_host', 'combine_flows_host', 'apply_combine_host',
-           'visualise_flows_host']
+__all__ = ['FlowBatch', 'FlowErrors', 'shard_range', 'apply_flow_host', 'combine_flows_host', 'apply_combine_host',
+           'visualise_flows_host', 'evaluate_flows_host']
 
 
 def shard_range(n, rank, world):
@@ -385,6 +385,84 @@ class FlowBatch(object):
                                       return_valid_area)
         return (out, valid) if return_valid_area else out
 
+    def evaluate(self, truth, region=None, return_epe=False):
+        """Error metrics of this batch, the estimated flows, against ``truth``, the ground truth of the same shape and
+        ref, in one ofk_evaluate call (two launches whatever N, none for N = 0; no synchronisation, no read-back).
+        Evaluated pixels are ``self.mask & truth.mask & region``: KITTI's valid channel or Sintel's invalid-pixel mask
+        come in as ``truth``'s mask, ``region`` (N,H,W) bool / uint8, numpy or device, restricts the metrics further
+        (KITTI's noc / occ split, or the occluded / visible split of ``consistent_with``). The ref is not used in the
+        arithmetic: the flows are compared pixel by pixel on their common grid. For every pixel, in float32 with every
+        operation rounded on its own, with (ue, ve) the estimate and (ug, vg) the truth:
+
+            epe = sqrt((ue - ug)^2 + (ve - vg)^2);  mg = sqrt(ug^2 + vg^2)
+            fl = epe > 3 and epe / mg > 0.05 (KITTI 2015);  out_k = epe > k for k = 1, 3, 5
+            band = 0 if mg < 10, 1 if mg < 40, else 2 (Sintel s0-10, s10-40, s40+)
+            ae = atan2(sqrt(d2 + cz^2), (1 + ue ug) + ve vg) in degrees, d2 = epe^2 before the root, cz = ue vg - ve ug:
+                 the angle between (ue, ve, 1) and (ug, vg, 1) (Barron et al.), 0 for a perfect estimate
+
+        Returns a :class:`FlowErrors` of device arrays: per-frame ``counts`` and ``sums`` (the float32 values added in
+        float64 in a fixed order, so a frame's rows do not depend on the batch it is in), and with ``return_epe`` the
+        EPE of every pixel, evaluated or not. ``.summary()`` gives the pixel-weighted figures of the whole batch."""
+        validate_evaluate_args(self, truth, region, return_epe, FlowBatch)
+        counts, sums, epe = _ops.evaluate(self.vecs, self.masks, truth.vecs, truth.masks, _region_device(region),
+                                          return_epe)
+        return FlowErrors(counts, sums, epe)
+
+
+def _region_device(region):
+    """A validated region (numpy or device, bool / uint8 0/1) as a device uint8 array, or None."""
+    if region is None:
+        return None
+    if isinstance(region, np.ndarray):
+        return DeviceArray.from_numpy(np.ascontiguousarray(region, dtype=np.bool_).view(np.uint8))
+    d = dev.as_device(region)
+    return DeviceArray(d.ptr, d.shape, np.uint8, owner=d)
+
+
+class FlowErrors(object):
+    """Error metrics of :meth:`FlowBatch.evaluate`, one row per frame:
+
+    ``counts`` int64 (N, 8): evaluated pixels, KITTI Fl outliers, pixels with EPE > 1, > 3, > 5, and evaluated pixels
+    in the Sintel bands s0-10, s10-40, s40+ (by the magnitude of the truth).
+    ``sums`` float64 (N, 5): EPE, angular error (degrees), EPE over the bands s0-10, s10-40, s40+.
+    ``epe`` float32 (N, H, W) or None: the EPE of every pixel.
+
+    The rows are kept so that callers can form frame-averaged figures, or add the rows of several GPUs' shards, which
+    ``summary`` does not do."""
+    COUNTS = ('evaluated', 'fl', 'out1', 'out3', 'out5', 's0-10', 's10-40', 's40+')
+    SUMS = ('epe', 'ae', 's0-10', 's10-40', 's40+')
+
+    def __init__(self, counts, sums, epe=None):
+        self.counts, self.sums, self.epe = counts, sums, epe
+
+    def numpy(self):
+        """Host copies: (counts, sums), and the EPE map as a third item when there is one."""
+        host = tuple(x if isinstance(x, np.ndarray) else x.numpy() for x in (self.counts, self.sums))
+        if self.epe is None:
+            return host
+        return host + (self.epe if isinstance(self.epe, np.ndarray) else self.epe.numpy(),)
+
+    def summary(self):
+        """Pixel-weighted figures of all frames as a host dict: 'epe', 'ae' (mean EPE and angular error), 'fl',
+        'out1', 'out3', 'out5' (fractions of the evaluated pixels), 's0-10', 's10-40', 's40+' (mean EPE in each band)
+        and 'pixels'. The per-frame rows are added in frame order in float64; a figure over no pixels is NaN."""
+        counts, sums = self.numpy()[:2]
+        c = [sum(int(v) for v in counts[:, k]) for k in range(8)]
+        s = []
+        for k in range(5):
+            t = 0.0
+            for v in sums[:, k]:
+                t += float(v)
+            s.append(t)
+
+        def ratio(a, b):
+            return a / b if b else float('nan')
+
+        n = c[0]
+        return {'epe': ratio(s[0], n), 'ae': ratio(s[1], n), 'fl': ratio(c[1], n), 'out1': ratio(c[2], n),
+                'out3': ratio(c[3], n), 'out5': ratio(c[4], n), 's0-10': ratio(s[2], c[5]),
+                's10-40': ratio(s[3], c[6]), 's40+': ratio(s[4], c[7]), 'pixels': n}
+
 
 def _track_range_fails(pts, lookup, is_int, status, h, w):
     """True if a host point fails a range test of Flow.track (the tests ofk_track repeats per frame), which only
@@ -582,3 +660,30 @@ def visualise_flows_host(flows, mode, masks=None, show_mask=False, show_mask_bor
               code, int(show_mask), int(show_mask_borders), _ops.vis_range_arg(range_max), out.ctypes.data, n, h, w,
               device)
     return out
+
+
+def evaluate_flows_host(estimates, truths, est_masks=None, truth_masks=None, regions=None, out_epe=None, device=None):
+    """``FlowBatch(estimates, masks=est_masks).evaluate(FlowBatch(truths, masks=truth_masks), regions)`` on HOST
+    arrays through ofh_evaluate: frames stream through the device ring, and only the per-frame rows (104 bytes per
+    frame) come back, plus the EPE map when ``out_epe`` (float32 (N,H,W)) is given. Pass pinned arrays
+    (device.pinned_empty) for full-rate copies. Returns numpy (counts (N,8) int64, sums (N,5) float64), and ``out_epe``
+    as a third item when given."""
+    est, tru = _c(estimates, np.float32), _c(truths, np.float32)
+    if est.ndim != 4 or est.shape[3] != 2 or tru.shape != est.shape:
+        raise ValueError("Error evaluating flow: estimates and truths need the same shape (N,H,W,2)")
+    n, h, w = est.shape[:3]
+    planes = []
+    for name, m in (('Est_masks', est_masks), ('Truth_masks', truth_masks), ('Regions', regions)):
+        if m is not None:
+            m = _c(m, np.bool_)
+            if m.shape != (n, h, w):
+                raise ValueError("Error evaluating flow: {} need shape {}".format(name, (n, h, w)))
+        planes.append(m)
+    if out_epe is not None:
+        _check_out(out_epe, (n, h, w), np.float32, 'out_epe')
+    counts, sums = np.empty((n, 8), np.int64), np.empty((n, 5), np.float64)
+    device = dev.get_device() if device is None else device
+    em, tm, rg = (None if m is None else m.ctypes.data for m in planes)
+    _lib.call('ofh_evaluate', est.ctypes.data, em, tru.ctypes.data, tm, rg,
+              None if out_epe is None else out_epe.ctypes.data, counts.ctypes.data, sums.ctypes.data, n, h, w, device)
+    return (counts, sums) if out_epe is None else (counts, sums, out_epe)

@@ -15,7 +15,7 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, 'csrc')
 LIBDIR = os.path.join(PKG, 'lib')
 LIBNAME = 'liboflib_b200.so'
-SOURCES = ['runtime.cu', 'staging.cu', 'warp_t.cu', 'warp_t_ws.cu', 'combine3.cu', 'combine3_ws.cu', 'fieldgen.cu', 'elementwise.cu', 'forward_s.cu', 'combine12.cu', 'visualise.cu', 'track.cu', 'fit_matrix.cu', 'accumulate.cu']
+SOURCES = ['runtime.cu', 'staging.cu', 'warp_t.cu', 'warp_t_ws.cu', 'combine3.cu', 'combine3_ws.cu', 'fieldgen.cu', 'elementwise.cu', 'forward_s.cu', 'combine12.cu', 'visualise.cu', 'track.cu', 'fit_matrix.cu', 'accumulate.cu', 'evaluate.cu']
 NVCC_FLAGS = (['-DOFK_FWD_INSTR'] if os.environ.get('OFK_FWD_INSTR') else []) + ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17', '--use_fast_math=false',
               '-Xcompiler', '-fPIC', '-Xcompiler', '-fvisibility=hidden', '-fmad=true']
 

@@ -215,21 +215,38 @@ constexpr int kSlots = 3;
 constexpr size_t kChunkTarget = 48u << 20;  // ~48 MiB of traffic per chunk keeps PCIe busy without hoarding HBM
 constexpr size_t kFlagBytes = 2 * sizeof(int);  // per frame: the zero flags of ofk_combine3
 constexpr int kMaxBuffers = 11;             // device buffers of one chunk (ofh_apply_combine3 has the most)
+constexpr int kMaxPieces = 2;               // staged results of one call (ofh_evaluate: counts and sums)
+
+// Small per-frame results (the zero flags of ofh_combine3, the rows of ofh_evaluate) that come back through the slot's
+// pinned staging buffer: a device-to-host copy into the caller's pageable array would block the host until the chunk
+// has finished and serialise the ring. The last device buffer of a chunk holds the pieces one after another, each
+// frame_bytes[i] for every frame of the chunk; piece i belongs at dst[i] + n0 * frame_bytes[i].
+struct Staged {
+    void* dst[kMaxPieces] = {};
+    size_t frame_bytes[kMaxPieces] = {};
+    size_t total() const {
+        size_t t = 0;
+        for (int i = 0; i < kMaxPieces; ++i) t += dst[i] ? frame_bytes[i] : 0;
+        return t;
+    }
+};
 
 struct Slot {
     cudaStream_t st = nullptr;
     char* dev = nullptr;
     size_t cap = 0;
-    // Small results (the zero flags of ofh_combine3) come back through a pinned staging buffer: a device-to-host copy
-    // into the caller's pageable array would block the host until the chunk has finished and serialise the ring.
-    int* hflags = nullptr;
-    size_t hflags_cap = 0;       // ints
-    int* flags_dst = nullptr;    // where the staged flags of the chunk in flight belong
-    size_t flags_n = 0;
+    char* hstage = nullptr;      // pinned
+    size_t hstage_cap = 0;       // bytes
+    char* pending_dst[kMaxPieces] = {};   // where the staged pieces of the chunk in flight belong
+    size_t pending_bytes[kMaxPieces] = {};
     void deliver() {             // call after the slot's stream has drained
-        if (flags_dst != nullptr && flags_n) memcpy(flags_dst, hflags, flags_n * sizeof(int));
-        flags_dst = nullptr;
-        flags_n = 0;
+        size_t off = 0;
+        for (int i = 0; i < kMaxPieces; ++i) {
+            if (pending_dst[i] != nullptr && pending_bytes[i]) memcpy(pending_dst[i], hstage + off, pending_bytes[i]);
+            off += pending_bytes[i];
+            pending_dst[i] = nullptr;
+            pending_bytes[i] = 0;
+        }
     }
 };
 struct Ring {
@@ -245,22 +262,24 @@ void ring_free() {
     for (auto& s : g_ring.slot) {
         if (s.st) cudaStreamSynchronize(s.st);
         if (s.dev) cudaFree(s.dev);
-        if (s.hflags) cudaFreeHost(s.hflags);
+        if (s.hstage) cudaFreeHost(s.hstage);
         if (s.st) cudaStreamDestroy(s.st);
         s = Slot();
     }
     g_ring.device = -1;
 }
 
-int ring_prepare(int device, size_t bytes_per_slot, size_t flag_ints) {
+int ring_prepare(int device, size_t bytes_per_slot, size_t stage_bytes) {
     if (g_ring.device != device) {
         ring_free();
         g_ring.device = device;
     }
     OFK_CUDA(cudaSetDevice(device));
     for (auto& s : g_ring.slot) {
-        s.flags_dst = nullptr;   // nothing is pending between calls (a call that failed half-way drops its flags)
-        s.flags_n = 0;
+        for (int i = 0; i < kMaxPieces; ++i) {   // nothing is pending between calls (a call that failed half-way
+            s.pending_dst[i] = nullptr;          // drops its staged results)
+            s.pending_bytes[i] = 0;
+        }
         if (!s.st) OFK_CUDA(cudaStreamCreateWithFlags(&s.st, cudaStreamNonBlocking));
         if (s.cap < bytes_per_slot) {
             if (s.dev) {
@@ -277,12 +296,12 @@ int ring_prepare(int device, size_t bytes_per_slot, size_t flag_ints) {
             }
             s.cap = bytes_per_slot;
         }
-        if (s.hflags_cap < flag_ints) {
-            if (s.hflags) OFK_CUDA(cudaFreeHost(s.hflags));
-            s.hflags = nullptr;
-            s.hflags_cap = 0;
-            OFK_CUDA(cudaHostAlloc((void**)&s.hflags, sizeof(int) * flag_ints, cudaHostAllocDefault));
-            s.hflags_cap = flag_ints;
+        if (s.hstage_cap < stage_bytes) {
+            if (s.hstage) OFK_CUDA(cudaFreeHost(s.hstage));
+            s.hstage = nullptr;
+            s.hstage_cap = 0;
+            OFK_CUDA(cudaHostAlloc((void**)&s.hstage, stage_bytes, cudaHostAllocDefault));
+            s.hstage_cap = stage_bytes;
         }
     }
     return OFK_OK;
@@ -372,10 +391,11 @@ struct Chunk {
 // frame_bytes lists the device buffers of a chunk in bytes per frame. launch(chunk) queues the chunk's uploads and
 // kernels on its slot's stream; download(chunk) queues its downloads, after the NEXT chunk has been launched: with
 // pageable user buffers a download blocks the host, and this order keeps the device busy meanwhile (with pinned buffers
-// the order is irrelevant, every copy is asynchronous). Where flags is not NULL, the last buffer holds kFlagBytes per
-// frame, which come back to flags through the slot's pinned staging.
+// the order is irrelevant, every copy is asynchronous). The pieces of `staged` come back through the slot's pinned
+// staging from the last buffer (see Staged).
 template <int NB, class Launch, class Download>
-int run_ring(int device, int N, const size_t (&frame_bytes)[NB], int* flags, Launch&& launch, Download&& download) {
+int run_ring(int device, int N, const size_t (&frame_bytes)[NB], const Staged& staged, Launch&& launch,
+             Download&& download) {
     static_assert(NB <= kMaxBuffers, "raise kMaxBuffers");
     if (N == 0) return OFK_OK;
     std::lock_guard<std::mutex> lk(g_ring.mu);
@@ -385,15 +405,18 @@ int run_ring(int device, int N, const size_t (&frame_bytes)[NB], int* flags, Lau
     const int cf = (int)std::min<size_t>(N, std::max<size_t>(1, kChunkTarget / per_frame));
     size_t per_slot = 0;
     for (size_t b : frame_bytes) per_slot += pad256(b * cf);
-    OFH_TRY(ring_prepare(device, per_slot, flags ? 2 * (size_t)cf : 0));
+    OFH_TRY(ring_prepare(device, per_slot, staged.total() * cf));
     DrainRing drain_on_exit;
     auto finish = [&](const Chunk& c) -> int {
         OFH_TRY(download(c));
-        if (flags) {
+        if (staged.total()) {
             Slot& s = *c.slot;
-            OFK_CUDA(cudaMemcpyAsync(s.hflags, c.buf[NB - 1], kFlagBytes * c.cn, cudaMemcpyDeviceToHost, s.st));
-            s.flags_dst = flags + (size_t)c.n0 * 2;
-            s.flags_n = (size_t)2 * c.cn;
+            OFK_CUDA(cudaMemcpyAsync(s.hstage, c.buf[NB - 1], staged.total() * c.cn, cudaMemcpyDeviceToHost, s.st));
+            for (int i = 0; i < kMaxPieces; ++i) {
+                char* dst = (char*)staged.dst[i];
+                s.pending_dst[i] = dst ? dst + (size_t)c.n0 * staged.frame_bytes[i] : nullptr;
+                s.pending_bytes[i] = dst ? staged.frame_bytes[i] * c.cn : 0;
+            }
         }
         return OFK_OK;
     };
@@ -431,7 +454,7 @@ extern "C" int ofh_warp_t(const void* payload, int dtype, int C, int arith, cons
     return run_ring(
         device, N,
         {px * 8, b_pay, b_pay, payload_mask ? px : 0, flow_mask ? px : 0, out_mask ? px : 0, pass ? sizeof(int) : 0},
-        nullptr,
+        Staged(),
         [&](const Chunk& c) {
             OFH_TRY(c.in(kFlow, flow));
             OFH_TRY(c.in(kPay, payload));
@@ -455,7 +478,7 @@ extern "C" int ofh_combine3(const float* A, const uint8_t* Am, const float* B, c
     const size_t px = (size_t)H * W, b_flow = px * 8;
     enum { kA, kB, kO, kAm, kBm, kOm, kF };
     return run_ring(
-        device, N, {b_flow, b_flow, b_flow, Am ? px : 0, Bm ? px : 0, px, kFlagBytes}, flags,
+        device, N, {b_flow, b_flow, b_flow, Am ? px : 0, Bm ? px : 0, px, kFlagBytes}, Staged{{flags}, {kFlagBytes}},
         [&](const Chunk& c) {
             OFH_TRY(c.in(kA, A));
             OFH_TRY(c.in(kB, B));
@@ -488,7 +511,7 @@ extern "C" int ofh_apply_combine3(const void* image, int dtype, int C, int arith
         device, N,
         {b_flow, b_flow, b_flow, b_img, b_img, Am ? px : 0, Bm ? px : 0, px, out_valid ? px : 0,
          pass ? sizeof(int) : 0, kFlagBytes},
-        flags,
+        Staged{{flags}, {kFlagBytes}},
         [&](const Chunk& c) {
             OFH_TRY(c.in(kA, A));
             OFH_TRY(c.in(kAm, Am));
@@ -523,7 +546,7 @@ extern "C" int ofh_visualise(const float* flow, const uint8_t* mask, float thr, 
     const size_t px = (size_t)H * W, b_ws = range_max > 0.f ? 0 : ofk_visualise_batch_workspace(1, H, W);
     enum { kFlow, kMask, kOut, kWs };
     return run_ring(
-        device, N, {px * 8, mask ? px : 0, px * 3, b_ws}, nullptr,
+        device, N, {px * 8, mask ? px : 0, px * 3, b_ws}, Staged(),
         [&](const Chunk& c) {
             OFH_TRY(c.in(kFlow, flow));
             OFH_TRY(c.in(kMask, mask));
@@ -532,6 +555,36 @@ extern "C" int ofh_visualise(const float* flow, const uint8_t* mask, float thr, 
                                        b_ws * c.cn, c.stream());
         },
         [&](const Chunk& c) { return c.out(out, kOut); });
+}
+
+// Error metrics of N host frames: the partials of ofk_evaluate are a per-frame buffer that is never copied, and the
+// rows (counts, then sums, of the chunk's frames) come back through the pinned staging.
+extern "C" int ofh_evaluate(const float* est, const uint8_t* est_mask, const float* truth, const uint8_t* truth_mask,
+                            const uint8_t* region, float* epe, long long* counts, double* sums, int N, int H, int W,
+                            int device) {
+    OFK_CHECK_ARG(est && truth && counts && sums && N >= 0 && H > 0 && W > 0, "ofh_evaluate: bad arguments");
+    OFK_CHECK_ARG(N <= 65535, "ofh_evaluate: N = %d exceeds 65535 frames", N);
+    OFK_CHECK_ARG((size_t)H * W < (1ull << 31), "ofh_evaluate: a frame needs fewer than 2^31 pixels");
+    const size_t px = (size_t)H * W, b_ws = ofk_evaluate_workspace(1, H, W);
+    const size_t b_counts = 8 * sizeof(long long), b_sums = 5 * sizeof(double);
+    enum { kEst, kTruth, kEm, kTm, kRg, kEpe, kWs, kRows };
+    return run_ring(
+        device, N,
+        {px * 8, px * 8, est_mask ? px : 0, truth_mask ? px : 0, region ? px : 0, epe ? px * 4 : 0, b_ws,
+         b_counts + b_sums},
+        Staged{{counts, sums}, {b_counts, b_sums}},
+        [&](const Chunk& c) {
+            OFH_TRY(c.in(kEst, est));
+            OFH_TRY(c.in(kTruth, truth));
+            OFH_TRY(c.in(kEm, est_mask));
+            OFH_TRY(c.in(kTm, truth_mask));
+            OFH_TRY(c.in(kRg, region));
+            char* rows = c.at<char>(kRows);
+            return ofk_evaluate(c.at<float>(kEst), c.at<uint8_t>(kEm), c.at<float>(kTruth), c.at<uint8_t>(kTm),
+                                c.at<uint8_t>(kRg), c.at<float>(kEpe), (long long*)rows,
+                                (double*)(rows + b_counts * c.cn), c.cn, H, W, c.at(kWs), b_ws * c.cn, c.stream());
+        },
+        [&](const Chunk& c) { return c.out(epe, kEpe); });
 }
 
 extern "C" int ofh_release(void) {

@@ -17,7 +17,7 @@ from . import _ops
 from . import device as dev
 from .device import DeviceArray
 from .validation import get_valid_ref, get_valid_padding, validate_shape, validate_visualise_args, \
-    validate_track_args, validate_consistency_args, DEFAULT_THRESHOLD
+    validate_track_args, validate_consistency_args, validate_evaluate_args, DEFAULT_THRESHOLD
 
 __all__ = ['Flow']
 
@@ -697,6 +697,19 @@ class Flow(object):
                                       return_valid_area)
         out = out.numpy()[0].view(np.bool_)
         return (out, valid.numpy()[0].view(np.bool_)) if return_valid_area else out
+
+    def evaluate(self, truth, region=None):
+        """Error metrics of this flow, the estimate, against ``truth``, the ground truth of the same shape and ref:
+        ``FlowBatch.evaluate(...).summary()`` of the one frame, through the same call. ``region`` (H,W) bool / uint8,
+        numpy or device, restricts the evaluated pixels (``self.mask & truth.mask & region``). Returns a dict of 'epe',
+        'ae', 'fl', 'out1', 'out3', 'out5', 's0-10', 's10-40', 's40+' and 'pixels'."""
+        from .batch import FlowBatch
+        validate_evaluate_args(self, truth, region, False, Flow)
+        if region is not None:
+            region = region[None] if isinstance(region, np.ndarray) else \
+                dev.as_device(region).reshape((1,) + self.shape)
+        batch = FlowBatch._wrap(self._vd(), self._ref, self._md())
+        return batch.evaluate(FlowBatch._wrap(truth._vd(), truth._ref, truth._md()), region).summary()
 
 
 def _ones_mask(shape):

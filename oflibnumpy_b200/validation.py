@@ -205,3 +205,32 @@ def validate_consistency_args(flow, other, alpha_1, alpha_2, return_valid_area, 
     if not isinstance(return_valid_area, bool):
         raise TypeError(pre + "Return_valid_area needs to be a boolean")
     return alphas[0], alphas[1]
+
+
+def validate_evaluate_args(flow, truth, region, return_epe, flow_type):
+    """Checks of Flow.evaluate / FlowBatch.evaluate: ``truth`` an instance of ``flow_type`` of the same shape and
+    reference as ``flow``; ``region`` None, or a numpy or device (``__cuda_array_interface__``) array of the flow's full
+    shape ((N,H,W) for a FlowBatch, (H,W) for a Flow) and dtype bool / uint8, a numpy one holding only 0 and 1;
+    ``return_epe`` a boolean."""
+    pre = "Error evaluating flow: "
+    if not isinstance(truth, flow_type):
+        raise TypeError(pre + "Truth needs to be of type '{}'".format(flow_type.__name__))
+    shape = ((len(flow),) if hasattr(flow, '__len__') else ()) + tuple(flow.shape)
+    if ((len(truth),) if hasattr(truth, '__len__') else ()) + tuple(truth.shape) != shape:
+        raise ValueError(pre + "Flow fields need to have the same shape")
+    if flow.ref != truth.ref:
+        raise ValueError(pre + "Flow fields need to have the same reference")
+    if region is not None:
+        if isinstance(region, np.ndarray):
+            r_shape, r_dtype = region.shape, region.dtype
+        elif hasattr(region, '__cuda_array_interface__'):
+            cai = region.__cuda_array_interface__
+            r_shape, r_dtype = tuple(cai['shape']), np.dtype(cai['typestr'])
+        else:
+            raise TypeError(pre + "Region needs to be a numpy or device array")
+        if tuple(r_shape) != shape or r_dtype not in (np.bool_, np.uint8):
+            raise ValueError(pre + "Region needs shape {} and dtype bool or uint8".format(shape))
+        if isinstance(region, np.ndarray) and r_dtype != np.bool_ and ((region != 0) & (region != 1)).any():
+            raise ValueError(pre + "Region values must be 0 or 1")
+    if not isinstance(return_epe, bool):
+        raise TypeError(pre + "Return_epe needs to be a boolean")
