@@ -251,6 +251,35 @@ int ofk_track(const float* flow, const uint8_t* mask, int ref, int exact, const 
               int pts_dtype, int pts_shared, int P, int arith, int int_out, void* out, const uint8_t* status_plane,
               uint8_t* status, int* errors, int N, int H, int W, ofk_stream_t stream);
 
+/* Point trajectories through clips of flows (Sundaram, Brox & Keutzer, ECCV 2010): every point is tracked through the
+ * L frames of its clip by a chain of Flow.track steps, and dropped where a step fails. flow [S*L,H,W,2] and mask
+ * [S*L,H,W] (or NULL, all valid) are S clips of L frames, clip-major: frame s*L+k is the flow from frame k to frame k+1
+ * of clip s. flow_nonzero int32 [S*L] (device, ofk_nonzero_flags(flow, NULL, 1e-3)). pts [S,P,2] (pts_shared = 0) or
+ * [P,2] for every clip (pts_shared != 0), (row, col) in frame 0, of pts_dtype OFK_F32 or OFK_F64; a point is tracked
+ * in float64. keep uint8 0/1 [S*L,H,W] or NULL (e.g. ofk_consistency of the clip's forward and backward flows).
+ * One step of a live point q through frame n = s*L+k (round = half to even; "in frame" = 0 <= y <= H-1 and
+ * 0 <= x <= W-1, no wrap of negative indices):
+ *   ref 's' (flow on frame k's grid):
+ *     1. (y, x) = round(q); lost unless in frame, valid_source of frame n at (y, x) is 1 (the per-pixel test of
+ *        valid_geom with sign +1, AND the mask: Flow.track's status) and keep[n][y, x] != 0 (when given).
+ *     2. q' = q where flow_nonzero[n] is 0; else ofk_track's float route, bit for bit: the float64 bilinear (lost
+ *        where it raises, outside [0,H-1]x[0,W-1]), or with exact != 0 the mesh on the undisplaced grid (lost where no
+ *        triangle contains q).
+ *     3. lost unless round(q') is in frame.
+ *   ref 't' (flow on frame k+1's grid; exact is ignored):
+ *     1. lost unless round(q) is in frame.
+ *     2. q' = q where flow_nonzero[n] is 0; else ofk_track's mesh p - flow[p], bit for bit (lost where no triangle
+ *        contains q).
+ *     3. (y', x') = round(q'); lost unless in frame, valid_target of frame n at (y', x') is 1 (valid_geom with sign -1,
+ *        AND the mask) and keep[n][y', x'] != 0 (when given).
+ * out float64 [S*L,P,2]: row s*L+k holds each point's position in frame k+1 of clip s, NaN from the step where the
+ * point is lost to the end of its clip; alive uint8 [S*L,P] 1 / 0 likewise. One launch whatever S, L and P (one
+ * thread per trajectory), none for S*P = 0; nothing is read back. S*L <= INT_MAX, frame offsets 64-bit; the mesh
+ * routes need H, W >= 2 and H*W < 2^30. Every argument is checked before any device work. */
+int ofk_track_clips(const float* flow, const uint8_t* mask, int ref, int exact, const int* flow_nonzero,
+                    const void* pts, int pts_dtype, int pts_shared, int S, int L, int P, const uint8_t* keep,
+                    double* out, uint8_t* alive, int H, int W, ofk_stream_t stream);
+
 /* Flow.matrix (flow_class.py:797-867) of N frames: a 3x3 float64 transform per frame fitted to the point pairs of the
  * valid pixels, resolved on the device with no synchronisation.
  *   flow [N,H,W,2]; mask [N,H,W] or NULL (all valid), read when masked != 0; ref 's' (src = grid, dst = grid + flow)

@@ -52,6 +52,7 @@ _SIGNATURES = {
     'ofk_visualise_batch': (_i, [_vp, _vp, _f, _i, _i, _i, _f, _vp, _i, _i, _i, _vp, _sz, _vp]),
     'ofk_track_bilinear': (_i, [_vp, _vp, _sz, _i, _i, _vp, _vp, _vp]),
     'ofk_track': (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
+    'ofk_track_clips': (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _i, _i, _vp]),
     'ofk_fit_matrix_workspace': (_sz, [_i, _i, _i, _i, _i, _i]),
     'ofk_fit_matrix': (_i, [_vp, _vp, _i, _i, _i, _i, _f, _i, _vp, _vp, _vp, _i, _i, _i, _vp, _sz, _vp]),
     'ofk_accumulate_workspace': (_sz, [_i, _i]),

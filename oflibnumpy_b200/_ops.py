@@ -372,6 +372,20 @@ def track(flow, mask, ref, exact, flow_nonzero, pts, arith_dtype, int_out, statu
     return out, status, errors
 
 
+def track_clips(flow, mask, ref, exact, flow_nonzero, pts, s, l, keep):
+    """Trajectories through S clips of L frames in one ofk_track_clips call: flow [S*L,H,W,2], pts device float32 /
+    float64 [S,P,2] or [P,2], keep uint8 [S*L,H,W] or None. Returns device arrays (positions float64 [S*L,P,2], alive
+    uint8 [S*L,P]); asynchronous."""
+    n, h, w = flow.shape[:3]
+    p = pts.shape[-2]
+    out = DeviceArray.empty((n, p, 2), np.float64)
+    alive = DeviceArray.empty((n, p), np.uint8)
+    _lib.call('ofk_track_clips', flow.ptr, _p(mask), ord(ref), int(exact), flow_nonzero.ptr, pts.ptr,
+              TRACK_PTS_CODES[pts.dtype], int(pts.ndim == 2), s, l, p, _p(keep), out.ptr, alive.ptr, h, w,
+              dev.current_stream())
+    return out, alive
+
+
 def resize_flow(vecs, mask, fy, fx):
     """cv2.resize semantics: output size = round-half-even(size * scale) (ofk_resize_flow)."""
     n, h, w = (vecs if vecs is not None else mask).shape[:3]

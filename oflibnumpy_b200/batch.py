@@ -13,7 +13,7 @@ from .device import DeviceArray
 from .flow import Flow
 from .validation import get_valid_ref, validate_shape, validate_transform_list, validate_visualise_args, \
     validate_track_args, validate_track_dtype, validate_matrix_args, validate_accumulate_args, \
-    validate_consistency_args, validate_evaluate_args, DEFAULT_THRESHOLD
+    validate_consistency_args, validate_evaluate_args, validate_track_clips_args, DEFAULT_THRESHOLD
 
 __all__ = ['FlowBatch', 'FlowErrors', 'shard_range', 'apply_flow_host', 'combine_flows_host', 'apply_combine_host',
            'visualise_flows_host', 'evaluate_flows_host']
@@ -305,6 +305,53 @@ class FlowBatch(object):
         if bad:
             _raise_track_error(errors.numpy(), h, w)
         return (out, status) if get_valid_status else out
+
+    def track_clips(self, pts, clip_length=None, keep=None, s_exact_mode=None):
+        """Point trajectories through clips (Sundaram, Brox & Keutzer, ECCV 2010) in one ofk_track_clips launch: each
+        point is chained through the frames of its clip by ``Flow.track`` steps and dropped where a step fails. The
+        batch is clip-major as for ``accumulate``: N / L clips of L = ``clip_length`` frames (default: one clip of
+        all N), frame ``s*L + k`` the flow from frame k to frame k+1 of clip s.
+
+        ``pts`` (row, col) in frame 0 is (S,P,2), points per clip, or (P,2), the same points in every clip; a numpy
+        array of a float or int dtype (integers are tracked as their float64 values, not looked up as ``Flow.track``
+        does), or a float32 / float64 device array (``DeviceArray``, any ``__cuda_array_interface__`` exporter such as
+        a torch.cuda tensor). ``keep`` (N,H,W) bool / uint8, numpy or device, on the grid of each frame of the batch:
+        ``fw.consistent_with(bw)`` stops trajectories at occlusions. ``s_exact_mode`` as in ``Flow.track``.
+
+        One step of a live point q (float64) through frame F = ``self[s*L + k]``, with round half to even and "in
+        frame" meaning 0 <= y <= H-1 and 0 <= x <= W-1 (no wrap of negative indices):
+
+        ref 's' (F on frame k's grid):
+            1. (y, x) = round(q); lost unless in frame, ``F.track(q, get_valid_status=True)``'s status is 1 (the
+               vector lands strictly inside the frame, AND the mask) and ``keep[s*L + k][y, x]`` (when given) is not 0.
+            2. q' = q if F is zero below the threshold, else ``F.track(q, s_exact_mode=s_exact_mode)`` bit for bit;
+               lost where the bilinear would raise IndexError or the mesh finds no triangle.
+            3. lost unless round(q') is in frame.
+        ref 't' (F on frame k+1's grid):
+            1. lost unless round(q) is in frame.
+            2. q' = q if F is zero below the threshold, else ``F.track(q)`` (the mesh) bit for bit; lost where no
+               triangle contains q.
+            3. (y', x') = round(q'); lost unless in frame, ``F.valid_target()[y', x']`` is 1 and ``keep[s*L + k][y',
+               x']`` (when given) is not 0.
+
+        Every test is on the flow's own grid, as in ``consistent_with``. The 's' bilinear keeps Flow.track's clipped
+        weights: on the last row or column they are all 0, so a point there does not move.
+
+        Returns device arrays (``.numpy()`` to download): ``positions`` float64 (N,P,2), row ``s*L + k`` the position
+        of each point in frame k+1 of clip s, and ``alive`` uint8 (N,P) of 0/1. A lost point is NaN and 0 from the
+        step where it is lost to the end of its clip. The call never raises for a point's position, never
+        synchronises and reads nothing back; N = 0 or P = 0 launches nothing."""
+        n, (h, w) = len(self), self.shape
+        clip, s_exact_mode = validate_track_clips_args(pts, clip_length, keep, s_exact_mode, n, (h, w))
+        p = pts.shape[-2]
+        if n == 0 or p == 0:
+            return DeviceArray.empty((n, p, 2), np.float64), DeviceArray.empty((n, p), np.uint8)
+        if isinstance(pts, np.ndarray):
+            dpts = DeviceArray.from_numpy(pts if pts.dtype in (np.float32, np.float64) else pts.astype(np.float64))
+        else:
+            dpts = dev.as_device(pts)
+        return _ops.track_clips(self.vecs, self.masks, self.ref, s_exact_mode, self._zero_flags(), dpts, n // clip,
+                                clip, _region_device(keep))
 
 
     def matrix(self, dof=None, method=None, masked=None, *, hypotheses=None, return_inliers=False):

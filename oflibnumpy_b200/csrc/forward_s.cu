@@ -2305,12 +2305,24 @@ __global__ void __launch_bounds__(128) mesh_sample_kernel(const float* __restric
     }
 }
 
+// Flow.track's mesh route for one float64 point (qy, qx) of the frame fn [H,W,2]: the vector at the point is the
+// barycentric interpolation of ofk_mesh_sample, rounded to float32 as ofk_mesh_sample stores it, and the result is
+// q + (v, u) in float64. Returns false (and leaves the outputs alone) where no triangle contains the point.
+__device__ __forceinline__ bool mesh_track_point(const float* __restrict__ fn, int H, int W, float mesh_sign, double qy,
+                                                 double qx, double& orow, double& ocol, double flip_tol) {
+    int vidx[3];
+    double w[3];
+    if (!mesh_locate(reinterpret_cast<const float2*>(fn), H, W, mesh_sign, 0, qx, qy, vidx, w, flip_tol)) return false;
+    orow = __dadd_rn(qy, (double)(float)mesh_interp(fn, 2, vidx, w, 1));
+    ocol = __dadd_rn(qx, (double)(float)mesh_interp(fn, 2, vidx, w, 0));
+    return true;
+}
+
 // ofk_track's mesh route: Flow.track for ref 't' (mesh p - flow[p]) and for float points on ref 's' with s_exact_mode
 // (mesh_sign = 0:
 // the undisplaced grid, the same vertex positions as the zero field Flow.track meshes), one thread per point of the
-// flat [N*P] index. The vector at the point is the barycentric interpolation of ofk_mesh_sample, rounded to float32 as
-// ofk_mesh_sample stores it; out = pts + (v, u) in float64, (0, 0) where no triangle contains the point (griddata's NaN
-// rows, utils.py:616-618), the points themselves in frames whose flow_nonzero is 0.
+// flat [N*P] index: out = mesh_track_point, (0, 0) where no triangle contains the point (griddata's NaN rows,
+// utils.py:616-618), the points themselves in frames whose flow_nonzero is 0.
 template <typename PT>
 __global__ void __launch_bounds__(128) track_mesh_kernel(const float* __restrict__ flow,
                                                          const uint8_t* __restrict__ mask, float mesh_sign,
@@ -2330,14 +2342,8 @@ __global__ void __launch_bounds__(128) track_mesh_kernel(const float* __restrict
         if (flow_nonzero[n] == 0) {
             store_passthrough<PT, double>(out, int_out, k, r, c);
         } else {
-            const double qy = (double)r, qx = (double)c;
-            int vidx[3];
-            double w[3];
             double orow = 0.0, ocol = 0.0;
-            if (mesh_locate(fl, H, W, mesh_sign, 0, qx, qy, vidx, w, flip_tol)) {
-                orow = __dadd_rn(qy, (double)(float)mesh_interp(fn, 2, vidx, w, 1));
-                ocol = __dadd_rn(qx, (double)(float)mesh_interp(fn, 2, vidx, w, 0));
-            }
+            mesh_track_point(fn, H, W, mesh_sign, (double)r, (double)c, orow, ocol, flip_tol);
             store_tracked<double>(out, int_out, k, orow, ocol);
         }
         int err = 0;
@@ -2345,6 +2351,61 @@ __global__ void __launch_bounds__(128) track_mesh_kernel(const float* __restrict
             track_status(r, c, fl, mask ? mask + n * hw : nullptr, status_plane ? status_plane + n * hw : nullptr, H, W,
                          k, status, err);
         if (err) atomicOr(errors + n, err);
+    }
+}
+
+// Routes of ofk_track_clips: ref 's' with the float64 bilinear of Flow.track, ref 's' with s_exact_mode (the mesh on
+// the undisplaced grid), ref 't' (the mesh p - flow[p]).
+enum { CLIPS_S_BILINEAR = 0, CLIPS_S_MESH = 1, CLIPS_T_MESH = 2 };
+
+// (y, x) = round half to even of (r, c); true if that pixel is in the frame (NaN and huge values are not).
+__device__ __forceinline__ bool rounded_in_frame(double r, double c, int H, int W, int& y, int& x) {
+    y = round_to_i32(r);
+    x = round_to_i32(c);
+    return y >= 0 && y < H && x >= 0 && x < W;
+}
+
+// ofk_track_clips: one thread per trajectory of the flat [S*P] index, walking the L frames of its clip in order with the
+// step rules of include/oflib_b200.h. A point lost at step j is NaN in out and 0 in alive from frame s*L + j on.
+template <int ROUTE, typename PT>
+__global__ void __launch_bounds__(128) track_clips_kernel(const float* __restrict__ flow,
+                                                          const uint8_t* __restrict__ mask,
+                                                          const int* __restrict__ flow_nonzero,
+                                                          const PT* __restrict__ pts, int pts_shared, int L, int P,
+                                                          const uint8_t* __restrict__ keep, double* __restrict__ out,
+                                                          uint8_t* __restrict__ alive, int H, int W, size_t total,
+                                                          double flip_tol) {
+    const size_t hw = (size_t)H * W;
+    const double nan = __longlong_as_double(0x7ff8000000000000LL);   // numpy's NaN
+    for (size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x; k < total; k += (size_t)gridDim.x * blockDim.x) {
+        const size_t s = k / (size_t)P, i = k - s * P;
+        const size_t src = pts_shared ? i : k;
+        double qy = (double)pts[2 * src], qx = (double)pts[2 * src + 1];
+        bool live = true;
+        for (int j = 0; j < L; ++j) {
+            const size_t n = s * L + j, o = n * P + i;
+            if (live) {
+                const float* fn = flow + n * hw * 2;
+                const float2* fl = reinterpret_cast<const float2*>(fn);
+                const uint8_t* mn = mask ? mask + n * hw : nullptr;
+                int y, x;
+                live = rounded_in_frame(qy, qx, H, W, y, x);
+                if (ROUTE != CLIPS_T_MESH && live)
+                    live = valid_source_s_at(fl, mn, H, W, y, x) && (keep == nullptr || keep[n * hw + (size_t)y * W + x]);
+                if (live && flow_nonzero[n] != 0) {
+                    if constexpr (ROUTE == CLIPS_S_BILINEAR)
+                        live = bilinear_track_point(fl, H, W, qy, qx, qy, qx);
+                    else
+                        live = mesh_track_point(fn, H, W, ROUTE == CLIPS_T_MESH ? -1.0f : 0.0f, qy, qx, qy, qx, flip_tol);
+                }
+                if (live) live = rounded_in_frame(qy, qx, H, W, y, x);
+                if (ROUTE == CLIPS_T_MESH && live)
+                    live = valid_target_t_at(fl, mn, H, W, y, x) && (keep == nullptr || keep[n * hw + (size_t)y * W + x]);
+            }
+            out[2 * o] = live ? qy : nan;
+            out[2 * o + 1] = live ? qx : nan;
+            alive[o] = live ? 1 : 0;
+        }
     }
 }
 
@@ -2369,6 +2430,28 @@ int launch_track_mesh(const float* flow, const uint8_t* mask, int ref, const int
         default: OFK_TRACK_MESH(int64_t); break;
     }
 #undef OFK_TRACK_MESH
+    OFK_LAUNCHED();
+    return OFK_OK;
+}
+
+int launch_track_clips(const float* flow, const uint8_t* mask, int ref, int exact, const int* flow_nonzero,
+                       const void* pts, int pts_dtype, int pts_shared, int S, int L, int P, const uint8_t* keep,
+                       double* out, uint8_t* alive, int H, int W, cudaStream_t st) {
+    const size_t total = (size_t)S * P;
+    const size_t blocks = std::min((total + 127) / 128, (size_t)sm_count() * 64);
+    const double tol = g_flip_tol.load();
+#define OFK_TRACK_CLIPS(R, T)                                                                                          \
+    legacy::track_clips_kernel<legacy::R, T><<<(unsigned)blocks, 128, 0, st>>>(                                        \
+        flow, mask, flow_nonzero, static_cast<const T*>(pts), pts_shared, L, P, keep, out, alive, H, W, total, tol)
+    const bool f32 = pts_dtype == OFK_F32;
+    if (ref == 't') {
+        if (f32) OFK_TRACK_CLIPS(CLIPS_T_MESH, float); else OFK_TRACK_CLIPS(CLIPS_T_MESH, double);
+    } else if (exact) {
+        if (f32) OFK_TRACK_CLIPS(CLIPS_S_MESH, float); else OFK_TRACK_CLIPS(CLIPS_S_MESH, double);
+    } else {
+        if (f32) OFK_TRACK_CLIPS(CLIPS_S_BILINEAR, float); else OFK_TRACK_CLIPS(CLIPS_S_BILINEAR, double);
+    }
+#undef OFK_TRACK_CLIPS
     OFK_LAUNCHED();
     return OFK_OK;
 }

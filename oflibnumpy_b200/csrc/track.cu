@@ -2,6 +2,10 @@
 // The 's' lookup kernel lives here; the mesh route ('t', 's' exact with float points) is next to ofk_mesh_sample in
 // forward_s.cu. Both fold the frame into a flat [N*P] point index and share the per-point arithmetic of
 // track_device.cuh.
+// Trajectories through clips, ofk_track_clips: the entry point and its checks are here, the kernel (which needs the
+// mesh) is next to the mesh kernel in forward_s.cu.
+#include <limits.h>
+
 #include <algorithm>
 
 #include "track_device.cuh"
@@ -107,4 +111,21 @@ extern "C" int ofk_track(const float* flow, const uint8_t* mask, int ref, int ex
             OFK_TRACK_S(int64_t, double);
     }
 #undef OFK_TRACK_S
+}
+
+extern "C" int ofk_track_clips(const float* flow, const uint8_t* mask, int ref, int exact, const int* flow_nonzero,
+                               const void* pts, int pts_dtype, int pts_shared, int S, int L, int P,
+                               const uint8_t* keep, double* out, uint8_t* alive, int H, int W, ofk_stream_t stream) {
+    OFK_CHECK_ARG(flow && flow_nonzero && pts && out && alive, "ofk_track_clips: NULL pointer");
+    OFK_CHECK_ARG(ref == 's' || ref == 't', "ofk_track_clips: ref must be 's' or 't'");
+    OFK_CHECK_ARG(pts_dtype == OFK_F32 || pts_dtype == OFK_F64, "ofk_track_clips: pts_dtype must be OFK_F32 or OFK_F64");
+    OFK_CHECK_ARG(S >= 0 && L > 0 && P >= 0 && H > 0 && W > 0, "ofk_track_clips: bad shape S=%d L=%d P=%d H=%d W=%d", S,
+                  L, P, H, W);
+    OFK_CHECK_ARG((long long)S * L <= INT_MAX, "ofk_track_clips: S*L must not exceed INT_MAX (S=%d L=%d)", S, L);
+    const bool mesh = ref == 't' || exact != 0;
+    OFK_CHECK_ARG(!mesh || (H > 1 && W > 1 && (size_t)H * W < ((size_t)1 << 30)),
+                  "ofk_track_clips: the mesh route needs 2 <= H, W and H*W < 2^30 (H=%d W=%d)", H, W);
+    if (S == 0 || P == 0) return OFK_OK;
+    return launch_track_clips(flow, mask, ref, exact, flow_nonzero, pts, pts_dtype, pts_shared, S, L, P, keep, out,
+                              alive, H, W, as_stream(stream));
 }

@@ -1,5 +1,6 @@
 // Per-point arithmetic of point tracking (Flow.track, utils.py:547-622), shared by ofk_track_bilinear (elementwise.cu),
-// the lookup kernel of ofk_track (track.cu) and its mesh kernel (forward_s.cu).
+// the lookup kernel of ofk_track (track.cu), its mesh kernel and the trajectory kernel of ofk_track_clips
+// (forward_s.cu).
 #pragma once
 #include <math.h>
 
@@ -63,6 +64,15 @@ __device__ __forceinline__ uint8_t valid_source_s_at(const float2* __restrict__ 
     return (uint8_t)(ok & (mask ? (unsigned)mask[q] : 1u));
 }
 
+// Frame-wise valid_target of a 't' flow at pixel (y, x): the per-pixel test of valid_geom_vec4 (warp_t.cu) with sign -1.
+__device__ __forceinline__ uint8_t valid_target_t_at(const float2* __restrict__ f, const uint8_t* __restrict__ mask,
+                                                     int H, int W, int y, int x) {
+    const size_t q = (size_t)y * W + x;
+    const float2 v = f[q];
+    const unsigned ok = strict_in_frame(__fmaf_rn(-1.0f, v.x, (float)x), __fmaf_rn(-1.0f, v.y, (float)y), H, W);
+    return (uint8_t)(ok & (mask ? (unsigned)mask[q] : 1u));
+}
+
 // The valid status of one point at its rounded position (ref 's': computed here from flow and mask; ref 't': gathered
 // from status_plane) and the error bit when that index is out of range. f, mask and status_plane point at the frame.
 template <typename PT>
@@ -115,5 +125,10 @@ __device__ __forceinline__ void store_passthrough(void* out, int int_out, size_t
 int launch_track_mesh(const float* flow, const uint8_t* mask, int ref, const int* flow_nonzero, const void* pts,
                       int pts_dtype, int pts_shared, int P, void* out, int int_out, const uint8_t* status_plane,
                       uint8_t* status, int* errors, int N, int H, int W, cudaStream_t st);
+
+// ofk_track_clips' kernel (forward_s.cu, next to the mesh it needs); arguments checked by the caller, S*P > 0
+int launch_track_clips(const float* flow, const uint8_t* mask, int ref, int exact, const int* flow_nonzero,
+                       const void* pts, int pts_dtype, int pts_shared, int S, int L, int P, const uint8_t* keep,
+                       double* out, uint8_t* alive, int H, int W, cudaStream_t st);
 
 }  // namespace ofk

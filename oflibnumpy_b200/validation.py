@@ -168,6 +168,11 @@ def validate_accumulate_args(clip_length, cumulative, thresholded, batch_size, f
         raise TypeError(pre + "Thresholded needs to be a boolean")
     if fold is not None and not (isinstance(fold, str) and fold in ('left', 'right')):
         raise ValueError(pre + "Fold needs to be 'left' or 'right', not {!r}".format(fold))
+    return _clip_length(clip_length, batch_size, pre)
+
+
+def _clip_length(clip_length, batch_size, pre):
+    """The clip length L of a clip-major batch: ``clip_length``, or the whole batch for None (1 for an empty batch)."""
     if clip_length is None:
         return max(batch_size, 1)
     if isinstance(clip_length, bool) or not isinstance(clip_length, (int, np.integer)) or clip_length < 1 or \
@@ -175,6 +180,54 @@ def validate_accumulate_args(clip_length, cumulative, thresholded, batch_size, f
         raise ValueError(pre + "Clip_length needs to be a positive integer that divides the batch size {}, not {!r}"
                          .format(batch_size, clip_length))
     return int(clip_length)
+
+
+def _array_meta(a):
+    """(shape, dtype) of a numpy array or a ``__cuda_array_interface__`` exporter, or None for anything else."""
+    if isinstance(a, np.ndarray):
+        return a.shape, a.dtype
+    if hasattr(a, '__cuda_array_interface__'):
+        cai = a.__cuda_array_interface__
+        return tuple(cai['shape']), np.dtype(cai['typestr'])
+    return None
+
+
+def _validate_plane(plane, shape, pre, name):
+    """A numpy or device bool / uint8 array of ``shape``, a numpy one holding only 0 and 1."""
+    meta = _array_meta(plane)
+    if meta is None:
+        raise TypeError(pre + "{} needs to be a numpy or device array".format(name))
+    if tuple(meta[0]) != shape or meta[1] not in (np.bool_, np.uint8):
+        raise ValueError(pre + "{} needs shape {} and dtype bool or uint8".format(name, shape))
+    if isinstance(plane, np.ndarray) and meta[1] != np.bool_ and ((plane != 0) & (plane != 1)).any():
+        raise ValueError(pre + "{} values must be 0 or 1".format(name))
+
+
+def validate_track_clips_args(pts, clip_length, keep, s_exact_mode, batch_size, shape):
+    """Checks of FlowBatch.track_clips on a batch of ``batch_size`` frames of ``shape`` (H, W). ``pts`` a numpy array
+    of a float or int dtype, or a float32 / float64 device array, of shape (S,P,2), S = batch_size / L, or (P,2);
+    ``keep`` None or a plane as ``validate_evaluate_args`` takes a region, of shape (N,H,W). Returns (L,
+    s_exact_mode); None stands for one clip and False."""
+    pre = "Error tracking points through clips: "
+    clip = _clip_length(clip_length, batch_size, pre)
+    meta = _array_meta(pts)
+    if meta is None:
+        raise TypeError(pre + "Pts needs to be a numpy or device array")
+    p_shape, p_dtype = meta
+    clips = batch_size // clip
+    if not (len(p_shape) == 2 or (len(p_shape) == 3 and p_shape[0] == clips)) or p_shape[-1] != 2:
+        raise ValueError(pre + "Pts needs to have shape ({},P,2) or (P,2)".format(clips))
+    if not isinstance(pts, np.ndarray):
+        if p_dtype not in (np.float32, np.float64):
+            raise TypeError(pre + "Device pts need dtype float32 or float64, not {}".format(p_dtype))
+    elif not (np.issubdtype(p_dtype, np.integer) or np.issubdtype(p_dtype, np.floating)):
+        raise TypeError(pre + "Pts numpy array needs to have a float or int dtype, not {}".format(p_dtype))
+    if keep is not None:
+        _validate_plane(keep, (batch_size,) + tuple(shape), pre, 'Keep')
+    s_exact_mode = False if s_exact_mode is None else s_exact_mode
+    if not isinstance(s_exact_mode, bool):
+        raise TypeError(pre + "S_exact_mode needs to be a boolean")
+    return clip, s_exact_mode
 
 
 def validate_consistency_args(flow, other, alpha_1, alpha_2, return_valid_area, flow_type):
@@ -221,16 +274,6 @@ def validate_evaluate_args(flow, truth, region, return_epe, flow_type):
     if flow.ref != truth.ref:
         raise ValueError(pre + "Flow fields need to have the same reference")
     if region is not None:
-        if isinstance(region, np.ndarray):
-            r_shape, r_dtype = region.shape, region.dtype
-        elif hasattr(region, '__cuda_array_interface__'):
-            cai = region.__cuda_array_interface__
-            r_shape, r_dtype = tuple(cai['shape']), np.dtype(cai['typestr'])
-        else:
-            raise TypeError(pre + "Region needs to be a numpy or device array")
-        if tuple(r_shape) != shape or r_dtype not in (np.bool_, np.uint8):
-            raise ValueError(pre + "Region needs shape {} and dtype bool or uint8".format(shape))
-        if isinstance(region, np.ndarray) and r_dtype != np.bool_ and ((region != 0) & (region != 1)).any():
-            raise ValueError(pre + "Region values must be 0 or 1")
+        _validate_plane(region, shape, pre, 'Region')
     if not isinstance(return_epe, bool):
         raise TypeError(pre + "Return_epe needs to be a boolean")
