@@ -195,23 +195,8 @@ int ofk_resize_flow(const float* vecs, const uint8_t* mask, float* out_vecs, uin
 /* out[i] = v[i] > thr (the `> .99` mask test of combine_with mode 2 / ref 't', flow_class.py:1410). */
 int ofk_greater(const float* v, float thr, uint8_t* out, size_t n, ofk_stream_t stream);
 
-/* Flow.visualise (flow_class.py:869-951), one frame per call (the N = 1 case of ofk_visualise_batch's kernels).
- * ofk_vis_magnitude: mag[p] = magnitude of threshold_vectors(flow)[p] as cv2.cartToPolar computes it (float32);
- *   *max_out (device float) receives the maximum.
- * ofk_kth_smallest: exact order statistics of a NON-NEGATIVE float32 device array of n < 2^32 values: out[q] (device)
- *   = the element of rank ranks_host[q] (0-based, host array, 1 <= n_ranks <= 4) in sorted order -- the values
- *   numpy.percentile interpolates between. ws: device workspace of ofk_kth_smallest_workspace(n_ranks) bytes.
- * ofk_visualise: out uint8 [H,W,3]; mode 0 'hsv', 1 'rgb', 2 'bgr'; range_max = magnitude mapped to full saturation
- *   (the caller derives it from the 99th percentile / maximum as the reference does); mask may be NULL (all valid). */
-int ofk_vis_magnitude(const float* flow, float thr, float* mag, float* max_out, size_t n_pixels, ofk_stream_t stream);
-size_t ofk_kth_smallest_workspace(int n_ranks);
-int ofk_kth_smallest(const float* values, size_t n, const unsigned long long* ranks_host, int n_ranks, float* out,
-                     void* ws, size_t ws_bytes, ofk_stream_t stream);
-int ofk_visualise(const float* flow, const uint8_t* mask, float thr, int mode, int show_mask, int show_mask_borders,
-                  float range_max, uint8_t* out, int H, int W, ofk_stream_t stream);
-
-/* Flow.visualise of N frames: frame n of out equals Flow(flow[n], ref, mask[n]).visualise(mode, show_mask,
- * show_mask_borders, range_max). range_max > 0: that range for every frame; range_max == 0: the reference's default per
+/* Flow.visualise (flow_class.py:869-951) of N frames, the one-frame call being the N = 1 case: frame n of out equals
+ * Flow(flow[n], ref, mask[n]).visualise(mode, show_mask, show_mask_borders, range_max). range_max > 0: that range for every frame; range_max == 0: the reference's default per
  * frame, resolved on the device (numpy's float32 percentile(mag, 99) over all H*W magnitudes, mask ignored; if that is
  * 0 the maximum, if that is 0 too then 1); < 0 or NaN: OFK_EINVAL. mask NULL = all valid. mode 0 hsv, 1 rgb, 2 bgr.
  * out uint8 [N,H,W,3]. ws: ofk_visualise_batch_workspace(N,H,W) bytes, 4-byte aligned (256-byte aligned keeps the
@@ -221,12 +206,6 @@ size_t ofk_visualise_batch_workspace(int N, int H, int W);
 int ofk_visualise_batch(const float* flow, const uint8_t* mask, float thr, int mode, int show_mask,
                         int show_mask_borders, float range_max, uint8_t* out, int N, int H, int W, void* ws,
                         size_t ws_bytes, ofk_stream_t stream);
-
-/* Point tracking through an 's' flow with float points: replaces bilinear_interpolation + `pts + flow_vecs`
- * (utils.py:161-196,605,608). flow [H,W,2] (one frame), pts float64 [n][2] (row, col); out float64 [n][2];
- * bad (int32, device) is set to 1 if any point lies outside the flow area (the reference raises IndexError). */
-int ofk_track_bilinear(const float* flow, const double* pts, size_t n, int H, int W, double* out, int* bad,
-                       ofk_stream_t stream);
 
 /* Flow.track (flow_class.py:755-795, utils.py:547-622) of N frames in one call: frame n of the outputs equals
  * Flow(flow[n], ref, mask[n]).track(pts_n, int_out, get_valid_status, exact), bit for bit.

@@ -44,13 +44,8 @@ _SIGNATURES = {
     'ofk_greater': (_i, [_vp, _f, _vp, _sz, _vp]),
     'ofk_decode_kitti': (_i, [_vp, _vp, _vp, _sz, _vp]),
     'ofk_decode_sintel_mask': (_i, [_vp, _vp, _sz, _vp]),
-    'ofk_vis_magnitude': (_i, [_vp, _f, _vp, _vp, _sz, _vp]),
-    'ofk_kth_smallest_workspace': (_sz, [_i]),
-    'ofk_kth_smallest': (_i, [_vp, _sz, _vp, _i, _vp, _vp, _sz, _vp]),
-    'ofk_visualise': (_i, [_vp, _vp, _f, _i, _i, _i, _f, _vp, _i, _i, _vp]),
     'ofk_visualise_batch_workspace': (_sz, [_i, _i, _i]),
     'ofk_visualise_batch': (_i, [_vp, _vp, _f, _i, _i, _i, _f, _vp, _i, _i, _i, _vp, _sz, _vp]),
-    'ofk_track_bilinear': (_i, [_vp, _vp, _sz, _i, _i, _vp, _vp, _vp]),
     'ofk_track': (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
     'ofk_track_clips': (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _i, _i, _vp]),
     'ofk_fit_matrix_workspace': (_sz, [_i, _i, _i, _i, _i, _i]),
@@ -107,7 +102,7 @@ _SIGNATURES = {
     'ofk_rt_path_count': (C.c_ulonglong, [C.c_int]),
 }
 
-_NO_CHECK = {'ofk_last_error', 'ofk_version', 'ofk_forward_s_workspace', 'ofk_combine12_workspace', 'ofk_kth_smallest_workspace',
+_NO_CHECK = {'ofk_last_error', 'ofk_version', 'ofk_forward_s_workspace', 'ofk_combine12_workspace',
              'ofk_visualise_batch_workspace', 'ofk_fit_matrix_workspace', 'ofk_accumulate_workspace',
              'ofk_accumulate_fold_workspace', 'ofk_evaluate_workspace', 'ofk_rt_launch_count', 'ofk_rt_path_count'}
 

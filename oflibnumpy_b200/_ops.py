@@ -3,8 +3,6 @@
 Shapes: flow vectors [N,H,W,2] float32, masks [N,H,W] uint8 (0/1), payloads [N,H,W,C]. Everything is asynchronous on
 the current stream (device.set_stream) unless a result has to be read on the host.
 """
-import ctypes
-
 import numpy as np
 
 from . import _lib
@@ -174,70 +172,10 @@ def extent(flow, mask, sign, thr):
     return out.numpy()
 
 
-def percentile_plan(n, q=99):
-    """numpy.percentile(a, q) (method 'linear') of a float32 array of n elements reads two order statistics and blends
-    them with a weight; this returns (rank_lo, rank_hi, gamma) exactly as numpy computes them for float32 input: the
-    quantile q/100, the virtual index and gamma are all float32 there (numpy/lib/_function_base_impl.py: percentile,
-    _QuantileMethods['linear'], _get_indexes, _get_gamma), which matters at megapixel sizes."""
-    quant = np.true_divide(q, np.float32(100))
-    vi = np.asanyarray((n - 1) * quant)                                       # method 'linear'
-    prev = np.floor(vi)
-    if vi >= n - 1:
-        lo = hi = n - 1
-    elif vi < 0:
-        lo = hi = 0
-    else:
-        lo, hi = int(prev), int(prev) + 1
-    gamma = np.asanyarray(np.asanyarray(vi - np.asanyarray(prev).astype(np.intp)), dtype=vi.dtype)
-    return lo, hi, gamma
-
-
-def percentile_from_order_stats(lo_value, hi_value, gamma):
-    """The blend of numpy's _lerp on float32 operands (two-sided, all float32)."""
-    a, b = np.asanyarray(np.float32(lo_value)), np.asanyarray(np.float32(hi_value))
-    diff = np.subtract(b, a)
-    res = np.asanyarray(np.add(a, diff * gamma))
-    if gamma >= 0.5:
-        res = np.asanyarray(np.subtract(b, diff * (1 - gamma)))
-    return float(res)
-
-
-def visualise(flow, mask, mode, show_mask, show_mask_borders, range_max, thr):
-    """Flow.visualise on the device (flow_class.py:869-951), one frame: flow [1,H,W,2], mask [1,H,W] or None."""
-    _, h, w = flow.shape[:3]
-    n = h * w
-    st = dev.current_stream()
-    if range_max is None:
-        mag = DeviceArray.empty((n,), np.float32)
-        res = DeviceArray.empty((4,), np.float32)            # {max, sorted[k0], sorted[k1], -}
-        _lib.call('ofk_vis_magnitude', flow.ptr, float(thr), mag.ptr, res.ptr, n, st)
-        k0, k1, gamma = percentile_plan(n)
-        ranks = (ctypes.c_ulonglong * 2)(k0, k1)
-        ws_bytes = _lib.call('ofk_kth_smallest_workspace', 2)
-        ws = DeviceArray.empty((ws_bytes,), np.uint8)
-        _lib.call('ofk_kth_smallest', mag.ptr, n, ranks, 2, res.ptr + 4, ws.ptr, ws_bytes, st)
-        r = res.numpy()
-        p99 = percentile_from_order_stats(r[1], r[2], gamma)
-        if p99 > 0:                                           # 99th percentile: extreme outliers do not skew the scale
-            range_max = p99
-        elif r[0]:                                            # percentile is 0: the actual maximum
-            range_max = float(r[0])
-        else:                                                 # the flow is zero everywhere
-            range_max = 1
-    if not isinstance(range_max, (float, int)):
-        raise TypeError("Error visualising flow: Range_max needs to be an integer or a float")
-    if range_max <= 0:
-        raise ValueError("Error visualising flow: Range_max needs to be larger than zero")
-    out = DeviceArray.empty((h, w, 3), np.uint8)
-    _lib.call('ofk_visualise', flow.ptr, _p(mask), float(thr), {'hsv': 0, 'rgb': 1, 'bgr': 2}[mode], int(show_mask),
-              int(show_mask_borders), float(np.float32(range_max)), out.ptr, h, w, st)
-    return out.numpy()
-
-
 def vis_range_arg(range_max):
     """The range_max argument of ofk_visualise_batch / ofh_visualise: 0 for None (each frame's default range, found
     on the device), else the float32 value. A positive range that float32 cannot hold (rounds to 0) becomes -1, which
-    the library rejects as ofk_visualise rejects it, instead of silently taking the default range."""
+    the library rejects, instead of silently taking the default range."""
     if range_max is None:
         return 0.0
     r = float(np.float32(range_max))
@@ -341,16 +279,6 @@ def greater(values, thr):
     out = DeviceArray.empty(values.shape, np.uint8)
     _lib.call('ofk_greater', values.ptr, float(thr), out.ptr, values.size, dev.current_stream())
     return out
-
-
-def track_bilinear(flow, pts):
-    """flow: DeviceArray [1,H,W,2]; pts: numpy float64 (n,2). Returns (numpy (n,2) float64, outside flag)."""
-    h, w = flow.shape[1:3]
-    p = DeviceArray.from_numpy(np.ascontiguousarray(pts, dtype=np.float64))
-    out = DeviceArray.empty(p.shape, np.float64)
-    bad = DeviceArray.empty((1,), np.int32)
-    _lib.call('ofk_track_bilinear', flow.ptr, p.ptr, p.shape[0], h, w, out.ptr, bad.ptr, dev.current_stream())
-    return out.numpy(), bool(bad.numpy()[0])
 
 
 TRACK_PTS_CODES = {np.dtype('float32'): _lib.F32, np.dtype('float64'): _lib.F64, np.dtype('int32'): _lib.I32,

@@ -8,7 +8,6 @@
 #include <algorithm>
 
 #include "ofk_common.cuh"
-#include "track_device.cuh"
 
 namespace ofk {
 
@@ -340,20 +339,6 @@ __global__ void __launch_bounds__(256) greater_kernel(const float* __restrict__ 
         out[i] = v[i] > thr ? 1 : 0;
 }
 
-// Flow vectors at float64 points (row, col) by exact bilinear interpolation (bilinear_track_point); out = pts + (v, u).
-// bad[0] is set when a point lies outside [0,H-1]x[0,W-1] (the reference raises IndexError).
-__global__ void __launch_bounds__(128) track_bilinear_kernel(const float* __restrict__ flow, const double* __restrict__ pts,
-                                                             size_t n, int H, int W, double* __restrict__ out,
-                                                             int* __restrict__ bad) {
-    const float2* f = reinterpret_cast<const float2*>(flow);
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
-        if (!bilinear_track_point(f, H, W, pts[i * 2], pts[i * 2 + 1], out[i * 2], out[i * 2 + 1])) {
-            *bad = 1;
-            out[i * 2] = out[i * 2 + 1] = 0.0;
-        }
-    }
-}
-
 __global__ void __launch_bounds__(256) inside_kernel(const double* __restrict__ pts, size_t n, int H, int W,
                                                      uint8_t* __restrict__ out) {
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
@@ -588,18 +573,6 @@ extern "C" int ofk_greater(const float* v, float thr, uint8_t* out, size_t n, of
     OFK_CHECK_ARG(v && out, "ofk_greater: NULL argument");
     if (n == 0) return OFK_OK;
     greater_kernel<<<stream_grid(n, 256), 256, 0, as_stream(stream)>>>(v, thr, out, n);
-    OFK_LAUNCHED();
-    return OFK_OK;
-}
-
-extern "C" int ofk_track_bilinear(const float* flow, const double* pts, size_t n, int H, int W, double* out, int* bad,
-                                  ofk_stream_t stream) {
-    OFK_CHECK_ARG(flow && pts && out && bad, "ofk_track_bilinear: NULL argument");
-    OFK_CHECK_ARG(H > 0 && W > 0, "ofk_track_bilinear: bad shape");
-    cudaStream_t st = as_stream(stream);
-    OFK_CUDA(cudaMemsetAsync(bad, 0, sizeof(int), st));
-    if (n == 0) return OFK_OK;
-    track_bilinear_kernel<<<stream_grid(n, 128), 128, 0, st>>>(flow, pts, n, H, W, out, bad);
     OFK_LAUNCHED();
     return OFK_OK;
 }

@@ -14,7 +14,7 @@ namespace ofk {
 
 // ref 's' lookup, one thread per point: integer points (in any mode) index the flow like numpy (an index in [-H,-1]
 // wraps) and add the vector in the arithmetic type AT (numpy's result type of pts + float32); float points (without
-// exact mode) interpolate it bilinearly in float64 (ofk_track_bilinear's arithmetic).
+// exact mode) interpolate it bilinearly in float64 (bilinear_track_point).
 template <typename PT, typename AT>
 __global__ void __launch_bounds__(256) track_s_kernel(const float2* __restrict__ flow, const uint8_t* __restrict__ mask,
                                                       const int* __restrict__ flow_nonzero, const PT* __restrict__ pts,

@@ -1,6 +1,5 @@
-// Per-point arithmetic of point tracking (Flow.track, utils.py:547-622), shared by ofk_track_bilinear (elementwise.cu),
-// the lookup kernel of ofk_track (track.cu), its mesh kernel and the trajectory kernel of ofk_track_clips
-// (forward_s.cu).
+// Per-point arithmetic of point tracking (Flow.track, utils.py:547-622), shared by the lookup kernel of ofk_track
+// (track.cu), its mesh kernel and the trajectory kernel of ofk_track_clips (forward_s.cu).
 #pragma once
 #include <math.h>
 

@@ -1,5 +1,5 @@
 // Flow visualisation on the device (SURVEY 8f rank 4): Flow.visualise of the reference (flow_class.py:869-951), for a
-// batch of N frames. The one-frame entry points are the N = 1 case of the same kernels.
+// batch of N frames. The package's Flow.visualise is the N = 1 case.
 //
 //   magnitude_kernel : mag[n,p] = |threshold(flow[n,p])| exactly as cv2.cartToPolar computes it (float32,
 //                      sqrt(fma(x, x, y*y))), the maximum of each frame and, fused, the first histogram pass of the
@@ -47,51 +47,43 @@ __device__ __forceinline__ float fast_atan2_deg(float y, float x) {
 
 // ------------------------------------------------------------------------------------------------ radix selection
 // (digits, histogram helpers: radix_select.cuh)
-constexpr int kMaxRanks = 4;
+constexpr int kRanks = 2;   // the two order statistics numpy.percentile(mag, 99) interpolates between
 
-// Per-frame selection record: head, then the histograms (pass 0: one, shared by every rank since no prefix is fixed
+// Per-frame selection record: head, then the histograms (pass 0: one, shared by both ranks since no prefix is fixed
 // yet; passes 1 and 2: one per rank). Zeroed before the magnitude / first histogram pass.
 struct SelectHead {
     unsigned int max_bits;            // maximum magnitude of the frame (bit pattern)
     float range;                      // the frame's range_max, written by the last pick
-    unsigned int prefix[kMaxRanks];   // digits found so far
-    unsigned int rank[kMaxRanks];     // rank still to resolve among the values with that prefix
+    unsigned int prefix[kRanks];      // digits found so far
+    unsigned int rank[kRanks];        // rank still to resolve among the values with that prefix
 };
 constexpr size_t kHeadBytes = 256;
 static_assert(sizeof(SelectHead) <= kHeadBytes, "SelectHead");
+constexpr size_t kSelectFrameBytes = kHeadBytes + sizeof(unsigned int) * (kBins0 + 2 * kRanks * kBins12);
 
-__host__ __device__ constexpr size_t select_frame_bytes(int nq) {
-    return kHeadBytes + sizeof(unsigned int) * (kBins0 + 2 * (size_t)nq * kBins12);
-}
-__host__ __device__ inline unsigned int* pass_hist(char* frame, int pass, int nq, int q) {
+__host__ __device__ inline unsigned int* pass_hist(char* frame, int pass, int q) {
     unsigned int* h = reinterpret_cast<unsigned int*>(frame + kHeadBytes);
     if (pass == 0) return h;
-    return h + kBins0 + ((size_t)(pass - 1) * nq + q) * kBins12;
+    return h + kBins0 + ((size_t)(pass - 1) * kRanks + q) * kBins12;
 }
 
-// Where the selection records of N frames live: frame n at base + n * stride.
+// Where the selection records of N frames live: frame n at base + n * kSelectFrameBytes.
 struct Select {
     char* base;
-    size_t stride;
-    int nq;
-    __device__ SelectHead* head(size_t n) const { return reinterpret_cast<SelectHead*>(base + n * stride); }
+    __device__ char* frame(size_t n) const { return base + n * kSelectFrameBytes; }
+    __device__ SelectHead* head(size_t n) const { return reinterpret_cast<SelectHead*>(frame(n)); }
 };
 
 constexpr int kUnroll = 4;   // elements per thread and loop trip, strided by the block (coalesced)
 
 // bpf blocks per frame, frame-major on grid x (block b of frame n is blockIdx.x = n * bpf + b: no limit on N but
-// grid x's). mag of frame n at mag + n * mag_stride; max_bits at max_base + n * max_stride (uints); sel.base == nullptr:
-// no histogram (ofk_vis_magnitude).
+// grid x's). mag of frame n at mag + n * mag_stride; the maximum and the pass-0 histogram go to the frame's record.
 __global__ void __launch_bounds__(256) magnitude_kernel(const float2* __restrict__ flow, float thr,
                                                         float* __restrict__ mag, size_t mag_stride, size_t hw,
-                                                        unsigned int* __restrict__ max_base, size_t max_stride,
                                                         Select sel, int bpf) {
     __shared__ unsigned int sh[kBins0];
-    const bool hist = sel.base != nullptr;
-    if (hist) {
-        for (int k = threadIdx.x; k < kBins0; k += blockDim.x) sh[k] = 0;
-        __syncthreads();
-    }
+    for (int k = threadIdx.x; k < kBins0; k += blockDim.x) sh[k] = 0;
+    __syncthreads();
     const size_t n = blockIdx.x / bpf, blk = blockIdx.x - n * bpf;
     const float2* f = flow + n * hw;
     float* m = mag + n * mag_stride;
@@ -112,32 +104,30 @@ __global__ void __launch_bounds__(256) magnitude_kernel(const float2* __restrict
                 m[i] = __uint_as_float(b);
                 mx = max(mx, b);
             }
-            if (hist) hist_add(sh, b >> 20, i < hw);
+            hist_add(sh, b >> 20, i < hw);
         }
     }
     mx = __reduce_max_sync(0xffffffffu, mx);
-    if ((threadIdx.x & 31) == 0 && mx) atomicMax(max_base + n * max_stride, mx);
-    if (hist) {
-        __syncthreads();
-        flush_hist(sh, pass_hist(sel.base + n * sel.stride, 0, sel.nq, 0), kBins0);
-    }
+    if ((threadIdx.x & 31) == 0 && mx) atomicMax(&sel.head(n)->max_bits, mx);
+    __syncthreads();
+    flush_hist(sh, pass_hist(sel.frame(n), 0, 0), kBins0);
 }
 
-// One histogram pass of the selection over the values of every frame (bpf blocks per frame on grid x): pass 0 counts
-// every value into one histogram, passes 1 and 2 count, per rank, the values whose higher digits equal its prefix.
+// Histogram pass 1 or 2 of the selection over the values of every frame (bpf blocks per frame on grid x): per rank, the
+// values whose higher digits equal its prefix. Pass 0 is fused into magnitude_kernel.
 template <int PASS>
 __global__ void __launch_bounds__(256) hist_kernel(const unsigned int* __restrict__ values, size_t stride, size_t n_vals,
                                                    Select sel, int bpf) {
-    constexpr int kBins = pass_bins(PASS), kShift = pass_shift(PASS);
-    constexpr unsigned int kHiMask = PASS == 0 ? 0u : ~0u << (kShift + 10);
-    __shared__ unsigned int sh[PASS == 0 ? kBins0 : kMaxRanks * kBins12];
+    static_assert(PASS == 1 || PASS == 2, "pass 0 runs in magnitude_kernel");
+    constexpr int kShift = pass_shift(PASS);
+    constexpr unsigned int kHiMask = ~0u << (kShift + 10);
+    __shared__ unsigned int sh[kRanks * kBins12];
     const size_t n = blockIdx.x / bpf, blk = blockIdx.x - n * bpf;
-    const int nh = PASS == 0 ? 1 : sel.nq;
-    for (int k = threadIdx.x; k < nh * kBins; k += blockDim.x) sh[k] = 0;
-    unsigned int prefix[kMaxRanks];
+    for (int k = threadIdx.x; k < kRanks * kBins12; k += blockDim.x) sh[k] = 0;
+    unsigned int prefix[kRanks];
     const SelectHead* hd = sel.head(n);
 #pragma unroll
-    for (int q = 0; q < kMaxRanks; ++q) prefix[q] = q < nh ? hd->prefix[q] : 0u;
+    for (int q = 0; q < kRanks; ++q) prefix[q] = hd->prefix[q];
     __syncthreads();
     const unsigned int* v = values + n * stride;
     const size_t step = (size_t)bpf * blockDim.x * kUnroll;
@@ -151,20 +141,19 @@ __global__ void __launch_bounds__(256) hist_kernel(const unsigned int* __restric
 #pragma unroll
         for (int j = 0; j < kUnroll; ++j) {
             const bool in = base + j * blockDim.x + threadIdx.x < n_vals;
-            const unsigned int bin = (b[j] >> kShift) & (kBins - 1);
-            for (int q = 0; q < nh; ++q) {
+            const unsigned int bin = (b[j] >> kShift) & (kBins12 - 1);
+            for (int q = 0; q < kRanks; ++q) {
                 const bool hit = in && (b[j] & kHiMask) == prefix[q];
-                if (__any_sync(0xffffffffu, hit)) hist_add(sh + q * kBins, bin, hit);
+                if (__any_sync(0xffffffffu, hit)) hist_add(sh + q * kBins12, bin, hit);
             }
         }
     }
     __syncthreads();
-    char* fr = sel.base + n * sel.stride;
-    for (int q = 0; q < nh; ++q) flush_hist(sh + q * kBins, pass_hist(fr, PASS, sel.nq, q), kBins);
+    for (int q = 0; q < kRanks; ++q) flush_hist(sh + q * kBins12, pass_hist(sel.frame(n), PASS, q), kBins12);
 }
 
 struct Ranks {
-    unsigned int r[kMaxRanks];
+    unsigned int r[kRanks];
 };
 
 // numpy's _lerp on float32 operands (two-sided, all float32, no contraction)
@@ -176,18 +165,17 @@ __device__ __forceinline__ float lerp_np(float a, float b, float gamma) {
 }
 
 // One block per frame: for each rank, the bin of this pass whose cumulative count passes the rank (block-wide scan).
-// Pass 0 starts from `ranks`. After pass 2 the prefixes are the values: with out != nullptr they are written to out
-// (frame 0 only: ofk_kth_smallest), otherwise ranks 0 / 1 are blended with gamma and the range rule gives head.range.
+// Pass 0 starts from `ranks`. After pass 2 the prefixes are the two order statistics: they are blended with gamma and
+// the range rule gives head.range.
 template <int PASS>
-__global__ void __launch_bounds__(256) pick_kernel(Select sel, Ranks ranks, float gamma, float* __restrict__ out) {
+__global__ void __launch_bounds__(256) pick_kernel(Select sel, Ranks ranks, float gamma) {
     constexpr int kBins = pass_bins(PASS), kShift = pass_shift(PASS), kPer = kBins / 256;
     __shared__ unsigned int warp_sum[8];
     const size_t n = blockIdx.x;
-    char* fr = sel.base + n * sel.stride;
     SelectHead* hd = sel.head(n);
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    for (int q = 0; q < sel.nq; ++q) {
-        const unsigned int* h = pass_hist(fr, PASS, sel.nq, q) + threadIdx.x * kPer;
+    for (int q = 0; q < kRanks; ++q) {
+        const unsigned int* h = pass_hist(sel.frame(n), PASS, q) + threadIdx.x * kPer;
         const unsigned int rank = PASS == 0 ? ranks.r[q] : hd->rank[q];
         unsigned int c[kPer], local = 0;
 #pragma unroll
@@ -221,12 +209,8 @@ __global__ void __launch_bounds__(256) pick_kernel(Select sel, Ranks ranks, floa
         __syncthreads();
     }
     if (PASS == 2 && threadIdx.x == 0) {
-        if (out != nullptr) {
-            for (int q = 0; q < sel.nq; ++q) out[q] = __uint_as_float(hd->prefix[q]);
-        } else {
-            const float p99 = lerp_np(__uint_as_float(hd->prefix[0]), __uint_as_float(hd->prefix[1]), gamma);
-            hd->range = p99 > 0.f ? p99 : (hd->max_bits ? __uint_as_float(hd->max_bits) : 1.f);
-        }
+        const float p99 = lerp_np(__uint_as_float(hd->prefix[0]), __uint_as_float(hd->prefix[1]), gamma);
+        hd->range = p99 > 0.f ? p99 : (hd->max_bits ? __uint_as_float(hd->max_bits) : 1.f);
     }
 }
 
@@ -365,7 +349,7 @@ __global__ void __launch_bounds__(256) colourise_kernel(const float2* __restrict
 // ------------------------------------------------------------------------------------------------ host helpers
 // numpy.percentile(a, 99) of n float32 values (method 'linear', numpy 2.x): ranks lo / hi and the weight, all float32
 // as numpy computes them for float32 input (numpy/lib/_function_base_impl.py: _QuantileMethods['linear'],
-// _get_indexes, _get_gamma). _ops.percentile_plan is the same plan in Python.
+// _get_indexes, _get_gamma).
 struct Plan {
     unsigned int lo, hi;
     float gamma;
@@ -393,26 +377,26 @@ static int blocks_per_frame(size_t n_vals, size_t frames) {
     return (int)std::min<size_t>(std::min(want, most), std::max<size_t>(1, 0x7fffffffu / frames));
 }
 
-// The three histogram / pick passes over values (frame n at values + n * stride), pass 0 optionally fused into the
-// magnitude kernel by the caller (fused = true).
-static int run_selection(const float* values, size_t stride, size_t n_vals, int N, Select sel, Ranks ranks,
-                         float gamma, float* out, bool fused, cudaStream_t st) {
-    const int bpf = blocks_per_frame(n_vals, N);
+// The default range of every frame into its selection record (zeroed by the caller): the magnitudes with the maximum
+// and the first histogram pass, then the pick / histogram passes over the magnitudes.
+static int find_ranges(const float* flow, float thr, float* mag, size_t mag_stride, size_t hw, int N, Select sel,
+                       cudaStream_t st) {
+    const int bpf = blocks_per_frame(hw, N);
     const unsigned int grid = (unsigned int)bpf * (unsigned int)N;
-    const unsigned int* v = reinterpret_cast<const unsigned int*>(values);
-    if (!fused) {
-        hist_kernel<0><<<grid, 256, 0, st>>>(v, stride, n_vals, sel, bpf);
-        OFK_LAUNCHED();
-    }
-    pick_kernel<0><<<N, 256, 0, st>>>(sel, ranks, gamma, out);
+    const Plan plan = percentile_plan(hw);
+    const Ranks ranks = {{plan.lo, plan.hi}};
+    const unsigned int* v = reinterpret_cast<const unsigned int*>(mag);
+    magnitude_kernel<<<grid, 256, 0, st>>>(reinterpret_cast<const float2*>(flow), thr, mag, mag_stride, hw, sel, bpf);
     OFK_LAUNCHED();
-    hist_kernel<1><<<grid, 256, 0, st>>>(v, stride, n_vals, sel, bpf);
+    pick_kernel<0><<<N, 256, 0, st>>>(sel, ranks, plan.gamma);
     OFK_LAUNCHED();
-    pick_kernel<1><<<N, 256, 0, st>>>(sel, ranks, gamma, out);
+    hist_kernel<1><<<grid, 256, 0, st>>>(v, mag_stride, hw, sel, bpf);
     OFK_LAUNCHED();
-    hist_kernel<2><<<grid, 256, 0, st>>>(v, stride, n_vals, sel, bpf);
+    pick_kernel<1><<<N, 256, 0, st>>>(sel, ranks, plan.gamma);
     OFK_LAUNCHED();
-    pick_kernel<2><<<N, 256, 0, st>>>(sel, ranks, gamma, out);
+    hist_kernel<2><<<grid, 256, 0, st>>>(v, mag_stride, hw, sel, bpf);
+    OFK_LAUNCHED();
+    pick_kernel<2><<<N, 256, 0, st>>>(sel, ranks, plan.gamma);
     OFK_LAUNCHED();
     return OFK_OK;
 }
@@ -438,59 +422,9 @@ static size_t mag_frame_bytes(int H, int W) { return pad256((size_t)H * W * size
 
 using namespace ofk;
 
-extern "C" int ofk_vis_magnitude(const float* flow, float thr, float* mag, float* max_out, size_t n_pixels,
-                                 ofk_stream_t stream) {
-    OFK_CHECK_ARG(flow != nullptr && mag != nullptr && max_out != nullptr, "ofk_vis_magnitude: NULL pointer");
-    OFK_CHECK_ARG((reinterpret_cast<uintptr_t>(flow) & 7) == 0, "ofk_vis_magnitude: flow must be 8-byte aligned");
-    cudaStream_t st = as_stream(stream);
-    OFK_CUDA(cudaMemsetAsync(max_out, 0, sizeof(float), st));
-    if (n_pixels == 0) return OFK_OK;
-    const vis::Select none = {nullptr, 0, 0};
-    const int bpf = vis::blocks_per_frame(n_pixels, 1);
-    vis::magnitude_kernel<<<bpf, 256, 0, st>>>(reinterpret_cast<const float2*>(flow), thr, mag, 0, n_pixels,
-                                               reinterpret_cast<unsigned int*>(max_out), 0, none, bpf);
-    OFK_LAUNCHED();
-    return OFK_OK;
-}
-
-extern "C" size_t ofk_kth_smallest_workspace(int n_ranks) {
-    if (n_ranks < 1 || n_ranks > vis::kMaxRanks) return 0;
-    return vis::select_frame_bytes(n_ranks);
-}
-
-extern "C" int ofk_kth_smallest(const float* values, size_t n, const unsigned long long* ranks_host, int n_ranks,
-                                float* out, void* ws, size_t ws_bytes, ofk_stream_t stream) {
-    OFK_CHECK_ARG(values != nullptr && out != nullptr && ranks_host != nullptr, "ofk_kth_smallest: NULL pointer");
-    OFK_CHECK_ARG(n_ranks >= 1 && n_ranks <= 4, "ofk_kth_smallest: 1 to 4 ranks per call, got %d", n_ranks);
-    OFK_CHECK_ARG(n > 0, "ofk_kth_smallest: empty array");
-    OFK_CHECK_ARG(n <= 0xffffffffull, "ofk_kth_smallest: at most 2^32 - 1 values (32-bit counts), got %zu", n);
-    vis::Ranks ranks = {};
-    for (int q = 0; q < n_ranks; ++q) {
-        OFK_CHECK_ARG(ranks_host[q] < n, "ofk_kth_smallest: rank %llu out of range (n = %zu)", ranks_host[q], n);
-        ranks.r[q] = (unsigned int)ranks_host[q];
-    }
-    OFK_CHECK_ARG(ws != nullptr && ws_bytes >= ofk_kth_smallest_workspace(n_ranks), "ofk_kth_smallest: workspace too small");
-    cudaStream_t st = as_stream(stream);
-    const vis::Select sel = {static_cast<char*>(ws), vis::select_frame_bytes(n_ranks), n_ranks};
-    OFK_CUDA(cudaMemsetAsync(ws, 0, sel.stride, st));
-    return vis::run_selection(values, 0, n, 1, sel, ranks, 0.f, out, false, st);
-}
-
-extern "C" int ofk_visualise(const float* flow, const uint8_t* mask, float thr, int mode, int show_mask,
-                             int show_mask_borders, float range_max, uint8_t* out, int H, int W, ofk_stream_t stream) {
-    OFK_CHECK_ARG(flow != nullptr && out != nullptr, "ofk_visualise: NULL pointer");
-    OFK_CHECK_ARG(H > 0 && W > 0, "ofk_visualise: bad shape H=%d W=%d", H, W);
-    OFK_CHECK_ARG(mode >= 0 && mode <= 2, "ofk_visualise: mode must be 0 (hsv), 1 (rgb) or 2 (bgr)");
-    OFK_CHECK_ARG(range_max > 0.f, "ofk_visualise: range_max must be positive");
-    OFK_CHECK_ARG((reinterpret_cast<uintptr_t>(flow) & 7) == 0, "ofk_visualise: flow must be 8-byte aligned");
-    const vis::RangeSrc range = {nullptr, 0, range_max};
-    return vis::launch_colourise(flow, mask, thr, mode, show_mask, show_mask_borders, range, out, 1, H, W,
-                                 as_stream(stream));
-}
-
 extern "C" size_t ofk_visualise_batch_workspace(int N, int H, int W) {
     if (N < 0 || H <= 0 || W <= 0) return 0;
-    return (size_t)N * (vis::mag_frame_bytes(H, W) + vis::select_frame_bytes(2));
+    return (size_t)N * (vis::mag_frame_bytes(H, W) + vis::kSelectFrameBytes);
 }
 
 extern "C" int ofk_visualise_batch(const float* flow, const uint8_t* mask, float thr, int mode, int show_mask,
@@ -513,21 +447,11 @@ extern "C" int ofk_visualise_batch(const float* flow, const uint8_t* mask, float
         return vis::launch_colourise(flow, mask, thr, mode, show_mask, show_mask_borders, range, out, N, H, W, st);
     }
     // ws: magnitudes of N frames, then N selection records
-    const size_t hw = (size_t)H * W, mag_stride = vis::mag_frame_bytes(H, W) / sizeof(float);
-    float* mag = static_cast<float*>(ws);
-    const vis::Select sel = {static_cast<char*>(ws) + (size_t)N * vis::mag_frame_bytes(H, W),
-                             vis::select_frame_bytes(2), 2};
-    OFK_CUDA(cudaMemsetAsync(sel.base, 0, sel.stride * N, st));
-    const int bpf = vis::blocks_per_frame(hw, N);
-    vis::magnitude_kernel<<<(unsigned int)bpf * (unsigned int)N, 256, 0, st>>>(
-        reinterpret_cast<const float2*>(flow), thr, mag, mag_stride, hw,
-        reinterpret_cast<unsigned int*>(sel.base + offsetof(vis::SelectHead, max_bits)),
-        sel.stride / sizeof(unsigned int), sel, bpf);
-    OFK_LAUNCHED();
-    const vis::Plan plan = vis::percentile_plan(hw);
-    const vis::Ranks ranks = {{plan.lo, plan.hi, 0u, 0u}};
-    const int rc = vis::run_selection(mag, mag_stride, hw, N, sel, ranks, plan.gamma, nullptr, true, st);
+    const size_t mag_stride = vis::mag_frame_bytes(H, W) / sizeof(float);
+    const vis::Select sel = {static_cast<char*>(ws) + (size_t)N * vis::mag_frame_bytes(H, W)};
+    OFK_CUDA(cudaMemsetAsync(sel.base, 0, vis::kSelectFrameBytes * N, st));
+    const int rc = vis::find_ranges(flow, thr, static_cast<float*>(ws), mag_stride, (size_t)H * W, N, sel, st);
     if (rc != OFK_OK) return rc;
-    const vis::RangeSrc range = {sel.base + offsetof(vis::SelectHead, range), sel.stride, 0.f};
+    const vis::RangeSrc range = {sel.base + offsetof(vis::SelectHead, range), vis::kSelectFrameBytes, 0.f};
     return vis::launch_colourise(flow, mask, thr, mode, show_mask, show_mask_borders, range, out, N, H, W, st);
 }

@@ -16,8 +16,8 @@ from . import _lib
 from . import _ops
 from . import device as dev
 from .device import DeviceArray
-from .validation import get_valid_ref, get_valid_padding, validate_shape, validate_visualise_args, \
-    validate_track_args, validate_consistency_args, validate_evaluate_args, DEFAULT_THRESHOLD
+from .validation import get_valid_ref, get_valid_padding, validate_shape, validate_track_args, \
+    validate_consistency_args, validate_evaluate_args, DEFAULT_THRESHOLD
 
 __all__ = ['Flow']
 
@@ -559,13 +559,22 @@ class Flow(object):
         return Flow._wrap(_ops.scale(_lib.OP_MUL, self._vd(), -1.0, -1.0, False), ref, self._md().copy())
 
     def track(self, pts, int_out=None, get_valid_status=None, s_exact_mode=None):
-        from .ops import _track_device
+        """Points (P,2) given as (row, col) tracked with this flow (flow_class.py:755-795): ``FlowBatch.track`` of the
+        one frame, through the same call. A flow that is zero below the threshold hands ``pts`` back unchanged (rounded
+        with ``int_out``), as the reference does, whatever their dtype."""
+        from .batch import FlowBatch
         int_out, get_valid_status, s_exact_mode = validate_track_args(pts, int_out, get_valid_status, s_exact_mode)
-        warped = _track_device(self, pts, int_out, s_exact_mode)
+        if int(_ops.nonzero_flags(self._vd(), None, DEFAULT_THRESHOLD)[0]) == 0:
+            warped = np.round(pts).astype('i') if int_out else pts
+            if get_valid_status:
+                return warped, self.valid_source()[np.round(pts[..., 0]).astype('i'), np.round(pts[..., 1]).astype('i')]
+            return warped
+        if self._ref == 't' and not (np.issubdtype(pts.dtype, np.integer) or np.issubdtype(pts.dtype, np.floating)):
+            pts = pts.astype(np.float64)        # the reference checks the dtype for 's' only (utils.py:600-602)
+        res = FlowBatch._wrap(self._vd(), self._ref, self._md()).track(pts, int_out, get_valid_status, s_exact_mode)
         if get_valid_status:
-            status = self.valid_source()[np.round(pts[..., 0]).astype('i'), np.round(pts[..., 1]).astype('i')]
-            return warped, status
-        return warped
+            return res[0].numpy()[0], res[1].numpy()[0].view(np.bool_)
+        return res.numpy()[0]
 
     # ------------------------------------------------------------------------------------------ valid areas
     def valid_target(self, consider_mask=None):
@@ -595,9 +604,11 @@ class Flow(object):
     def visualise(self, mode, show_mask=None, show_mask_borders=None, range_max=None):
         """Flow as an rgb / bgr / hsv image (flow_class.py:869-951): hue = direction, saturation = magnitude scaled to
         `range_max` (default: 99th percentile of the magnitudes, found by radix selection on the device), optionally
-        invalid areas greyed out and the mask outline in black. Returns a numpy uint8 array (H, W, 3)."""
-        _, show_mask, show_mask_borders = validate_visualise_args(mode, show_mask, show_mask_borders, range_max)
-        return _ops.visualise(self._vd(), self._md(), mode, show_mask, show_mask_borders, range_max, DEFAULT_THRESHOLD)
+        invalid areas greyed out and the mask outline in black: ``FlowBatch.visualise`` of the one frame, through the
+        same call. Returns a numpy uint8 array (H, W, 3)."""
+        from .batch import FlowBatch
+        batch = FlowBatch._wrap(self._vd(), self._ref, self._md())
+        return batch.visualise(mode, show_mask, show_mask_borders, range_max).numpy()[0]
 
     # ---- host-side presentation / estimation (SURVEY section 2 rows 19-20: not on the hot path, delegated)
     def _host_reference(self):

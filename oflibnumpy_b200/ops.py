@@ -11,8 +11,8 @@ from . import _lib
 from . import _ops
 from .device import DeviceArray
 from .flow import Flow
-from .validation import (get_valid_ref, validate_shape, validate_flow_array, validate_transform_list,
-                         validate_track_args, validate_track_dtype, DEFAULT_THRESHOLD)
+from .validation import get_valid_ref, validate_shape, validate_flow_array, validate_transform_list, \
+    DEFAULT_THRESHOLD
 
 __all__ = ['apply_flow', 'combine_flows', 'invert_flow', 'switch_flow_ref', 'valid_target', 'valid_source',
            'get_flow_padding', 'from_matrix', 'from_transforms', 'matrix_from_transforms', 'matrix_from_transform',
@@ -211,53 +211,10 @@ def resize_flow(flow, scale):
     return out.numpy()[0]
 
 
-def _track_device(flow, pts, int_out, s_exact_mode):
-    """Point tracking (utils.py:547-622) on the device. `flow` is a Flow object; the arguments have passed
-    validate_track_args."""
-    vecs = flow._vd()
-    if int(_ops.nonzero_flags(vecs, None, DEFAULT_THRESHOLD)[0]) == 0:      # thresholded-zero flow: points unchanged
-        warped = pts
-    else:
-        if flow.ref == 's' and np.issubdtype(pts.dtype, np.integer):
-            # direct lookup of the vectors at integer positions: a gather through the same mesh sampler would be
-            # overkill; the points are few, so index a (lazy) host view like the reference does
-            d = vecs.numpy()[0][pts[:, 0], pts[:, 1], ::-1]
-            warped = pts + d
-        elif flow.ref == 's' and not np.issubdtype(pts.dtype, np.floating):
-            validate_track_dtype(pts.dtype)
-        elif flow.ref == 's' and not s_exact_mode:
-            warped, outside = _ops.track_bilinear(vecs, pts)
-            if outside:
-                raise IndexError("Some points are outside of the data area.")
-        else:
-            # 's' exact mode: interpolate the flow on the undisplaced grid; 't': on the grid displaced by -flow
-            zero = DeviceArray.zeros(vecs.shape, np.float32) if flow.ref == 's' else None
-            mesh = zero if flow.ref == 's' else vecs
-            q = DeviceArray.from_numpy(np.ascontiguousarray(pts, dtype=np.float64)[None])
-            vals, _, found = _ops.mesh_sample(mesh, -1.0, vecs, None, query_pts=q, want_mask=False, want_found=True)
-            d = vals.numpy()[0].astype(np.float64)[:, ::-1]
-            warped = pts + d
-            warped[found.numpy()[0] == 0] = 0                               # NaN rows of griddata -> 0 (utils.py:616-618)
-    if int_out:
-        warped = np.round(warped).astype('i')
-    return warped
-
-
 def track_pts(flow, ref, pts, int_out=None, s_exact_mode=None):
     """Warp points (N,2) given as (row, col) with a flow field (utils.py:547-622)."""
     flow = validate_flow_array(flow, "Error tracking points: ")
-    flow = Flow(flow, ref)
-    int_out, _, s_exact_mode = validate_track_args(pts, int_out, None, s_exact_mode)
-    return _track_device(flow, pts, int_out, s_exact_mode)
-
-
-def _combine2_t_device(a, b):
-    """combine_with(mode=2) for ref 't' (flow_class.py:1398-1410): A, resampled from its source positions
-    grid - A to the source positions grid - B of B, is subtracted from B."""
-    vals, mval, _ = _ops.mesh_sample(a._vd(), -1.0, a._vd(), a._md(), query_flow=b._vd(), query_sign=-1.0,
-                                     pos_f32=True)
-    resampled = Flow._wrap(vals, 't', _ops.greater(mval, 0.99))
-    return b - resampled
+    return Flow(flow, ref).track(pts, int_out, s_exact_mode=s_exact_mode)
 
 
 # ---- host-side presentation / estimation wrappers of flow_operations.py:25-68,251-350 (SURVEY section 2 row 21: not on

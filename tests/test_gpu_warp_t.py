@@ -729,7 +729,7 @@ def test_dataset_constructors_decode_on_device(of):
 
 
 def test_visualise_matches_reference_and_oracle(of):
-    """Flow.visualise on the device (ofk_vis_magnitude, ofk_kth_smallest, ofk_visualise) against the reference's own
+    """Flow.visualise on the device (ofk_visualise_batch of one frame) against the reference's own
     outputs (tests/golden/visualise.npz) and, at 1080p, against the oracle: uint8 images, bit for bit -- hue from the
     same FMA polynomial as cv2.cartToPolar, default range from an exact radix selection of the 99th percentile."""
     from test_oracle_golden import VIS_VARIANTS

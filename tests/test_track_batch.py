@@ -1,11 +1,16 @@
-"""Batched point tracking: FlowBatch.track (ofk_track). Frame i of the result must equal
-Flow(vecs[i], ref, masks[i]).track(pts_i, ...) byte for byte, dtype included, on every route: 's' integer lookup, 's'
-float bilinear, 's' exact, 't', zero-flow frames and int_out; the status equals Flow.track's. IndexError is raised where
-a loop of Flow.track would raise, for the lowest such frame."""
+"""Batched point tracking: FlowBatch.track (ofk_track). Frame i of the result must equal the single-frame tracking of
+Flow(vecs[i], ref, masks[i]) as track_reference restates it, byte for byte, dtype included, on every route: 's' integer
+lookup, 's' float bilinear, 's' exact, 't', zero-flow frames and int_out; the status equals the reference's. IndexError
+is raised where a loop of Flow.track would raise, for the lowest such frame. Flow.track itself, the one-frame case of
+FlowBatch.track, is held to the same reference."""
+import itertools
+
 import numpy as np
 import pytest
 
+import track_reference
 from conftest import load_golden
+from oracle import flowref as R
 
 PT_DTYPES = (np.float64, np.float32, np.int64, np.int32, np.int16)
 
@@ -159,8 +164,7 @@ def as_dtype(fpts, ipts, dt):
 
 
 def expected_frame(of, vecs, ref, masks, i, pts_i, int_out, status, exact):
-    f = of.Flow(vecs[i], ref, masks[i])
-    return f.track(pts_i, int_out, status, exact)
+    return track_reference.track(of.Flow(vecs[i], ref, masks[i]), pts_i, int_out, status, exact)
 
 
 def check_against_loop(of, vecs, masks, ref, fpts, ipts, zero_frames, shared_cases=(False, True)):
@@ -228,15 +232,53 @@ def test_next_rows_golden_in_a_batch(of):
             assert got_int.dtype == g['out_track_int_' + r].dtype
             assert np.abs(got_int[i] - g['out_track_int_' + r]).max() <= (1 if r == 't' else 0)
             np.testing.assert_allclose(got_i[i], g['out_track_ipts_' + r], rtol=0, atol=1e-3)
-            assert got[i].tobytes() == f.track(g['in_pts_f']).tobytes()
-            np.testing.assert_array_equal(got_st[i], f.track(g['in_pts_f'], get_valid_status=True)[1])
-            assert got_int[i].tobytes() == f.track(g['in_pts_f'], int_out=True).tobytes()
-            assert got_i[i].tobytes() == f.track(g['in_pts_i']).tobytes()
+            assert got[i].tobytes() == track_reference.track(f, g['in_pts_f']).tobytes()
+            np.testing.assert_array_equal(got_st[i], track_reference.track(f, g['in_pts_f'], get_valid_status=True)[1])
+            assert got_int[i].tobytes() == track_reference.track(f, g['in_pts_f'], int_out=True).tobytes()
+            assert got_i[i].tobytes() == track_reference.track(f, g['in_pts_i']).tobytes()
     fs = FlowBatch(np.stack([g['in_flow']] * 3), 's')
     got = fs.track(g['in_pts_f'], s_exact_mode=True).numpy()
+    want = track_reference.track(of.Flow(g['in_flow'], 's'), g['in_pts_f'], s_exact_mode=True)
     for i in range(3):
         np.testing.assert_allclose(got[i], g['out_track_exact_s'], rtol=0, atol=1e-3)
-        assert got[i].tobytes() == of.Flow(g['in_flow'], 's').track(g['in_pts_f'], s_exact_mode=True).tobytes()
+        assert got[i].tobytes() == want.tobytes()
+
+
+def check_flow_track(of, vecs, masks, ref, fpts, ipts):
+    """Flow.track of every frame against track_reference, byte for byte, for every point dtype and option. A flow that
+    is zero below the threshold hands back the points object itself (rounded with int_out); bool points are tracked as
+    float64 on a 't' flow and refused on a non-zero 's' flow."""
+    for i in range(len(vecs)):
+        f = of.Flow(vecs[i], ref, masks[i])
+        zero = R.is_zero_array(vecs[i])
+        for dt in PT_DTYPES + (np.bool_,):
+            pts = as_dtype(fpts, ipts, dt)[i]
+            for exact, int_out, status in itertools.product((False, True), repeat=3):
+                what = (ref, i, np.dtype(dt).name, exact, int_out, status)
+                if ref == 's' and dt is np.bool_ and not zero:
+                    for fn in (f.track, lambda *a: track_reference.track(f, *a)):
+                        with pytest.raises(TypeError, match="needs to have a float or int dtype"):
+                            fn(pts, int_out, status, exact)
+                    continue
+                got = f.track(pts, int_out, status, exact)
+                want = track_reference.track(f, pts, int_out, status, exact)
+                if status:
+                    (got, got_s), (want, want_s) = got, want
+                    assert got_s.dtype == want_s.dtype == np.bool_, what
+                    np.testing.assert_array_equal(got_s, want_s, err_msg=str(what))
+                assert (got is pts) == (want is pts) == (zero and not int_out), what
+                assert got.dtype == want.dtype and got.shape == want.shape, (what, got.dtype, want.dtype)
+                assert got.tobytes() == want.tobytes(), what
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize('ref', ['s', 't'])
+@pytest.mark.parametrize('size', [(1080, 1920, 6, 4096), (37, 53, 5, 300)], ids=['1080p', '37x53'])
+def test_flow_track_matches_the_reference(of, ref, size):
+    h, w, n, p = size
+    vecs, masks = make_batch(of, h, w, n, ref, seed=h)
+    fpts, ipts = make_points(h, w, n, p, 7)
+    check_flow_track(of, vecs, masks, ref, fpts, ipts)
 
 
 @pytest.mark.gpu

@@ -1,11 +1,12 @@
 """Point trajectories through clips: FlowBatch.track_clips (ofk_track_clips). Its oracle is the loop a user writes
 today, in this file: ``q = F[k].track(q)`` for every step, with the step rules of the docstring applied on the host
-through ``Flow.track``, ``Flow.track(get_valid_status=True)``, ``FlowBatch.valid_target()`` and numpy indexing, and the
-lost points dropped between the steps. On the CPU the same loop runs on ``oracle.flowref`` and is pinned on hand-made
+through the single-frame tracking and status of ``track_reference``, ``FlowBatch.valid_target()`` and numpy indexing,
+and the lost points dropped between the steps. On the CPU the same loop runs on ``oracle.flowref`` and is pinned on hand-made
 cases; on the GPU the kernel must give its positions byte for byte and its alive flags exactly."""
 import numpy as np
 import pytest
 
+import track_reference
 from oracle import flowref as R
 
 
@@ -59,17 +60,17 @@ class HostFrame(object):
 
 
 class DeviceFrame(object):
-    """One frame of the loop through the package's single-frame Flow.track."""
+    """One frame of the loop through the single-frame tracking of track_reference (device mesh, host bilinear)."""
 
     def __init__(self, flow, zero, target):
         self.f, self.zero, self.target = flow, zero, target
 
     def track(self, q, exact):
-        return self.f.track(q, s_exact_mode=exact)
+        return track_reference.track(self.f, q, s_exact_mode=exact)
 
     def status(self, q):
         # exact mode never raises, and the status does not depend on the mode
-        return self.f.track(q, get_valid_status=True, s_exact_mode=True)[1]
+        return track_reference.track(self.f, q, get_valid_status=True, s_exact_mode=True)[1]
 
 
 def loop_oracle(frames, pts, ref, exact, keep, h, w):
@@ -307,7 +308,7 @@ def make_points(h, w, S, P, seed):
 
 
 def device_loop(of, fb, vecs, pts, L, exact, keep):
-    """The loop of single-frame Flow.track calls over the batch fb (host vecs for the zero test)."""
+    """The loop of single-frame tracking steps (track_reference) over the batch fb (host vecs for the zero test)."""
     target = fb.valid_target().numpy() if fb.ref == 't' else [None] * len(fb)
     frames = [DeviceFrame(fb[i], R.is_zero_array(vecs[i]), target[i]) for i in range(len(fb))]
     h, w = fb.shape

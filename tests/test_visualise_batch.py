@@ -144,8 +144,8 @@ def test_1080p_batch_equals_flow_visualise_and_oracle(of):
 
 @pytest.mark.gpu
 def test_odd_shapes(of):
-    """Shapes whose rows do not fill whole 8-pixel groups, frames of one row or column, and single frames of the sizes
-    the host percentile test uses (up to 4K)."""
+    """Shapes whose rows do not fill whole 8-pixel groups, frames of one row or column, and single frames from 1x1 to
+    4K, where the device's plan of numpy.percentile(mag, 99) (float32 virtual index and lerp) must match numpy's."""
     from oflibnumpy_b200.batch import FlowBatch
     rng = np.random.default_rng(7)
     for (h, w) in ((1, 1), (1, 37), (29, 1), (37, 53), (5, 7), (9, 30), (13, 17)):

@@ -135,26 +135,16 @@ timeit("switch_ref / invert same-ref: forward_s of vecs||mask (18 B/px)", 18,
 timeit("apply 's' f32x3 + valid (8+12+12+1 = 33 B/px)", 33,
        lambda: c('ofk_forward_s', imgf.ptr, 3, fa.vecs.ptr, 1.0, None, None, o_imgf.ptr, o_m.ptr, _lib.RULE_STRICT, N, H,
                  W, ws.ptr, ws_bytes, s))
-# Flow.visualise is a per-frame call: default range (magnitudes + exact 99th percentile by radix selection) + colourise
-import ctypes  # noqa: E402
+# Flow.visualise is a per-frame call: ofk_visualise_batch of one frame, default range (magnitudes + exact 99th
+# percentile by radix selection, on the device) + colourise
 px_all, px = px, H * W
-mag = DeviceArray.empty((H * W,), np.float32)
-res4 = DeviceArray.empty((4,), np.float32)
 vis = DeviceArray.empty((H, W, 3), np.uint8)
-k0, k1, _g = _ops.percentile_plan(H * W)
-ranks = (ctypes.c_ulonglong * 2)(k0, k1)
-kws_b = c('ofk_kth_smallest_workspace', 2)
-kws = DeviceArray.empty((kws_b,), np.uint8)
-
-
-def vis_default():
-    c('ofk_vis_magnitude', fa.vecs.ptr, 1e-3, mag.ptr, res4.ptr, H * W, s)
-    c('ofk_kth_smallest', mag.ptr, H * W, ranks, 2, res4.ptr + 4, kws.ptr, kws_b, s)
-    c('ofk_visualise', fa.vecs.ptr, fa.masks.ptr, 1e-3, 1, 1, 1, 25.0, vis.ptr, H, W, s)
-
-
-timeit("visualise 'rgb', ONE frame, default range (8+1+3 = 12 B/px)", 12, vis_default)
+vws_b = c('ofk_visualise_batch_workspace', 1, H, W)
+vws = DeviceArray.empty((vws_b,), np.uint8)
+timeit("visualise 'rgb', ONE frame, default range (8+1+3 = 12 B/px)", 12,
+       lambda: c('ofk_visualise_batch', fa.vecs.ptr, fa.masks.ptr, 1e-3, 1, 1, 1, 0.0, vis.ptr, 1, H, W, vws.ptr, vws_b,
+                 s))
 timeit("visualise 'rgb', ONE frame, range_max given (12 B/px)", 12,
-       lambda: c('ofk_visualise', fa.vecs.ptr, fa.masks.ptr, 1e-3, 1, 1, 1, 25.0, vis.ptr, H, W, s))
+       lambda: c('ofk_visualise_batch', fa.vecs.ptr, fa.masks.ptr, 1e-3, 1, 1, 1, 25.0, vis.ptr, 1, H, W, None, 0, s))
 px = px_all
 print(json.dumps({"N": N, "H": H, "W": W, "peak_gbs": PEAK, "ops": results}))
