@@ -394,8 +394,9 @@ int ofk_decode_sintel_mask(const uint8_t* invalid, uint8_t* mask, size_t n_pixel
  *   point_mask    [N,H,W] or NULL: `consider_mask`, the points with 0 are removed before triangulating (utils.py:249-251)
  *   mask bytes    must be 0 or 1
  *   ws            device workspace of ofk_forward_s_workspace(N,H,W) bytes; payload/out may be NULL with C = 0
- * Folding fields (a displaced cell with a non-positive triangle) have no defined result in the reference; such frames
- * are resolved deterministically (largest source index wins, cells with a removed corner left empty).
+ * Folding fields (a displaced cell with a non-positive triangle anywhere in the frame): such a frame is triangulated
+ * as a whole -- every kept point is a vertex of the Delaunay triangulation griddata builds, and every pixel is located
+ * in it -- so the result is griddata's, at a far higher cost than a frame that does not fold.
  * ofk_forward_s_ex: flow_nonzero (int32 [N], device, e.g. from ofk_nonzero_flags(flow, NULL, 1e-3)) or NULL; frames
  * with 0 are passed through (out = payload, out_mask = payload_mask) like apply_flow's early return for a flow that is
  * zero below the threshold (utils.py:215-216).

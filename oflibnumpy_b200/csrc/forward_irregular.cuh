@@ -385,7 +385,12 @@ OFK_HD uint32_t apex_site(const SiteGrid& g, uint32_t a, uint32_t b, const P2& p
 
 constexpr int LOC_FOUND = 0, LOC_OUTSIDE = 1, LOC_FAILED = 2, LOC_HEAVY = 3;
 constexpr int NO_BUDGET = 0x7fffffff;
-constexpr int LOC_MAX_STEPS = 512;
+// a safety net against a walk that cycles on rounding, not a budget: the walk from the nearest site crosses every
+// triangle between it and q, and in a frame stretched 3x (a 375 x 1242 non-affine zoom) those are more than 512
+#ifndef OFK_LOC_MAX_STEPS
+#define OFK_LOC_MAX_STEPS 65536
+#endif
+constexpr int LOC_MAX_STEPS = OFK_LOC_MAX_STEPS;
 
 // The walk: from the Delaunay edge a -> b (q on its left or on its line) to the triangle that contains q.
 OFK_HD int locate_walk(const SiteGrid& g, const P2& q, uint32_t a, uint32_t b, P2 pa, P2 pb, uint32_t (&ids)[3],

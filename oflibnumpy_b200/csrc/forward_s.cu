@@ -17,9 +17,10 @@
 //                       located in the Delaunay triangulation of the boundary sites (frame border, rims of removed
 //                       points), binned by position with two counting passes and a scan; a per-frame hull polygon
 //                       rejects the pixels outside the hull without a search.
-//   legacy::fwd_scatter / fwd_gather   folding fields (a displaced cell with a non-positive triangle): several
-//                       triangles cover a pixel, "exactly one" no longer holds; such frames are redone completely by
-//                       the order-independent atomicMax(triangle id) resolve of round 1 (largest source index wins).
+//   folding frames      a displaced cell with a non-positive triangle (any cell of the frame, also one that holds no
+//                       pixel) flags the frame: the mesh of the cells is not a triangulation there. After the join the
+//                       frame is triangulated as a whole: every kept point is a site, the cover plane goes back to the
+//                       marker and every pixel is located by the irr_* kernels (fwd_fold_reset_kernel, second run).
 //
 // Deviation left (DESIGN.md): cells whose four corners are co-circular to within rounding have no unique Delaunay
 // diagonal (similarity transforms of the pixel grid); Qhull's pick there is an artefact of its facet merging.
@@ -31,21 +32,13 @@
 #include "forward_irregular.cuh"
 #include "track_device.cuh"
 
-// ============================================================ order-independent resolve for folding fields (round 1)
+// ========================================================== predicates of the mesh sampler (mesh_sample_kernel below)
 namespace ofk {
 namespace legacy {
 
 struct P2 {
     double x, y;
 };
-
-__device__ __forceinline__ P2 displaced(const float2* __restrict__ fl, int W, int row, int col, float sign) {
-    const float2 f = __ldg(fl + row * W + col);
-    P2 p;
-    p.x = static_cast<double>(col) + static_cast<double>(sign * f.x);
-    p.y = static_cast<double>(row) + static_cast<double>(sign * f.y);
-    return p;
-}
 
 __device__ __forceinline__ double orient(const P2& a, const P2& b, const P2& c) {
     return (b.x - a.x) * (c.y - a.y) - (b.y - a.y) * (c.x - a.x);
@@ -86,149 +79,6 @@ __device__ __forceinline__ int corner_of(int diag, int tri, int k) {
 __device__ __forceinline__ double edge_fn(const P2& u, int iu, const P2& v, int iv, double qx, double qy) {
     if (iu < iv) return (v.x - u.x) * (qy - u.y) - (v.y - u.y) * (qx - u.x);
     return -((u.x - v.x) * (qy - v.y) - (u.y - v.y) * (qx - v.x));
-}
-
-__device__ __forceinline__ void scatter_tile(const float* __restrict__ flow, float sign,
-                                             const uint8_t* __restrict__ point_mask,
-                                             unsigned int* __restrict__ winner, int H, int W, int bx, int by, int n) {
-    const int j = bx * 32 + (threadIdx.x & 31);
-    const int i = by * 8 + (threadIdx.x >> 5);
-    if (i >= H - 1 || j >= W - 1) return;
-    const size_t fbase = (size_t)n * H * W;
-    const float2* fl = reinterpret_cast<const float2*>(flow) + fbase;
-    if (point_mask != nullptr) {
-        const uint8_t* pm = point_mask + fbase;
-        const int o = i * W + j;
-        if (!(pm[o] && pm[o + 1] && pm[o + W] && pm[o + W + 1])) return;
-    }
-    P2 v[4];
-    v[0] = displaced(fl, W, i, j, sign);
-    v[1] = displaced(fl, W, i, j + 1, sign);
-    v[2] = displaced(fl, W, i + 1, j, sign);
-    v[3] = displaced(fl, W, i + 1, j + 1, sign);
-    const int vid[4] = {i * W + j, i * W + j + 1, (i + 1) * W + j, (i + 1) * W + j + 1};
-    const int diag = choose_diagonal(v[0], v[1], v[2], v[3]);
-    unsigned int* win = winner + fbase;
-#pragma unroll
-    for (int tri = 0; tri < 2; ++tri) {
-        const int c0 = corner_of(diag, tri, 0), c1 = corner_of(diag, tri, 1), c2 = corner_of(diag, tri, 2);
-        const P2 p0 = v[c0], p1 = v[c1], p2 = v[c2];
-        const double area2 = orient(p0, p1, p2);
-        if (area2 == 0.0) continue;
-        const double sgn = area2 > 0 ? 1.0 : -1.0;
-        // candidate pixels: bounding box in float32, rounded outwards (a superset is enough: coverage is decided by
-        // the exact edge functions below)
-        int xmin = (int)ceilf(fminf(__double2float_rd(p0.x), fminf(__double2float_rd(p1.x), __double2float_rd(p2.x))));
-        int xmax = (int)floorf(fmaxf(__double2float_ru(p0.x), fmaxf(__double2float_ru(p1.x), __double2float_ru(p2.x))));
-        int ymin = (int)ceilf(fminf(__double2float_rd(p0.y), fminf(__double2float_rd(p1.y), __double2float_rd(p2.y))));
-        int ymax = (int)floorf(fmaxf(__double2float_ru(p0.y), fmaxf(__double2float_ru(p1.y), __double2float_ru(p2.y))));
-        xmin = max(xmin, 0);
-        ymin = max(ymin, 0);
-        xmax = min(xmax, W - 1);
-        ymax = min(ymax, H - 1);
-        const unsigned int id = ((unsigned int)(i * W + j) << 2 | (unsigned int)(tri << 1) | (unsigned int)diag) + 1u;
-        for (int y = ymin; y <= ymax; ++y) {
-            for (int x = xmin; x <= xmax; ++x) {
-                const double qx = x, qy = y;
-                const double e0 = sgn * edge_fn(p1, vid[c1], p2, vid[c2], qx, qy);
-                const double e1 = sgn * edge_fn(p2, vid[c2], p0, vid[c0], qx, qy);
-                const double e2 = sgn * edge_fn(p0, vid[c0], p1, vid[c1], qx, qy);
-                if (e0 >= 0.0 && e1 >= 0.0 && e2 >= 0.0) atomicMax(win + y * W + x, id);
-            }
-        }
-    }
-}
-
-// The resolve kernels run on small grids that loop over the tiles of the frames flagged as folded: for every other
-// frame (the normal case) a launch costs a few hundred empty CTAs instead of one per tile.
-__global__ void __launch_bounds__(256, 4) fwd_scatter(const float* __restrict__ flow, float sign,
-                                                   const uint8_t* __restrict__ point_mask,
-                                                   unsigned int* __restrict__ winner, int H, int W,
-                                                   const int* __restrict__ folded) {
-    const int n = blockIdx.y;
-    if (folded[n] != 1) return;
-    const int tx = (W - 1 + 31) / 32, ty = (H - 1 + 7) / 8;
-    for (int t = blockIdx.x; t < tx * ty; t += gridDim.x) scatter_tile(flow, sign, point_mask, winner, H, W, t % tx, t / tx, n);
-}
-
-__device__ __forceinline__ void gather_tile(const float* __restrict__ payload, int C,
-                                            const float* __restrict__ flow, float sign,
-                                            const uint8_t* __restrict__ payload_mask,
-                                            const unsigned int* __restrict__ winner, float* __restrict__ out,
-                                            uint8_t* __restrict__ out_mask, int rule, int H, int W,
-                                            unsigned long long inv_w /* ceil(2^64 / W) */, int bx, int by, int n) {
-    const int x = bx * 32 + (threadIdx.x & 31);
-    const int y = by * 8 + (threadIdx.x >> 5);
-    if (x >= W || y >= H) return;
-    const size_t fbase = (size_t)n * H * W;
-    const int pix = y * W + x;
-    const unsigned int id = winner[fbase + pix];
-    if (id == 0u) {
-        for (int c = 0; c < C; ++c) out[(fbase + pix) * C + c] = 0.f;
-        if (out_mask) out_mask[fbase + pix] = 0;
-        return;
-    }
-    const unsigned int code = id - 1u;
-    const int diag = code & 1, tri = (code >> 1) & 1, cell = (int)(code >> 2);
-    const int i = (int)__umul64hi((unsigned long long)cell, inv_w), j = cell - i * W;   // exact: cell < 2^29
-    const float2* fl = reinterpret_cast<const float2*>(flow) + fbase;
-    int vidx[3];
-    P2 p[3];
-#pragma unroll
-    for (int k = 0; k < 3; ++k) {
-        const int c = corner_of(diag, tri, k);
-        const int r = i + (c >> 1), q = j + (c & 1);
-        vidx[k] = r * W + q;
-        p[k] = displaced(fl, W, r, q, sign);
-    }
-    const double area2 = orient(p[0], p[1], p[2]);
-    const double qx = x, qy = y;
-    // one reciprocal instead of two divisions: the weights move by an ulp at most (values are compared at 1e-3, the
-    // mask tests below are decided by exact zeros and by margins far above an ulp)
-    const double inv_area = __drcp_rn(area2);
-    double w0 = edge_fn(p[1], vidx[1], p[2], vidx[2], qx, qy) * inv_area;
-    double w1 = edge_fn(p[2], vidx[2], p[0], vidx[0], qx, qy) * inv_area;
-    double w2 = 1.0 - w0 - w1;
-    const float* pay = payload + fbase * C;
-    for (int c = 0; c < C; ++c) {
-        const double val = w0 * (double)__ldg(pay + (size_t)vidx[0] * C + c) +
-                           w1 * (double)__ldg(pay + (size_t)vidx[1] * C + c) +
-                           w2 * (double)__ldg(pay + (size_t)vidx[2] * C + c);
-        out[(fbase + pix) * C + c] = (float)val;
-    }
-    if (out_mask) {
-        double m = w0 + w1 + w2;
-        if (payload_mask) {
-            const uint8_t* pm = payload_mask + fbase;
-            m = (pm[vidx[0]] ? w0 : 0.0) + (pm[vidx[1]] ? w1 : 0.0) + (pm[vidx[2]] ? w2 : 0.0);
-        }
-        bool ok;
-        if (rule == OFK_RULE_STRICT) ok = ((float)m == 1.0f);   // float payloads: `== 1` after the float32 cast
-        else ok = (m > 0.5);                                    // integer payloads: np.round(m) == 1
-        out_mask[fbase + pix] = ok ? 1 : 0;
-    }
-}
-
-
-__global__ void __launch_bounds__(256) fwd_gather(const float* __restrict__ payload, int C,
-                                                  const float* __restrict__ flow, float sign,
-                                                  const uint8_t* __restrict__ payload_mask,
-                                                  const unsigned int* __restrict__ winner, float* __restrict__ out,
-                                                  uint8_t* __restrict__ out_mask, int rule, int H, int W,
-                                                  unsigned long long inv_w, const int* __restrict__ folded) {
-    const int n = blockIdx.y;
-    if (folded[n] != 1) return;
-    const int tx = (W + 31) / 32, ty = (H + 7) / 8;
-    for (int t = blockIdx.x; t < tx * ty; t += gridDim.x)
-        gather_tile(payload, C, flow, sign, payload_mask, winner, out, out_mask, rule, H, W, inv_w, t % tx, t / tx, n);
-}
-
-__global__ void __launch_bounds__(256) fwd_clear(unsigned int* __restrict__ winner, size_t frame_px,
-                                                 const int* __restrict__ folded) {
-    const int n = blockIdx.y;
-    if (folded[n] != 1) return;
-    for (size_t t = (size_t)blockIdx.x * 256 + threadIdx.x; t < frame_px; t += (size_t)gridDim.x * 256)
-        winner[(size_t)n * frame_px + t] = 0u;
 }
 
 }  // namespace legacy
@@ -428,7 +278,7 @@ __global__ void __launch_bounds__(256, OFK_RASTER_CTAS) fwd_raster_kernel(const 
         } else {
             double ar[2];
             diag = cell_diagonal(a, b, c, d, ar, A.flip_tol);
-            if (diag < 0) return;   // folded: the frame is redone by the resolve kernels
+            if (diag < 0) return;   // folded: the frame is triangulated as a whole after the join
             tri = owner_triangle(a, b, c, d, diag, qx, qy);
             if (tri < 0) return;
             area2 = ar[tri];
@@ -496,19 +346,19 @@ __global__ void __launch_bounds__(256, OFK_RASTER_CTAS) fwd_raster_kernel(const 
                 const int ny = y1 - y0 + 1;
                 if (nx > 0 && ny > 0) ncand = nx * ny;
             }
-            if (ncand > 0) {
-                const float mo = 16.0f * eps * ext;
-                const bool ok = orientf(af, bf, df) > mo && orientf(af, df, cf) > mo && orientf(af, bf, cf) > mo &&
-                                orientf(bf, df, cf) > mo;
-                if (ok) {
-                    flag = REC_OK;
-                } else {
-                    const P2 a = s_pos[sb], b = s_pos[sb + 1], c = s_pos[sb + SW], d = s_pos[sb + SW + 1];
-                    double ar[2];
-                    if (cell_diagonal(a, b, c, d, ar, A.flip_tol) < 0) {
-                        A.folded[n] = 1;
-                        ncand = 0;
-                    }
+            // every intact cell is checked, also one without candidate pixels: a fold anywhere changes the Delaunay
+            // triangulation of the whole frame
+            const float mo = 16.0f * eps * ext;
+            const bool ok = orientf(af, bf, df) > mo && orientf(af, df, cf) > mo && orientf(af, bf, cf) > mo &&
+                            orientf(bf, df, cf) > mo;
+            if (ok) {
+                flag = REC_OK;
+            } else {
+                const P2 a = s_pos[sb], b = s_pos[sb + 1], c = s_pos[sb + SW], d = s_pos[sb + SW + 1];
+                double ar[2];
+                if (cell_diagonal(a, b, c, d, ar, A.flip_tol) < 0) {
+                    A.folded[n] = 1;
+                    ncand = 0;
                 }
             }
             if (ncand > 4) {   // a stretched cell: rasterised on the spot by the generic float64 loop
@@ -563,6 +413,8 @@ struct IrrArgs {
     unsigned long long* holes;   // removed points (frame << 32 | index), the candidates for hole_fill()
     unsigned int* hole_count;
     unsigned int hole_cap;
+    int all_points;      // folded frames: every kept point is a site
+    long long span;      // threads per frame the kernels cover (grid-strided)
 };
 
 __device__ __forceinline__ bool frame_is_plain(const int* masked, int n, int H, int W) {
@@ -570,6 +422,12 @@ __device__ __forceinline__ bool frame_is_plain(const int* masked, int n, int H, 
 }
 
 __device__ __forceinline__ bool irr_site_of_thread(const IrrArgs& A, int n, long long t, int& row, int& col) {
+    if (A.all_points) {
+        if (t >= (long long)A.H * A.W) return false;
+        row = (int)(t / A.W);
+        col = (int)(t - (long long)row * A.W);
+        return A.point_mask == nullptr || A.point_mask[(size_t)n * A.H * A.W + t] != 0;
+    }
     if (A.perimeter_only || frame_is_plain(A.masked, n, A.H, A.W)) {
         const long long P = 2ll * A.W + 2ll * (A.H - 2);
         if (t >= P) return false;
@@ -627,40 +485,44 @@ template <int PASS>   // 0: count sites per bin, 1: fill the site lists (bins ho
 __global__ void __launch_bounds__(256) irr_sites_kernel(const IrrArgs A) {
     const int n = blockIdx.y;
     if (A.folded[n]) return;
-    int row, col;
     const size_t frame = (size_t)n * A.H * A.W;
-    const long long t = (long long)blockIdx.x * 256 + threadIdx.x;
-    const bool site = irr_site_of_thread(A, n, t, row, col);
-    if (PASS == 0 && !A.perimeter_only && !frame_is_plain(A.masked, n, A.H, A.W)) {
-        // removed points are queued for the small-face pass: one atomic per warp
-        const bool removed = !site && t < (long long)A.H * A.W && A.point_mask != nullptr && !A.point_mask[frame + t];
-        const unsigned bal = __ballot_sync(0xffffffffu, removed);
-        if (bal) {
-            const int lane = threadIdx.x & 31, leader = __ffs(bal) - 1;
-            unsigned slot = 0;
-            if (lane == leader) slot = atomicAdd(A.hole_count, (unsigned)__popc(bal));
-            slot = __shfl_sync(0xffffffffu, slot, leader) + __popc(bal & ((1u << lane) - 1u));
-            if (removed && slot < A.hole_cap) A.holes[slot] = ((unsigned long long)n << 32) | (unsigned long long)t;
+    // block-uniform stride loop: one trip per CTA when the grid covers `span` (small grids for the folded-frame run)
+    for (long long t0 = (long long)blockIdx.x * 256; t0 < A.span; t0 += (long long)gridDim.x * 256) {
+        const long long t = t0 + threadIdx.x;
+        int row, col;
+        const bool site = irr_site_of_thread(A, n, t, row, col);
+        if (PASS == 0 && !A.perimeter_only && !A.all_points && !frame_is_plain(A.masked, n, A.H, A.W)) {
+            // removed points are queued for the small-face pass: one atomic per warp
+            const bool removed = !site && t < (long long)A.H * A.W && A.point_mask != nullptr && !A.point_mask[frame + t];
+            const unsigned bal = __ballot_sync(0xffffffffu, removed);
+            if (bal) {
+                const int lane = threadIdx.x & 31, leader = __ffs(bal) - 1;
+                unsigned slot = 0;
+                if (lane == leader) slot = atomicAdd(A.hole_count, (unsigned)__popc(bal));
+                slot = __shfl_sync(0xffffffffu, slot, leader) + __popc(bal & ((1u << lane) - 1u));
+                if (removed && slot < A.hole_cap) A.holes[slot] = ((unsigned long long)n << 32) | (unsigned long long)t;
+            }
         }
-    }
-    if (!site) return;
-    if (PASS == 0 && A.point_mask != nullptr && !A.perimeter_only && !frame_is_plain(A.masked, n, A.H, A.W) &&
-        site_is_isolated(A.point_mask + frame, A.H, A.W, row, col))
-        A.isolated[n] = 1;
-    const uint32_t id = (uint32_t)(row * A.W + col);
-    const float2 f = __ldg(reinterpret_cast<const float2*>(A.flow) + frame + id);
-    const P2 p = displaced(f.x, f.y, row, col, A.sign);
-    const int bx = bin_coord(p.x, A.nbx), by = bin_coord(p.y, A.nby);
-    const int nb = grid_slots(A.nbx, A.nby);
-    uint32_t* bins = A.bins + (size_t)n * (nb + 1);
-    const int bi = bin_index(A.nbx, bx, by);
-    if (PASS == 0) {
-        atomicAdd(bins + bi, 1u);
-        atomicOr(A.occ + (size_t)n * A.ncx * A.ncy + (by >> COARSE_SHIFT) * A.ncx + (bx >> COARSE_SHIFT),
-                 1ull << ((((by & ((1 << COARSE_SHIFT) - 1)) << COARSE_SHIFT)) | (bx & ((1 << COARSE_SHIFT) - 1))));
-    } else {
-        const uint32_t slot = atomicSub(bins + bi, 1u) - 1u;
-        A.sites[frame + slot] = id;
+        if (!site) continue;
+        if (PASS == 0 && A.point_mask != nullptr && !A.perimeter_only && !A.all_points &&
+            !frame_is_plain(A.masked, n, A.H, A.W) &&
+            site_is_isolated(A.point_mask + frame, A.H, A.W, row, col))
+            A.isolated[n] = 1;
+        const uint32_t id = (uint32_t)(row * A.W + col);
+        const float2 f = __ldg(reinterpret_cast<const float2*>(A.flow) + frame + id);
+        const P2 p = displaced(f.x, f.y, row, col, A.sign);
+        const int bx = bin_coord(p.x, A.nbx), by = bin_coord(p.y, A.nby);
+        const int nb = grid_slots(A.nbx, A.nby);
+        uint32_t* bins = A.bins + (size_t)n * (nb + 1);
+        const int bi = bin_index(A.nbx, bx, by);
+        if (PASS == 0) {
+            atomicAdd(bins + bi, 1u);
+            atomicOr(A.occ + (size_t)n * A.ncx * A.ncy + (by >> COARSE_SHIFT) * A.ncx + (bx >> COARSE_SHIFT),
+                     1ull << ((((by & ((1 << COARSE_SHIFT) - 1)) << COARSE_SHIFT)) | (bx & ((1 << COARSE_SHIFT) - 1))));
+        } else {
+            const uint32_t slot = atomicSub(bins + bi, 1u) - 1u;
+            A.sites[frame + slot] = id;
+        }
     }
 }
 
@@ -668,8 +530,10 @@ __global__ void __launch_bounds__(256) irr_sites_kernel(const IrrArgs A) {
 // sums, scan inside the chunks): a single CTA per frame took 100 us for the 130 k bins of a 1080p frame.
 constexpr int SCAN_CHUNK = 2048;   // bins per CTA, 8 per thread
 
+// skip (or nullptr): frames with skip[n] != 0 are left alone (the folded-frame run rescans only the folded frames)
 __global__ void __launch_bounds__(256) irr_scan_sums_kernel(const uint32_t* bins_all, int nb, uint32_t* chunk_sums,
-                                                            int chunks) {
+                                                            int chunks, const int* skip) {
+    if (skip != nullptr && skip[blockIdx.y]) return;
     const uint32_t* a = bins_all + (size_t)blockIdx.y * (nb + 1);
     const int b0 = blockIdx.x * SCAN_CHUNK + threadIdx.x * 8;
     uint32_t sum = 0;
@@ -686,7 +550,8 @@ __global__ void __launch_bounds__(256) irr_scan_sums_kernel(const uint32_t* bins
     }
 }
 
-__global__ void irr_scan_chunks_kernel(uint32_t* chunk_sums, int chunks) {   // exclusive, in place; one warp per frame
+__global__ void irr_scan_chunks_kernel(uint32_t* chunk_sums, int chunks, const int* skip) {   // exclusive, in place;
+    if (skip != nullptr && skip[blockIdx.x]) return;                                          // one warp per frame
     uint32_t* c = chunk_sums + (size_t)blockIdx.x * chunks;
     uint32_t carry = 0;
     for (int base = 0; base < chunks; base += 32) {
@@ -703,7 +568,8 @@ __global__ void irr_scan_chunks_kernel(uint32_t* chunk_sums, int chunks) {   // 
 }
 
 __global__ void __launch_bounds__(256) irr_scan_final_kernel(uint32_t* bins_all, int nb, const uint32_t* chunk_sums,
-                                                             int chunks) {
+                                                             int chunks, const int* skip) {
+    if (skip != nullptr && skip[blockIdx.y]) return;
     uint32_t* a = bins_all + (size_t)blockIdx.y * (nb + 1);
     const int b0 = blockIdx.x * SCAN_CHUNK + threadIdx.x * 8;
     uint32_t v[8], sum = 0;
@@ -779,50 +645,51 @@ __global__ void __launch_bounds__(256) hull_sites_kernel(const HullArgs A) {
     const int n = blockIdx.y;
     if (A.folded[n]) return;
     const uint32_t total = A.bins[(size_t)n * (A.nb + 1) + A.nb];
-    const uint32_t s0 = blockIdx.x * (256 * HULL_ITEMS);
-    if (s0 >= total) return;
-    const SiteGrid g = hull_grid(A, n);
-    HullWs& ws = A.ws[n];
-    const HullInfo& info = A.info[n];
-    const int lane = threadIdx.x & 31;
-    const int count = PASS == 2 ? info.m : HULL_DIRS;
-    // every thread folds its sites first, one warp reduction and one atomic per direction at the end (with removed
-    // points the rims of all holes are boundary sites: a hundred times more of them than on the frame border)
-    unsigned long long acc[HULL_DIRS];
+    // block-uniform stride loop (one trip per CTA when the grid covers the sites)
+    for (uint32_t s0 = blockIdx.x * (256 * HULL_ITEMS); s0 < total; s0 += gridDim.x * (256 * HULL_ITEMS)) {
+        const SiteGrid g = hull_grid(A, n);
+        HullWs& ws = A.ws[n];
+        const HullInfo& info = A.info[n];
+        const int lane = threadIdx.x & 31;
+        const int count = PASS == 2 ? info.m : HULL_DIRS;
+        // every thread folds its sites first, one warp reduction and one atomic per direction at the end (with removed
+        // points the rims of all holes are boundary sites: a hundred times more of them than on the frame border)
+        unsigned long long acc[HULL_DIRS];
 #pragma unroll
-    for (int k = 0; k < HULL_DIRS; ++k) acc[k] = PASS == 2 ? ~0ull : 0ull;
-    for (int it = 0; it < HULL_ITEMS; ++it) {
-        const uint32_t s = s0 + it * 256 + threadIdx.x;
-        if (s >= total) break;
-        const uint32_t id = g.sites[s];
-        const P2 p = site_pos(g, id);
+        for (int k = 0; k < HULL_DIRS; ++k) acc[k] = PASS == 2 ? ~0ull : 0ull;
+        for (int it = 0; it < HULL_ITEMS; ++it) {
+            const uint32_t s = s0 + it * 256 + threadIdx.x;
+            if (s >= total) break;
+            const uint32_t id = g.sites[s];
+            const P2 p = site_pos(g, id);
 #pragma unroll
-        for (int k = 0; k < HULL_DIRS; ++k) {
-            if (PASS == 0) {
-                const unsigned long long key = order_key(dfma(A.dirs.dx[k], p.x, dmul(A.dirs.dy[k], p.y)));
-                acc[k] = key > acc[k] ? key : acc[k];
-            } else if (PASS == 1) {
-                if (order_key(dfma(A.dirs.dx[k], p.x, dmul(A.dirs.dy[k], p.y))) == ws.dotkey[k]) atomicMin(&ws.ext[k], id);
-            } else if (k < count) {
-                const unsigned long long key = order_key(hull_edge_orient(info, k, p));
-                acc[k] = key < acc[k] ? key : acc[k];
+            for (int k = 0; k < HULL_DIRS; ++k) {
+                if (PASS == 0) {
+                    const unsigned long long key = order_key(dfma(A.dirs.dx[k], p.x, dmul(A.dirs.dy[k], p.y)));
+                    acc[k] = key > acc[k] ? key : acc[k];
+                } else if (PASS == 1) {
+                    if (order_key(dfma(A.dirs.dx[k], p.x, dmul(A.dirs.dy[k], p.y))) == ws.dotkey[k]) atomicMin(&ws.ext[k], id);
+                } else if (k < count) {
+                    const unsigned long long key = order_key(hull_edge_orient(info, k, p));
+                    acc[k] = key < acc[k] ? key : acc[k];
+                }
             }
         }
-    }
-    if (PASS == 1) return;
+        if (PASS == 1) continue;
 #pragma unroll
-    for (int k = 0; k < HULL_DIRS; ++k) {
-        if (PASS == 2 && k >= count) break;
-        unsigned long long key = acc[k];
-        for (int o = 16; o > 0; o >>= 1) {
-            const unsigned long long other = __shfl_xor_sync(0xffffffffu, key, o);
-            key = PASS == 0 ? (other > key ? other : key) : (other < key ? other : key);
-        }
-        if (lane == 0) {
-            if (PASS == 0) {
-                if (key != 0ull) atomicMax(&ws.dotkey[k], key);
-            } else {
-                atomicMin(&ws.slackkey[k], key);
+        for (int k = 0; k < HULL_DIRS; ++k) {
+            if (PASS == 2 && k >= count) break;
+            unsigned long long key = acc[k];
+            for (int o = 16; o > 0; o >>= 1) {
+                const unsigned long long other = __shfl_xor_sync(0xffffffffu, key, o);
+                key = PASS == 0 ? (other > key ? other : key) : (other < key ? other : key);
+            }
+            if (lane == 0) {
+                if (PASS == 0) {
+                    if (key != 0ull) atomicMax(&ws.dotkey[k], key);
+                } else {
+                    atomicMin(&ws.slackkey[k], key);
+                }
             }
         }
     }
@@ -1395,7 +1262,7 @@ struct SolveArgs {
     const HullPoly* poly;
     float* out;
     uint8_t* out_mask;
-    const uint8_t* cover;
+    uint8_t* cover;
     unsigned long long* heavy;       // work items of the pocket pass: frame << 40 | 8-pixel block << 8 | pixel bits
     unsigned int* heavy_count;
     unsigned long long* todo;        // pixels that need a search: frame << 32 | pixel
@@ -1409,8 +1276,8 @@ struct SolveArgs {
 constexpr int SOLVE_SPAN = 4096;          // pixels per CTA, 16 per thread
 constexpr int THREAD_BUDGET = 320;        // sites one thread looks at per apex search before the pixel goes to a warp
 
-// a located pixel is written; one outside the hull keeps its marker (fwd_finalize_kernel zeroes whatever is left: a
-// marker that turned into 0 here would look like a produced pixel to the neighbour test of irr_solve_kernel)
+// a located pixel is written and leaves the marker (without a validity plane the cover plane records it: else
+// fwd_finalize_kernel would zero it); one outside the hull keeps its marker (fwd_finalize_kernel zeroes whatever is left)
 __device__ __forceinline__ void solve_store(const SolveArgs& A, size_t frame, uint32_t p, int st, const uint32_t (&vid)[3],
                                             const double (&w)[3]) {
     if (st != LOC_FOUND) return;
@@ -1420,6 +1287,7 @@ __device__ __forceinline__ void solve_store(const SolveArgs& A, size_t frame, ui
     interp_store(pay + (size_t)vid[0] * A.C, pay + (size_t)vid[1] * A.C, pay + (size_t)vid[2] * A.C,
                  pm ? pm[vid[0]] != 0 : true, pm ? pm[vid[1]] != 0 : true, pm ? pm[vid[2]] != 0 : true, w[0], w[1],
                  w[2], A.C, A.out + px * A.C, A.out_mask ? A.out_mask + px : nullptr, A.rule_strict);
+    if (A.out_mask == nullptr) A.cover[px] = 1;
 }
 
 // Whatever still carries the marker after all passes lies outside the convex hull of the points: 0 / invalid
@@ -1737,6 +1605,7 @@ struct WsLayout {
     size_t sites, cover, heavy, todo, chain, hull_pos, chain_n, first_valid, isolated, todo_count, heavy_count, hole_count, masked, bins, coarse, hullws, hullinfo, folded, state_side, chunks, opos, oids, ocount, poly, total;
     size_t zero_begin, zero_bytes;   // region cleared before every call (bins, coarse, hull keys, folded flags)
     int nbx, nby, ncx, ncy, nb, nc, chain_cap;
+    size_t todo_cap;
 };
 
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
@@ -1751,14 +1620,17 @@ static WsLayout ws_layout(int N, int H, int W) {
     L.nc = L.ncx * L.ncy;
     const size_t px = (size_t)N * H * W;
     size_t o = 0;
-    L.sites = o;            // also the triangle-id plane of the legacy resolve (never used at the same time)
+    L.sites = o;
     o = align_up(o + px * 4, 256);
     L.cover = o;
     o = align_up(o + px, 256);
-    L.heavy = o;            // at most one item per 8 pixels
-    o = align_up(o + px + 8, 256);
-    L.todo = o;             // the same for the pixels waiting for a search
-    o = align_up(o + px + 8, 256);
+    // the pixels waiting for a search (8 B each): one per 8 pixels of the batch, at least a whole frame (every pixel
+    // of a folding frame is searched); the work items of the pocket pass come from that list, as many at most
+    L.todo_cap = std::max<size_t>((px + 8) / 8, (size_t)H * W);
+    L.heavy = o;
+    o = align_up(o + L.todo_cap * 8, 256);
+    L.todo = o;
+    o = align_up(o + L.todo_cap * 8, 256);
     L.chain_cap = 4 * (H + W);   // traced outer boundary of a masked frame
     L.chain = o;
     o = align_up(o + (size_t)N * L.chain_cap * 4, 256);
@@ -1804,6 +1676,39 @@ static WsLayout ws_layout(int N, int H, int W) {
     L.zero_bytes = o - L.zero_begin;
     L.total = o;
     return L;
+}
+
+// Frames the raster kernel flagged as folded are triangulated as a whole after the join. Their cover plane goes back to
+// the marker (raster CTAs may have produced parts of the frame before the flag was raised), their site grid and hull
+// (built before the join from the border sites) are cleared, and skip[n] = 0 selects them for the second run of the
+// site, hull and search kernels (1 for every other frame); the search lists of the first run are emptied.
+__global__ void __launch_bounds__(256) fwd_fold_reset_kernel(const int* __restrict__ state, int* __restrict__ skip,
+                                                             uint8_t* __restrict__ cover, size_t frame_px,
+                                                             uint32_t* __restrict__ bins, int nb,
+                                                             unsigned long long* __restrict__ occ, int nc,
+                                                             HullWs* __restrict__ hullws, unsigned int* __restrict__ ocount,
+                                                             unsigned int* __restrict__ todo_count,
+                                                             unsigned int* __restrict__ heavy_count) {
+    const int n = blockIdx.y;
+    const bool fold = state[n] == 1;
+    const size_t t0 = (size_t)blockIdx.x * 256 + threadIdx.x, step = (size_t)gridDim.x * 256;
+    if (t0 == 0) {
+        skip[n] = fold ? 0 : 1;
+        if (n == 0) {
+            *todo_count = 0u;
+            *heavy_count = 0u;
+        }
+    }
+    if (!fold) return;
+    for (size_t p = t0; p < frame_px; p += step) cover[(size_t)n * frame_px + p] = UNCOVERED;
+    for (size_t b = t0; b <= (size_t)nb; b += step) bins[(size_t)n * (nb + 1) + b] = 0u;
+    for (size_t c = t0; c < (size_t)nc; c += step) occ[(size_t)n * nc + c] = 0ull;
+    if (t0 < (size_t)HULL_DIRS) {
+        hullws[n].dotkey[t0] = 0ull;
+        hullws[n].slackkey[t0] = 0ull;
+        hullws[n].ext[t0] = NO_SITE;
+    }
+    if (t0 == 0) ocount[n] = 0u;
 }
 
 __global__ void hull_ws_init_kernel(HullWs* ws, int N) {
@@ -2008,6 +1913,7 @@ extern "C" int ofk_forward_s_ex(const float* payload, int C, const float* flow, 
     // finds folded is processed like any other here and skipped by everything after the join)
     // the list of removed points shares its buffer with the work items of the pocket pass (used one after the other)
     const unsigned int hole_cap = (unsigned int)std::min<size_t>(((size_t)N * H * W + 8) / 8, 0xffffffffu);
+    const unsigned int todo_cap = (unsigned int)std::min<size_t>(L.todo_cap, 0xffffffffu);
     int* d_masked = point_mask != nullptr ? reinterpret_cast<int*>(base + L.masked) : nullptr;
     unsigned int* d_first = reinterpret_cast<unsigned int*>(base + L.first_valid);
     int* d_isolated = reinterpret_cast<int*>(base + L.isolated);
@@ -2020,18 +1926,19 @@ extern "C" int ofk_forward_s_ex(const float* payload, int C, const float* flow, 
     IrrArgs I{flow, point_mask, d_state_side, d_bins, d_coarse, d_sites, flow_sign, H, W, L.nbx, L.nby, L.ncx, L.ncy,
               (point_mask == nullptr && H >= 3 && W >= 3) ? 1 : 0, d_masked, d_isolated,
               reinterpret_cast<unsigned long long*>(base + L.heavy),
-              reinterpret_cast<unsigned int*>(base + L.hole_count), hole_cap};
+              reinterpret_cast<unsigned int*>(base + L.hole_count), hole_cap, 0, 0};
     const long long cand = I.perimeter_only ? 2ll * W + 2ll * (H - 2) : (long long)H * W;
     dim3 sgrid((unsigned)((cand + 255) / 256), N);
+    I.span = (long long)sgrid.x * 256;
     irr_sites_kernel<0><<<sgrid, 256, 0, ss>>>(I);
     OFK_LAUNCHED();
     const int chunks = (L.nb + SCAN_CHUNK - 1) / SCAN_CHUNK;
     uint32_t* d_chunks = reinterpret_cast<uint32_t*>(base + L.chunks);
-    irr_scan_sums_kernel<<<dim3(chunks, N), 256, 0, ss>>>(d_bins, L.nb, d_chunks, chunks);
+    irr_scan_sums_kernel<<<dim3(chunks, N), 256, 0, ss>>>(d_bins, L.nb, d_chunks, chunks, nullptr);
     OFK_LAUNCHED();
-    irr_scan_chunks_kernel<<<N, 32, 0, ss>>>(d_chunks, chunks);
+    irr_scan_chunks_kernel<<<N, 32, 0, ss>>>(d_chunks, chunks, nullptr);
     OFK_LAUNCHED();
-    irr_scan_final_kernel<<<dim3(chunks, N), 256, 0, ss>>>(d_bins, L.nb, d_chunks, chunks);
+    irr_scan_final_kernel<<<dim3(chunks, N), 256, 0, ss>>>(d_bins, L.nb, d_chunks, chunks, nullptr);
     OFK_LAUNCHED();
     irr_sites_kernel<1><<<sgrid, 256, 0, ss>>>(I);
     OFK_LAUNCHED();
@@ -2109,7 +2016,7 @@ extern "C" int ofk_forward_s_ex(const float* payload, int C, const float* flow, 
                 reinterpret_cast<unsigned long long*>(base + L.heavy),
                 reinterpret_cast<unsigned int*>(base + L.heavy_count),
                 reinterpret_cast<unsigned long long*>(base + L.todo), reinterpret_cast<unsigned int*>(base + L.todo_count),
-                hole_cap, (disable & 4) ? 0 : 1, flow_sign, C, strict, H, W, L.nbx, L.nby, L.ncx, L.ncy};
+                todo_cap, (disable & 4) ? 0 : 1, flow_sign, C, strict, H, W, L.nbx, L.nby, L.ncx, L.ncy};
     dim3 vgrid((unsigned)(((size_t)H * W + SOLVE_SPAN - 1) / SOLVE_SPAN), N);
     irr_solve_kernel<<<vgrid, 256, 0, st>>>(S);
     OFK_LAUNCHED();
@@ -2130,18 +2037,65 @@ extern "C" int ofk_forward_s_ex(const float* payload, int C, const float* flow, 
             payload, C, payload_mask, out, out_mask, (size_t)H * W, d_folded);
         OFK_LAUNCHED();
     }
-    // ---- folding frames: redone by the order-independent resolve (no-ops for all other frames)
+    // ---- folding frames: triangulated as a whole, every kept point a site (empty CTAs for all other frames)
     if (H > 1 && W > 1) {
-        unsigned int* winner = reinterpret_cast<unsigned int*>(d_sites);
-        const int per_frame = std::max(8, std::min(1184, 4736 / N));   // ~ 8 CTAs per SM over the whole batch
-        dim3 lgrid(per_frame, N);
-        legacy::fwd_clear<<<lgrid, 256, 0, st>>>(winner, (size_t)H * W, d_folded);
+        int* d_skip = d_state_side;   // not read after the join: 0 = folded frame, 1 = done
+        const int per_frame = std::max(8, std::min(1184, 4736 / N));
+        fwd_fold_reset_kernel<<<dim3(per_frame, N), 256, 0, st>>>(
+            d_folded, d_skip, d_cover, (size_t)H * W, d_bins, L.nb, d_coarse, L.nc, d_hullws,
+            reinterpret_cast<unsigned int*>(base + L.ocount), S.todo_count, S.heavy_count);
         OFK_LAUNCHED();
-        legacy::fwd_scatter<<<lgrid, 256, 0, st>>>(flow, flow_sign, point_mask, winner, H, W, d_folded);
+        IrrArgs F = I;
+        F.folded = d_skip;
+        F.perimeter_only = 0;
+        F.all_points = 1;
+        const long long all = (long long)H * W;
+        F.span = all;
+        // small grids: a launch of one CTA per 256 pixels of every frame costs tens of microseconds per call even when
+        // no frame folds and every CTA returns at once
+        dim3 fgrid((unsigned)std::min<long long>((all + 255) / 256, 64), N);
+        irr_sites_kernel<0><<<fgrid, 256, 0, st>>>(F);
         OFK_LAUNCHED();
-        const unsigned long long inv_w = ~0ull / (unsigned long long)W + 1ull;   // ceil(2^64 / W), W >= 2
-        legacy::fwd_gather<<<lgrid, 256, 0, st>>>(payload, C, flow, flow_sign, payload_mask, winner, out, out_mask,
-                                                 mask_rule, H, W, inv_w, d_folded);
+        irr_scan_sums_kernel<<<dim3(chunks, N), 256, 0, st>>>(d_bins, L.nb, d_chunks, chunks, d_skip);
+        OFK_LAUNCHED();
+        irr_scan_chunks_kernel<<<N, 32, 0, st>>>(d_chunks, chunks, d_skip);
+        OFK_LAUNCHED();
+        irr_scan_final_kernel<<<dim3(chunks, N), 256, 0, st>>>(d_bins, L.nb, d_chunks, chunks, d_skip);
+        OFK_LAUNCHED();
+        irr_sites_kernel<1><<<fgrid, 256, 0, st>>>(F);
+        OFK_LAUNCHED();
+        HullArgs Hf = Hh;
+        Hf.folded = d_skip;
+        dim3 fhgrid((unsigned)std::min<long long>((all + 256 * HULL_ITEMS - 1) / (256 * HULL_ITEMS), 64), N);
+        hull_sites_kernel<0><<<fhgrid, 256, 0, st>>>(Hf);
+        OFK_LAUNCHED();
+        hull_sites_kernel<1><<<fhgrid, 256, 0, st>>>(Hf);
+        OFK_LAUNCHED();
+        hull_frame_kernel<0><<<N, 32, 0, st>>>(Hf);
+        OFK_LAUNCHED();
+        hull_sites_kernel<2><<<fhgrid, 256, 0, st>>>(Hf);
+        OFK_LAUNCHED();
+        hull_frame_kernel<1><<<N, 32, 0, st>>>(Hf);
+        OFK_LAUNCHED();
+        OuterArgs Of = O;
+        Of.folded = d_skip;
+        hull_outer_kernel<<<dim3((unsigned)std::min<long long>((all + 255) / 256, 64), N), 256, 0, st>>>(Of);
+        OFK_LAUNCHED();
+        hull_wrap_kernel<<<N, 256, 0, st>>>(Of);
+        OFK_LAUNCHED();
+        SolveArgs Sf = S;
+        Sf.folded = d_skip;
+        Sf.lonely_ok = 0;   // no pocket pass ran: a marked pixel among marked pixels can lie inside the hull
+        irr_solve_kernel<<<vgrid, 256, 0, st>>>(Sf);
+        OFK_LAUNCHED();
+        irr_search_kernel<<<sm_count() * 8, 128, 0, st>>>(Sf);
+        OFK_LAUNCHED();
+        irr_heavy_kernel<<<sm_count() * 4, 256, 0, st>>>(Sf);
+        OFK_LAUNCHED();
+        const size_t frame_px = (size_t)H * W;
+        const int fin_ctas = (int)std::max<size_t>(1, std::min<size_t>((frame_px + 4095) / 4096,
+                                                                       (size_t)std::max(8, 4736 / N)));
+        fwd_finalize_kernel<<<dim3(fin_ctas, N), 256, 0, st>>>(out, C, out_mask, d_cover, frame_px, d_skip);
         OFK_LAUNCHED();
     }
     return OFK_OK;

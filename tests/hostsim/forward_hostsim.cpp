@@ -6,6 +6,7 @@
 #include <stdint.h>
 #include <string.h>
 
+#include <algorithm>
 #include <vector>
 
 #include "../../oflibnumpy_b200/csrc/forward_irregular.cuh"
@@ -49,7 +50,10 @@ struct EmitHost {
 }  // namespace
 
 // stats: [0] pixels from intact cells, [1] irregular pixels located, [2] outside the hull (located), [3] walk failures,
-//        [4] rejected by the hull pre-filter, [5] folded cells, [6] pixels produced more than once, [7] boundary sites
+//        [4] rejected by the hull pre-filter, [5] folded cells, [6] pixels produced more than once, [7] boundary sites,
+//        [10] 1 when the frame folds and was triangulated as a whole
+// A frame with a folded cell (a displaced cell that is not a positively oriented quadrilateral) is not a mesh of its
+// cells: every kept point becomes a site and every pixel is located in their Delaunay triangulation, as on the device.
 extern "C" int fwd_hostsim(const float* payload, int C, const float* flow, float sign, const uint8_t* payload_mask,
                            const uint8_t* point_mask, float* out, uint8_t* out_mask, int rule_strict, int H, int W,
                            int use_prefilter, double flip_tol, long long* stats) {
@@ -82,6 +86,12 @@ extern "C" int fwd_hostsim(const float* payload, int C, const float* flow, float
     }
     for (size_t k = 0; k < cover.size(); ++k)
         if (cover[k] > 1) ++stats[6];
+    const bool whole = stats[5] > 0;
+    if (whole) {
+        stats[10] = 1;
+        stats[0] = stats[6] = 0;
+        std::fill(cover.begin(), cover.end(), 0);
+    }
     // ---- boundary sites, binned by position
     SiteGrid g;
     g.H = H;
@@ -99,7 +109,9 @@ extern "C" int fwd_hostsim(const float* payload, int C, const float* flow, float
     std::vector<uint32_t> ids;
     for (int i = 0; i < H; ++i)
         for (int j = 0; j < W; ++j)
-            if (is_boundary_site(point_mask, H, W, i, j)) ids.push_back((uint32_t)(i * W + j));
+            if (whole ? (point_mask == nullptr || point_mask[(size_t)i * W + j] != 0)
+                      : is_boundary_site(point_mask, H, W, i, j))
+                ids.push_back((uint32_t)(i * W + j));
     stats[7] = (long long)ids.size();
     std::vector<int> bin_of(ids.size());
     for (size_t k = 0; k < ids.size(); ++k) {
@@ -150,7 +162,7 @@ extern "C" int fwd_hostsim(const float* payload, int C, const float* flow, float
     std::vector<int> hull_pos;
     Chain ch{nullptr, 0, H, W};
     bool have_chain = false;
-    if (poly.ok && H >= 3 && W >= 3 && (flags & 4) == 0) {
+    if (!whole && poly.ok && H >= 3 && W >= 3 && (flags & 4) == 0) {
         bool removed_any = false;
         if (point_mask != nullptr)
             for (size_t k = 0; k < (size_t)H * W && !removed_any; ++k) removed_any = point_mask[k] == 0;
@@ -228,7 +240,7 @@ extern "C" int fwd_hostsim(const float* payload, int C, const float* flow, float
         }
     }
     // ---- small faces left by removed points: triangulated by the thread of their first removed point
-    if (point_mask != nullptr && (flags & 8) == 0) {
+    if (!whole && point_mask != nullptr && (flags & 8) == 0) {
         const uint8_t* pm = payload_mask;
         for (int r = 0; r < H; ++r)
             for (int c = 0; c < W; ++c) {

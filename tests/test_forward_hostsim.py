@@ -47,7 +47,7 @@ def sim(tmp_path_factory):
                         flags, C.c_double(flip), ptr(stats))
         run.stats = stats
         assert stats[3] == 0, "point-location walks that did not terminate"
-        assert stats[5] == 0, "folded cells"
+        assert stats[5] == 0 or stats[10] == 1, "folded cells left to the mesh of the cells"
         assert stats[6] == 0, "pixels produced by more than one triangle: the fill rule is broken"
         return out[..., :c], om.astype(bool)
     return run

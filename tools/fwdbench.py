@@ -2,8 +2,10 @@
 
     python tools/fwdbench.py [N] [H] [W]
 
-rotation-type flows (cfg 4 transforms) without / with 2 % of the points removed (`consider_mask`), and a smooth
-non-affine field (curved frame border -> hull pockets). Device-resident inputs, CUDA events on the library's stream.
+rotation-type flows (cfg 4 transforms) without / with 2 % of the points removed (`consider_mask`), a smooth
+non-affine field (curved frame border -> hull pockets), and a folding field (an occlusion band: the frame is
+triangulated as a whole) as one frame and as a batch of 16. Device-resident inputs, CUDA events on the library's
+stream.
 """
 import json
 import os
@@ -81,6 +83,46 @@ timeit("rotation: invert, 2 % masked, consider_mask=False (18 B/px)", 18, fwd(fa
 timeit("smooth field: invert, full masks (18 B/px)", 18, fwd(fsm.vecs, 2, fsm.vecs, fsm.masks, None, o_v), reps=3)
 timeit("smooth field: invert, 2 % points removed (18 B/px)", 18, fwd(fsm.vecs, 2, fsm.vecs, mask, mask, o_v), reps=3)
 stats1 = [c('ofk_rt_path_count', k) for k in range(6, 10)]
+
+
+def folds(vecs):
+    """Cells of the displaced grid that are not positively oriented convex quadrilaterals (a folding field)."""
+    y, x = np.mgrid[:vecs.shape[0], :vecs.shape[1]].astype(np.float64)
+    px, py = x + vecs[..., 0].astype(np.float64), y + vecs[..., 1].astype(np.float64)
+    a, b, cc, d = [(px[i:i + vecs.shape[0] - 1, j:j + vecs.shape[1] - 1], py[i:i + vecs.shape[0] - 1, j:j + vecs.shape[1] - 1])
+                   for i, j in ((0, 0), (0, 1), (1, 0), (1, 1))]
+
+    def orient(p, q, r):
+        return (q[0] - p[0]) * (r[1] - p[1]) - (q[1] - p[1]) * (r[0] - p[0])
+    ok = (orient(a, b, d) > 0) & (orient(a, d, cc) > 0) & (orient(a, b, cc) > 0) & (orient(b, d, cc) > 0)
+    return int((~ok).sum())
+
+
+# the fields of bench.py's forward_s block must not fold (a folding frame is triangulated as a whole, far slower)
+print("cells that fold: rotation %d, smooth %d" % (sum(folds(v) for v in fa.vecs.numpy()), folds(gi.smooth_field(H, W))),
+      flush=True)
+
+
+def fold_field(h, w):
+    """An occlusion band moving 6 px over a slightly sheared background, as estimated flows have them."""
+    y, x = np.mgrid[:h, :w].astype(np.float64)
+    band = (x > 0.4 * w) & (x < 0.65 * w)
+    return np.dstack([np.where(band, 6.0, 0.3) + 0.02 * y + 0.013 * x, 0.1 + 0.01 * x + 0.017 * y]).astype(np.float32)
+
+
+for nf in (1, 16):
+    fv = DeviceArray.from_numpy(np.ascontiguousarray(np.broadcast_to(fold_field(H, W)[None], (nf, H, W, 2))))
+    fo = DeviceArray.empty((nf, H, W, 2), np.float32)
+    fm = DeviceArray.empty((nf, H, W), np.uint8)
+    fws_bytes = _lib.call('ofk_forward_s_workspace', nf, H, W)
+    fws = DeviceArray.empty((max(fws_bytes, 16),), np.uint8)
+    run = (lambda nf=nf, fv=fv, fo=fo, fm=fm, fws=fws, fws_bytes=fws_bytes:
+           c('ofk_forward_s', fv.ptr, 2, fv.ptr, 1.0, None, None, fo.ptr, fm.ptr, _lib.RULE_STRICT, nf, H, W, fws.ptr,
+             fws_bytes, s))
+    px_all = px
+    px = nf * H * W
+    timeit("folding field (occlusion band): invert, %d frame%s (18 B/px)" % (nf, "s" if nf > 1 else ""), 18, run, reps=3)
+    px = px_all
 print(json.dumps({"N": N, "H": H, "W": W, "peak_gbs": PEAK, "ops": results,
                   "irregular_pixels": dict(zip(("located", "outside_by_search", "failed", "hull_rejected"),
                                                [b - a for a, b in zip(stats0, stats1)]))}))
